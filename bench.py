@@ -362,8 +362,42 @@ class DeviceBundle:
                                                    st.ctypes.data_as(self._lib.c_ip), C.byref(cnt)))
         return cnt.as_dict(), dep, st
 
+    def results(self):
+        """Every array torj_bundle_results hands its caller after the last trace, and the counters."""
+        dp, ip = (lambda a: a.ctypes.data_as(self._lib.c_dp)), (lambda a: a.ctypes.data_as(self._lib.c_ip))
+        r = dict(dP_dV=np.zeros((self.n_beams, N_PSI)), deposited_power=np.zeros(self.n_beams), P_final=np.zeros(self.n),
+                 P_deposited_ray=np.zeros(self.n), n_points=np.zeros(self.n, dtype=np.int32), status=np.zeros(self.n, dtype=np.int32))
+        cnt = self._lib.TorjCounters()
+        self._lib.check(self.L.torj_bundle_results(self.bh, dp(r["dP_dV"]), dp(r["deposited_power"]), dp(r["P_final"]),
+                                                   dp(r["P_deposited_ray"]), ip(r["n_points"]), ip(r["status"]), C.byref(cnt)))
+        r["counters"] = np.array(list(cnt.as_dict().values()))
+        return r
+
     def close(self):
         self.L.torj_bundle_destroy(self.bh)
+
+
+PER_RAY = ("P_final", "P_deposited_ray", "n_points", "status")
+
+
+def dump_outputs(out_dir, bundles, rank, world, budget=64_000_000):
+    """--dump-outputs: the results of the last timed step as float64 .npy files, rays of several bundles concatenated,
+    profile rows stacked and counters summed; under several ranks each rank writes its own, prefixed rank<r>_. Per-ray
+    arrays that would take the file set over `budget` bytes are cut to a fixed seeded sample of rays, whose indices go to
+    ray_index.npy."""
+    rs = [b.results() for b in bundles]
+    out = {k: np.concatenate([r[k] for r in rs]).astype(np.float64) for k in rs[0] if k != "counters"}
+    out["counters"] = np.sum([r["counters"] for r in rs], axis=0).astype(np.float64)
+    n = len(out["P_final"])
+    fixed = sum(v.nbytes for k, v in out.items() if k not in PER_RAY)
+    if n * 8 * len(PER_RAY) > budget // world - fixed:
+        keep = (budget // world - fixed) // (8 * (len(PER_RAY) + 1))
+        idx = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        out.update({k: out[k][idx] for k in PER_RAY}, ray_index=idx.astype(np.float64))
+    os.makedirs(out_dir, exist_ok=True)
+    prefix = f"rank{rank}_" if world > 1 else ""
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, f"{prefix}{k}.npy"), v)
 
 
 def run_gpu_arm(args, wl):
@@ -452,6 +486,8 @@ def run_gpu_arm(args, wl):
         cb, _, _ = b.counters()
         for k, v in cb.items():
             c[k] = c.get(k, 0) + v
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, bundles, rank, world)  # before the alpha_floor = 0 pass below traces the bundles again
     kms = C.c_double()
     _lib.check(L.torj_ctx_last_trace_ms(ctx, C.byref(kms)))  # the last trace kernel alone, CUDA events on its own stream
 
@@ -666,7 +702,13 @@ def main():
     ap.add_argument("--schedule", type=int, default=0, choices=[0, 1, 2],
                     help="torj_options.schedule: 0 automatic (default), 1 whole rays per lane, 2 segment hand-off")
     ap.add_argument("--lanes-per-ray", type=int, default=0, choices=[0, 1, 32])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step to DIR/<name>.npy (float64; default --impl only)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the results of the CUDA path of the default --impl")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     wl = args.workload or ("small" if args.small else ("sweep1m" if max(world, args.gpus) > 1 else "beam64k"))
     if args.impl == "reference":
