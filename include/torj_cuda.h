@@ -193,6 +193,16 @@ int torj_bundle_set_beams(torj_bundle* b, int32_t n_beams, const int32_t* beam_i
  * make_ray (src/solve.jl:135-181) incl. power_deposition_profile (src/plasma.jl:91-151). */
 int torj_bundle_trace(torj_bundle* b, const torj_plasma* p, const torj_options* opt, double s_max, int32_t n_psi,
                       const double* psi_edges);
+/* Beams of one bundle traced through several equilibria on one (R,Z) grid: beam b through plasmas[beam_plasma[b]]; its
+ * profile row is normalised by that plasma's V(psi). n_beams from torj_bundle_set_beams. The plasmas must have bitwise
+ * equal grids (torj_grid of the same values) and live on the bundle's device. Refused (non-zero, torj_last_error):
+ * n_plasmas < 1, a NULL plasma, a plasma on another device, two different grids, and with n_plasmas > 1 a NULL or
+ * out-of-range beam_plasma or a single beam (a profile row belongs to one plasma). n_plasmas = 1 is torj_bundle_trace
+ * (beam_plasma unused). Like torj_bundle_trace it returns without synchronising: the plasmas must outlive the results
+ * read. Keep each beam's rays contiguous: a warp whose rays share a plasma shares its table rows. */
+int torj_bundle_trace_plasmas(torj_bundle* b, int32_t n_plasmas, const torj_plasma* const* plasmas,
+                              const int32_t* beam_plasma /* [n_beams] */, const torj_options* opt, double s_max,
+                              int32_t n_psi, const double* psi_edges);
 /* Device pointer to n_beams x (n_psi+2) doubles: dP_dV[n_psi], deposited_power, sum of weights per beam — for a caller-side
  * NCCL all-reduce (sum) across GPUs; valid after torj_bundle_trace, ordered on the context stream. */
 void* torj_bundle_device_profile(torj_bundle* b);
@@ -220,6 +230,15 @@ int torj_trace(torj_ctx* ctx, const torj_plasma* p, const torj_options* opt, int
                int32_t* n_points, int32_t* status,
                /* optional trajectories */ int64_t traj_first, int64_t traj_count, int32_t traj_max_pts, double* traj_s,
                double* traj_xyz, double* traj_P, double* traj_dP_ds, double* traj_dP_dV_ray, torj_counters* counters);
+/* torj_trace through a plasma set (torj_bundle_trace_plasmas): beam b of beam_id through plasmas[beam_plasma[b]]; the
+ * trajectory window's dP_dV_ray rows use the volume of each ray's plasma. Same refusals; blocking like torj_trace. */
+int torj_trace_plasmas(torj_ctx* ctx, int32_t n_plasmas, const torj_plasma* const* plasmas, const int32_t* beam_plasma,
+                       const torj_options* opt, int64_t n_rays, const double* pos, const double* dir, const double* weight,
+                       const double* freq_hz, const int32_t* mode, int32_t per_ray_fm, double s_max, int32_t n_psi,
+                       const double* psi_edges, int32_t n_beams, const int32_t* beam_id, double* dP_dV, double* deposited_power,
+                       double* P_final, double* P_deposited_ray, int32_t* n_points, int32_t* status, int64_t traj_first,
+                       int64_t traj_count, int32_t traj_max_pts, double* traj_s, double* traj_xyz, double* traj_P,
+                       double* traj_dP_ds, double* traj_dP_dV_ray, torj_counters* counters);
 
 /* --- single-process multi-GPU front end ----------------------------------------------------------------------- */
 /* For a host that is ONE process on a multi-GPU box (a Julia session calling make_beam): the same call as torj_trace,

@@ -133,6 +133,31 @@ function make_beam(plasma::Plasma, r, phi, z, tor, pol, spot, invRc, f, mode::In
     return arc, traj, pw, q.dP_dV, q.deposited, w
 end
 
+# make_beam_series — make_beam of one launcher on each plasma of a vector of plasmas on ONE (R,Z) grid (time slices, an
+# equilibrium ensemble) in one call, torj_trace_plasmas: the beam's rays go in once per plasma, contiguous, beam k through
+# plasmas[k] with its profile normalised by that plasma's V(psi). No trajectories. The plasmas' tables must outlive the call
+# (they do: torj_plasma(p) keeps them with p). Returns (dP_dV[n_psi, n_plasmas], deposited_power[n_plasmas], ray_weights,
+# P_final[n_rays, n_plasmas]).
+function make_beam_series(plasmas::Vector, r, phi, z, tor, pol, spot, invRc, f, mode::Integer, s_max::Float64, psi_dP_dV;
+                          options=torj_options(), kwargs...)
+    N0 = collect(IMAS.pol_tor_angles_2_vector(pol, tor)); x0 = [r * cos(phi), r * sin(phi), z]
+    pos, dir, w = launch_peripheral_rays(x0, N0, spot, invRc, f; kwargs...)
+    n = length(w); K = length(plasmas); npsi = length(psi_dP_dV)
+    hs = Ptr{Cvoid}[torj_plasma(p) for p in plasmas]
+    beam = Int32.(repeat(0:K-1, inner=n)); bp = Int32.(collect(0:K-1))
+    dP_dV = zeros(npsi, K); dep = zeros(K); Pf = zeros(n * K); Pd = zeros(n * K); npts = zeros(Int32, n * K); st = zeros(Int32, n * K)
+    cnt = Ref{TorjCounters}()
+    torj_check(ccall((:torj_trace_plasmas, libtorj), Cint,
+        (Ptr{Cvoid}, Int32, Ptr{Ptr{Cvoid}}, Ptr{Int32}, Ref{TorjOptions}, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ref{Float64},
+         Ref{Int32}, Int32, Float64, Int32, Ptr{Float64}, Int32, Ptr{Int32}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+         Ptr{Int32}, Ptr{Int32}, Int64, Int64, Int32, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+         Ref{TorjCounters}),
+        torj_ctx(), K, hs, bp, options, n * K, repeat(pos, K), repeat(dir, K), repeat(w, K), Float64(f), Int32(mode), 0, s_max,
+        npsi, psi_dP_dV, K, beam, dP_dV, dep, Pf, Pd, npts, st, 0, 0, 0, C_NULL, C_NULL, C_NULL, C_NULL, C_NULL, cnt))
+    all(ray_ok, st) || throw(AssertionError("ray status $(st)"))
+    return dP_dV, dep, w, reshape(Pf, n, K)
+end
+
 # α(omega, X, Y, N_r, theta, te, v_g_perp, imod) — src/general_absorption.jl:1328-1337 on the device (no set_extv! needed)
 function α(omega::Real, X::Real, Y::Real, N_r::Real, theta::Real, te::Real, v_g_perp::Real, imod::Integer)
     Nw = Ref(0.0); al = Ref(0.0); lrm = Ref(Int32(0)); ierr = Ref(Int32(0))

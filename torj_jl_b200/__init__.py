@@ -8,6 +8,6 @@ from .absorption import abs_Al_init, alpha_approx, warm_alpha  # noqa: F401
 from .launch import launch_peripheral_rays  # noqa: F401
 from .multi import MultiGPU  # noqa: F401
 from .plasma import Plasma, evaluate_psi  # noqa: F401
-from .solve import cylindrical_state, make_beam, make_beams, make_ray, trace_bundle  # noqa: F401
+from .solve import cylindrical_state, make_beam, make_beam_series, make_beams, make_ray, trace_bundle  # noqa: F401
 from .synthetic import pol_tor_angles_2_vector, solovev_arrays  # noqa: F401
-from .imas import plasma_arrays_from_dd, plasma_from_dd, plasma_from_imas_json, solovev_dd  # noqa: F401
+from .imas import plasma_arrays_from_dd, plasma_from_dd, plasma_from_imas_json, plasmas_from_dd, solovev_dd  # noqa: F401

@@ -68,6 +68,8 @@ SIGNATURES = {
     "torj_bundle_set_window": (C.c_int, [c_vp, C.c_int64, C.c_int64, C.c_int32]),
     "torj_bundle_set_beams": (C.c_int, [c_vp, C.c_int32, c_ip]),
     "torj_bundle_trace": (C.c_int, [c_vp, c_vp, C.POINTER(TorjOptions), C.c_double, C.c_int32, c_dp]),
+    "torj_bundle_trace_plasmas": (C.c_int, [c_vp, C.c_int32, C.POINTER(c_vp), c_ip, C.POINTER(TorjOptions), C.c_double,
+                                            C.c_int32, c_dp]),
     "torj_bundle_device_profile": (c_vp, [c_vp]),
     "torj_bundle_results": (C.c_int, [c_vp, c_dp, c_dp, c_dp, c_dp, c_ip, c_ip, C.POINTER(TorjCounters)]),
     "torj_bundle_trajectories": (C.c_int, [c_vp, c_dp, c_dp, c_dp, c_dp, c_dp]),
@@ -76,6 +78,10 @@ SIGNATURES = {
     "torj_trace": (C.c_int, [c_vp, c_vp, C.POINTER(TorjOptions), C.c_int64, c_dp, c_dp, c_dp, c_dp, c_ip, C.c_int32,
                              C.c_double, C.c_int32, c_dp, C.c_int32, c_ip, c_dp, c_dp, c_dp, c_dp, c_ip, c_ip, C.c_int64, C.c_int64,
                              C.c_int32, c_dp, c_dp, c_dp, c_dp, c_dp, C.POINTER(TorjCounters)]),
+    "torj_trace_plasmas": (C.c_int, [c_vp, C.c_int32, C.POINTER(c_vp), c_ip, C.POINTER(TorjOptions), C.c_int64, c_dp, c_dp, c_dp,
+                                     c_dp, c_ip, C.c_int32, C.c_double, C.c_int32, c_dp, C.c_int32, c_ip, c_dp, c_dp, c_dp, c_dp,
+                                     c_ip, c_ip, C.c_int64, C.c_int64, C.c_int32, c_dp, c_dp, c_dp, c_dp, c_dp,
+                                     C.POINTER(TorjCounters)]),
     "torj_multi_create": (C.c_int, [C.c_int32, C.POINTER(c_vp)]),
     "torj_multi_destroy": (None, [c_vp]),
     "torj_multi_device_count": (C.c_int32, [c_vp]),

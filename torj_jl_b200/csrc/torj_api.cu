@@ -98,12 +98,20 @@ struct torj_bundle {
     int traj_max = 0;
     double *d_ts = nullptr, *d_txyz = nullptr, *d_tP = nullptr, *d_tdP = nullptr, *d_tprof = nullptr;
     int traj_prof_npsi = 0;
-    // what the device copies of psi_edges / dV were computed from (skips the re-upload when unchanged)
+    // what the device copies of psi_edges / dV were computed from (skips the re-upload when unchanged): the edges and the
+    // plasma of every dV row (one row, or one per beam for a plasma set)
     std::vector<double> h_edges;
-    uint64_t edges_plasma = 0;
+    std::vector<uint64_t> dV_plasmas;
     // beams
     int n_beams = 1, prof_rows = 0;
     int* d_beam = nullptr;
+    // plasma set of the last torj_bundle_trace_plasmas (n_plasmas > 1): table bases then DevTables pointers, and the plasma
+    // of every beam, as last uploaded
+    std::vector<const void*> h_set;
+    std::vector<int> h_beam_plasma;
+    const void** d_set = nullptr;
+    int* d_beam_plasma = nullptr;
+    int dV_rows = 1;  // rows of d_dV the last trace used
 };
 
 // Error paths: temporaries are owned by dev_ptr, objects under construction by a guard that destroys them unless the
@@ -580,15 +588,22 @@ static double volume_at(const torj_plasma* p, double x) {
 }
 
 typedef void (*trace_kernel_t)(TraceArgs);
-static trace_kernel_t pick_trace_kernel(int scheme, bool high, int model, int lpr) {
+extern "C++" {  // (inside the extern "C" block)
+template <bool SET>
+static trace_kernel_t pick_trace_kernel_set(int scheme, bool high, int model, int lpr) {
     const bool z3 = scheme == 1;
-    if (model == 1) return lpr == 32 ? (z3 ? k_trace<1, false, 1, 32> : k_trace<0, false, 1, 32>)
-                                     : (z3 ? k_trace<1, false, 1, 1> : k_trace<0, false, 1, 1>);
-    if (lpr == 32) return high ? (z3 ? k_trace<1, true, 0, 32> : k_trace<0, true, 0, 32>) : (z3 ? k_trace<1, false, 0, 32> : k_trace<0, false, 0, 32>);
-    if (lpr == 8) return high ? (z3 ? k_trace<1, true, 0, 8> : k_trace<0, true, 0, 8>) : (z3 ? k_trace<1, false, 0, 8> : k_trace<0, false, 0, 8>);
-    if (lpr == 4) return high ? (z3 ? k_trace<1, true, 0, 4> : k_trace<0, true, 0, 4>) : (z3 ? k_trace<1, false, 0, 4> : k_trace<0, false, 0, 4>);
-    if (lpr == 2) return high ? (z3 ? k_trace<1, true, 0, 2> : k_trace<0, true, 0, 2>) : (z3 ? k_trace<1, false, 0, 2> : k_trace<0, false, 0, 2>);
-    return high ? (z3 ? k_trace<1, true> : k_trace<0, true>) : (z3 ? k_trace<1, false> : k_trace<0, false>);
+    if (model == 1) return lpr == 32 ? (z3 ? k_trace<1, false, 1, 32, SET> : k_trace<0, false, 1, 32, SET>)
+                                     : (z3 ? k_trace<1, false, 1, 1, SET> : k_trace<0, false, 1, 1, SET>);
+    if (lpr == 32) return high ? (z3 ? k_trace<1, true, 0, 32, SET> : k_trace<0, true, 0, 32, SET>) : (z3 ? k_trace<1, false, 0, 32, SET> : k_trace<0, false, 0, 32, SET>);
+    if (lpr == 8) return high ? (z3 ? k_trace<1, true, 0, 8, SET> : k_trace<0, true, 0, 8, SET>) : (z3 ? k_trace<1, false, 0, 8, SET> : k_trace<0, false, 0, 8, SET>);
+    if (lpr == 4) return high ? (z3 ? k_trace<1, true, 0, 4, SET> : k_trace<0, true, 0, 4, SET>) : (z3 ? k_trace<1, false, 0, 4, SET> : k_trace<0, false, 0, 4, SET>);
+    if (lpr == 2) return high ? (z3 ? k_trace<1, true, 0, 2, SET> : k_trace<0, true, 0, 2, SET>) : (z3 ? k_trace<1, false, 0, 2, SET> : k_trace<0, false, 0, 2, SET>);
+    return high ? (z3 ? k_trace<1, true, 0, 1, SET> : k_trace<0, true, 0, 1, SET>) : (z3 ? k_trace<1, false, 0, 1, SET> : k_trace<0, false, 0, 1, SET>);
+}
+}
+// set: the plasma-set instantiations (torj_bundle_trace_plasmas with more than one plasma)
+static trace_kernel_t pick_trace_kernel(int scheme, bool high, int model, int lpr, bool set) {
+    return set ? pick_trace_kernel_set<true>(scheme, high, model, lpr) : pick_trace_kernel_set<false>(scheme, high, model, lpr);
 }
 
 static SolverOpts to_sopts(const torj_options* o, double s_max) {
@@ -833,6 +848,7 @@ void torj_bundle_destroy(torj_bundle* b) {
     cudaFree(b->d_queue); cudaFree(b->d_counters); cudaFree(b->d_edges); cudaFree(b->d_bins); cudaFree(b->d_dV);
     cudaFree(b->d_profile);
     cudaFree(b->d_beam);
+    cudaFree(b->d_set); cudaFree(b->d_beam_plasma);
     cudaFree(b->d_ufinal);
     free_traj(b);
     delete b;
@@ -871,9 +887,50 @@ int torj_bundle_set_beams(torj_bundle* b, int32_t n_beams, const int32_t* beam_i
     return 0;
 }
 
-int torj_bundle_trace(torj_bundle* b, const torj_plasma* p, const torj_options* opt, double s_max, int32_t n_psi,
-                      const double* psi_edges) {
+}  // extern "C"
+
+// The refusals of a plasma set (torj_bundle_trace_plasmas / torj_trace_plasmas); n_beams: the bundle's beams
+static int check_plasma_set(const char* fn, const torj_ctx* c, int32_t n_pl, const torj_plasma* const* pls,
+                            const int32_t* beam_plasma, int n_beams) {
+    char msg[256];
+    if (n_pl < 1) { snprintf(msg, sizeof msg, "%s: n_plasmas must be >= 1", fn); FAIL(msg); }
+    if (!pls) { snprintf(msg, sizeof msg, "%s: plasmas is NULL", fn); FAIL(msg); }
+    for (int k = 0; k < n_pl; ++k) {
+        if (!pls[k]) { snprintf(msg, sizeof msg, "%s: plasmas[%d] is NULL", fn, k); FAIL(msg); }
+        if (pls[k]->ctx->device != c->device) {
+            snprintf(msg, sizeof msg, "%s: plasmas[%d] is on device %d, the bundle's context on device %d", fn, k,
+                     pls[k]->ctx->device, c->device);
+            FAIL(msg);
+        }
+        const DevTables &T0 = pls[0]->T, &T = pls[k]->T;
+        if (T.nR != T0.nR || T.nZ != T0.nZ || T.row != T0.row || memcmp(&T.r0, &T0.r0, sizeof(double)) ||
+            memcmp(&T.z0, &T0.z0, sizeof(double)) || memcmp(&T.inv_hr, &T0.inv_hr, sizeof(double)) ||
+            memcmp(&T.inv_hz, &T0.inv_hz, sizeof(double)) || memcmp(&T.rlast, &T0.rlast, sizeof(double)) ||
+            memcmp(&T.zlast, &T0.zlast, sizeof(double))) {
+            snprintf(msg, sizeof msg, "%s: plasmas[%d] is on another (R,Z) grid than plasmas[0]; a set shares one grid", fn, k);
+            FAIL(msg);
+        }
+    }
+    if (n_pl == 1) return 0;
+    if (n_beams < 2) {
+        snprintf(msg, sizeof msg, "%s: %d plasmas need beams (torj_bundle_set_beams): a profile row belongs to one plasma", fn, n_pl);
+        FAIL(msg);
+    }
+    if (!beam_plasma) { snprintf(msg, sizeof msg, "%s: beam_plasma is NULL", fn); FAIL(msg); }
+    for (int q = 0; q < n_beams; ++q)
+        if (beam_plasma[q] < 0 || beam_plasma[q] >= n_pl) {
+            snprintf(msg, sizeof msg, "%s: beam_plasma[%d] = %d is outside [0, %d)", fn, q, beam_plasma[q], n_pl);
+            FAIL(msg);
+        }
+    return 0;
+}
+
+// torj_bundle_trace (one plasma) and torj_bundle_trace_plasmas: beam q through pls[beam_plasma[q]] when n_pl > 1
+static int bundle_trace(torj_bundle* b, int32_t n_pl, const torj_plasma* const* pls, const int32_t* beam_plasma,
+                        const torj_options* opt, double s_max, int32_t n_psi, const double* psi_edges) {
     torj_ctx* c = b->ctx;
+    const torj_plasma* p = pls[0];  // the set's grid; its tables alone with one plasma
+    const bool set = n_pl > 1;
     if (!c->gl_set) FAIL("The weights and abscissae for the absorption were never initialized. Call `abs_Al_init` before using the absorption.");
     if (n_psi < 2) FAIL("torj_bundle_trace: need at least 2 psi levels");
     for (int j = 1; j < n_psi; ++j) if (!(psi_edges[j] > psi_edges[j - 1])) FAIL("torj_bundle_trace: psi_dP_dV must be strictly increasing");
@@ -906,7 +963,7 @@ int torj_bundle_trace(torj_bundle* b, const torj_plasma* p, const torj_options* 
         b->h_edges.clear();
         CK(cudaMalloc(&b->d_edges, n_psi * sizeof(double)));
         CK(cudaMalloc(&b->d_bins, (size_t)b->n_beams * (n_psi + 2) * sizeof(double)));
-        CK(cudaMalloc(&b->d_dV, n_psi * sizeof(double)));
+        CK(cudaMalloc(&b->d_dV, (size_t)b->n_beams * n_psi * sizeof(double)));  // one row, or one per beam for a plasma set
         CK(cudaMalloc(&b->d_profile, (size_t)b->n_beams * (n_psi + 2) * sizeof(double)));
         b->n_psi = n_psi;
         b->prof_rows = b->n_beams;
@@ -918,15 +975,48 @@ int torj_bundle_trace(torj_bundle* b, const torj_plasma* p, const torj_options* 
         CK(cudaMalloc(&b->d_tprof, (size_t)b->traj_count * n_psi * sizeof(double)));
         b->traj_prof_npsi = n_psi;
     }
-    if (b->edges_plasma != p->id || (int)b->h_edges.size() != n_psi ||
+    const int dV_rows = set ? b->n_beams : 1;
+    std::vector<uint64_t> row_plasma(dV_rows);
+    for (int q = 0; q < dV_rows; ++q) row_plasma[q] = pls[set ? beam_plasma[q] : 0]->id;
+    if (b->dV_plasmas != row_plasma || (int)b->h_edges.size() != n_psi ||
         memcmp(b->h_edges.data(), psi_edges, n_psi * sizeof(double)) != 0) {
-        std::vector<double> dV(n_psi, 1.0);
-        for (int j = 0; j + 1 < n_psi; ++j) dV[j] = volume_at(p, psi_edges[j + 1]) - volume_at(p, psi_edges[j]);
+        std::vector<double> dV((size_t)dV_rows * n_psi, 1.0);
+        for (int q = 0; q < dV_rows; ++q) {
+            const torj_plasma* pq = pls[set ? beam_plasma[q] : 0];
+            for (int j = 0; j + 1 < n_psi; ++j) dV[(size_t)q * n_psi + j] = volume_at(pq, psi_edges[j + 1]) - volume_at(pq, psi_edges[j]);
+        }
         CK(cudaMemcpyAsync(b->d_edges, psi_edges, n_psi * sizeof(double), cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(b->d_dV, dV.data(), n_psi * sizeof(double), cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(b->d_dV, dV.data(), dV.size() * sizeof(double), cudaMemcpyHostToDevice, st));
         CK(cudaStreamSynchronize(st));  // dV is a local; psi_edges belongs to the caller
         b->h_edges.assign(psi_edges, psi_edges + n_psi);
-        b->edges_plasma = p->id;
+        b->dV_plasmas = row_plasma;
+    }
+    b->dV_rows = dV_rows;
+    PlasmaSetDev P{nullptr, nullptr, nullptr, nullptr};
+    if (set) {
+        std::vector<const void*> hs(2 * (size_t)n_pl);
+        for (int k = 0; k < n_pl; ++k) { hs[k] = pls[k]->dA; hs[n_pl + k] = pls[k]->dT; }
+        std::vector<int> hb(beam_plasma, beam_plasma + b->n_beams);
+        if (hs != b->h_set || hb != b->h_beam_plasma) {
+            CK(cudaStreamSynchronize(st));  // an earlier trace may still read them
+            if (hs.size() != b->h_set.size()) {
+                cudaFree(b->d_set);
+                b->d_set = nullptr; b->h_set.clear();
+                CK(cudaMalloc(&b->d_set, hs.size() * sizeof(void*)));
+            }
+            if (hb.size() != b->h_beam_plasma.size()) {
+                cudaFree(b->d_beam_plasma);
+                b->d_beam_plasma = nullptr; b->h_beam_plasma.clear();
+                CK(cudaMalloc(&b->d_beam_plasma, hb.size() * sizeof(int)));
+            }
+            CK(cudaMemcpyAsync(b->d_set, hs.data(), hs.size() * sizeof(void*), cudaMemcpyHostToDevice, st));
+            CK(cudaMemcpyAsync(b->d_beam_plasma, hb.data(), hb.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+            CK(cudaStreamSynchronize(st));  // hs and hb are locals
+            b->h_set = hs; b->h_beam_plasma = hb;
+        }
+        P.A = reinterpret_cast<const double2* const*>(b->d_set);
+        P.T = reinterpret_cast<const DevTables* const*>(b->d_set + n_pl);
+        P.beam_plasma = b->d_beam_plasma; P.beam_id = b->d_beam;
     }
     CK(cudaMemsetAsync(b->d_bins, 0, (size_t)b->n_beams * (n_psi + 2) * sizeof(double), st));
     CK(cudaMemsetAsync(b->d_queue, 0, sizeof(unsigned long long), st));
@@ -934,12 +1024,12 @@ int torj_bundle_trace(torj_bundle* b, const torj_plasma* p, const torj_options* 
     if (b->traj_count > 0) CK(cudaMemsetAsync(b->d_tprof, 0, (size_t)b->traj_count * n_psi * sizeof(double), st));
 
     SolverOpts so = to_sopts(&od, s_max);
-    k_ray_init<<<(unsigned)((b->n + 127) / 128), 128, 0, st>>>(p->T, b->B, so);
+    k_ray_init<<<(unsigned)((b->n + 127) / 128), 128, 0, st>>>(p->T, b->B, so, P);
     c->launches++;
     CK(cudaGetLastError());
 
     TraceArgs a;
-    a.T = p->T; a.B = b->B; a.O = so;
+    a.T = p->T; a.B = b->B; a.O = so; a.P = P;
     a.J.first = b->traj_first; a.J.count = b->traj_count; a.J.max_pts = b->traj_max;
     a.J.s = b->d_ts; a.J.xyz = b->d_txyz; a.J.P = b->d_tP; a.J.dP = b->d_tdP; a.J.prof = b->d_tprof;
     a.n_psi = n_psi; a.n_beams = b->n_beams; a.beam_id = b->d_beam; a.psi_edges = b->d_edges; a.bins = b->d_bins; a.next_ray = b->d_queue; a.counters = b->d_counters;
@@ -973,7 +1063,7 @@ int torj_bundle_trace(torj_bundle* b, const torj_plasma* p, const torj_options* 
     // default kernels do not carry the code
     void (*kern)(TraceArgs);
     const bool high = od.max_harmonic > 3;
-    kern = pick_trace_kernel(od.scheme, high, model, lpr);
+    kern = pick_trace_kernel(od.scheme, high, model, lpr, set);
     CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, kern, TORJ_TPB, smem));
     if (bps < 1) FAIL("torj_bundle_trace: trace kernel does not fit on an SM (n_psi too large for shared memory)");
@@ -1004,7 +1094,8 @@ int torj_bundle_trace(torj_bundle* b, const torj_plasma* p, const torj_options* 
     if (interleave && model == 0 && od.schedule != 3) {
         if (!b->d_life) CK(cudaMalloc(&b->d_life, ((size_t)b->n + 1) * sizeof(int)));
         CK(cudaMemsetAsync(b->d_life + b->n, 0, sizeof(int), st));
-        k_predict_life<<<(unsigned)((b->n + 127) / 128), 128, 0, st>>>(p->T, b->B, so, TORJ_LIFE_HARM_COST, b->d_life, b->d_life + b->n);
+        k_predict_life<<<(unsigned)((b->n + 127) / 128), 128, 0, st>>>(p->T, b->B, so, P, TORJ_LIFE_HARM_COST, b->d_life,
+                                                                      b->d_life + b->n);
         c->launches++;
         CK(cudaGetLastError());
         a.life = b->d_life; a.lmax = b->d_life + b->n;
@@ -1015,10 +1106,24 @@ int torj_bundle_trace(torj_bundle* b, const torj_plasma* p, const torj_options* 
     CK(cudaEventRecord(c->ev1, st));
     c->ev_valid = true;
     k_finalize<<<(unsigned)(((size_t)b->n_beams * (n_psi + 2) + 127) / 128), 128, 0, st>>>(b->d_bins, b->d_dV, n_psi, b->n_beams,
-                                                                                         b->d_profile);
+                                                                                         (int)set, b->d_profile);
     c->launches++;
     CK(cudaGetLastError());
     return 0;
+}
+
+extern "C" {
+
+int torj_bundle_trace(torj_bundle* b, const torj_plasma* p, const torj_options* opt, double s_max, int32_t n_psi,
+                      const double* psi_edges) {
+    return bundle_trace(b, 1, &p, nullptr, opt, s_max, n_psi, psi_edges);
+}
+
+int torj_bundle_trace_plasmas(torj_bundle* b, int32_t n_plasmas, const torj_plasma* const* plasmas, const int32_t* beam_plasma,
+                              const torj_options* opt, double s_max, int32_t n_psi, const double* psi_edges) {
+    if (!b) FAIL("torj_bundle_trace_plasmas: bundle is NULL");
+    if (int rc = check_plasma_set("torj_bundle_trace_plasmas", b->ctx, n_plasmas, plasmas, beam_plasma, b->n_beams)) return rc;
+    return bundle_trace(b, n_plasmas, plasmas, beam_plasma, opt, s_max, n_psi, psi_edges);
 }
 
 void* torj_bundle_device_profile(torj_bundle* b) { return b->d_profile; }
@@ -1065,12 +1170,15 @@ int torj_bundle_trajectories(torj_bundle* b, double* s, double* xyz, double* P, 
     if (dP_dV_ray && b->d_tprof)
         CK(cudaMemcpyAsync(dP_dV_ray, b->d_tprof, (size_t)b->traj_count * b->n_psi * sizeof(double), cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
-    if (dP_dV_ray) {  // shell power -> dP/dV per ray (reference src/plasma.jl:141)
-        std::vector<double> dV(b->n_psi);
-        CK(cudaMemcpy(dV.data(), b->d_dV, b->n_psi * sizeof(double), cudaMemcpyDeviceToHost));
+    if (dP_dV_ray) {  // shell power -> dP/dV per ray (reference src/plasma.jl:141), with the volume of the ray's plasma
+        std::vector<double> dV((size_t)b->dV_rows * b->n_psi);
+        std::vector<int> beam(b->dV_rows > 1 ? b->traj_count : 0);
+        CK(cudaMemcpy(dV.data(), b->d_dV, dV.size() * sizeof(double), cudaMemcpyDeviceToHost));
+        if (!beam.empty()) CK(cudaMemcpy(beam.data(), b->d_beam + b->traj_first, beam.size() * sizeof(int), cudaMemcpyDeviceToHost));
         for (int64_t r = 0; r < b->traj_count; ++r) {
             double* row = dP_dV_ray + (size_t)r * b->n_psi;
-            for (int j = 0; j + 1 < b->n_psi; ++j) row[j] /= dV[j];
+            const double* dVr = dV.data() + (beam.empty() ? 0 : (size_t)beam[r] * b->n_psi);
+            for (int j = 0; j + 1 < b->n_psi; ++j) row[j] /= dVr[j];
             row[b->n_psi - 1] = 0.0;
         }
     }
@@ -1121,13 +1229,16 @@ int torj_bundle_trajectories_cyl(torj_bundle* b, double* R, double* phi, double*
     return 0;
 }
 
-int torj_trace(torj_ctx* c, const torj_plasma* p, const torj_options* opt, int64_t n_rays, const double* pos,
-               const double* dir, const double* weight, const double* freq_hz, const int32_t* mode, int32_t per_ray_fm,
-               double s_max, int32_t n_psi, const double* psi_edges, int32_t n_beams, const int32_t* beam_id, double* dP_dV,
-               double* deposited_power, double* P_final, double* P_dep, int32_t* n_points, int32_t* status, int64_t traj_first,
-               int64_t traj_count,
-               int32_t traj_max_pts, double* traj_s, double* traj_xyz, double* traj_P, double* traj_dP_ds,
-               double* traj_dP_dV_ray, torj_counters* counters) {
+}  // extern "C"
+
+// torj_trace (one plasma) and torj_trace_plasmas
+static int trace_oneshot(torj_ctx* c, int32_t n_pl, const torj_plasma* const* pls, const int32_t* beam_plasma,
+                         const torj_options* opt, int64_t n_rays, const double* pos, const double* dir, const double* weight,
+                         const double* freq_hz, const int32_t* mode, int32_t per_ray_fm, double s_max, int32_t n_psi,
+                         const double* psi_edges, int32_t n_beams, const int32_t* beam_id, double* dP_dV, double* deposited_power,
+                         double* P_final, double* P_dep, int32_t* n_points, int32_t* status, int64_t traj_first, int64_t traj_count,
+                         int32_t traj_max_pts, double* traj_s, double* traj_xyz, double* traj_P, double* traj_dP_ds,
+                         double* traj_dP_dV_ray, torj_counters* counters) {
     // the device workspace of the previous call is reused when the bundle shape is unchanged (no cudaMalloc/cudaFree
     // on the repeated-call path of make_beam scans)
     int rc = 0;
@@ -1148,7 +1259,7 @@ int torj_trace(torj_ctx* c, const torj_plasma* p, const torj_options* opt, int64
     if (traj_count != b->traj_count || traj_first != b->traj_first || (traj_count > 0 && traj_max_pts != b->traj_max))
         rc = torj_bundle_set_window(b, traj_first, traj_count, traj_max_pts);
     if (!rc) rc = torj_bundle_set_beams(b, n_beams, beam_id);
-    if (!rc) rc = torj_bundle_trace(b, p, opt, s_max, n_psi, psi_edges);
+    if (!rc) rc = bundle_trace(b, n_pl, pls, beam_plasma, opt, s_max, n_psi, psi_edges);
     if (!rc) rc = torj_bundle_results(b, dP_dV, deposited_power, P_final, P_dep, n_points, status, counters);
     if (!rc && traj_count > 0) rc = torj_bundle_trajectories(b, traj_s, traj_xyz, traj_P, traj_dP_ds, traj_dP_dV_ray);
     if (rc) {  // do not keep a workspace in an unknown state
@@ -1156,6 +1267,35 @@ int torj_trace(torj_ctx* c, const torj_plasma* p, const torj_options* opt, int64
         c->ws = nullptr;
     }
     return rc;
+}
+
+extern "C" {
+
+int torj_trace(torj_ctx* c, const torj_plasma* p, const torj_options* opt, int64_t n_rays, const double* pos,
+               const double* dir, const double* weight, const double* freq_hz, const int32_t* mode, int32_t per_ray_fm,
+               double s_max, int32_t n_psi, const double* psi_edges, int32_t n_beams, const int32_t* beam_id, double* dP_dV,
+               double* deposited_power, double* P_final, double* P_dep, int32_t* n_points, int32_t* status, int64_t traj_first,
+               int64_t traj_count, int32_t traj_max_pts, double* traj_s, double* traj_xyz, double* traj_P, double* traj_dP_ds,
+               double* traj_dP_dV_ray, torj_counters* counters) {
+    return trace_oneshot(c, 1, &p, nullptr, opt, n_rays, pos, dir, weight, freq_hz, mode, per_ray_fm, s_max, n_psi, psi_edges,
+                         n_beams, beam_id, dP_dV, deposited_power, P_final, P_dep, n_points, status, traj_first, traj_count,
+                         traj_max_pts, traj_s, traj_xyz, traj_P, traj_dP_ds, traj_dP_dV_ray, counters);
+}
+
+int torj_trace_plasmas(torj_ctx* c, int32_t n_plasmas, const torj_plasma* const* plasmas, const int32_t* beam_plasma,
+                       const torj_options* opt, int64_t n_rays, const double* pos, const double* dir, const double* weight,
+                       const double* freq_hz, const int32_t* mode, int32_t per_ray_fm, double s_max, int32_t n_psi,
+                       const double* psi_edges, int32_t n_beams, const int32_t* beam_id, double* dP_dV, double* deposited_power,
+                       double* P_final, double* P_dep, int32_t* n_points, int32_t* status, int64_t traj_first, int64_t traj_count,
+                       int32_t traj_max_pts, double* traj_s, double* traj_xyz, double* traj_P, double* traj_dP_ds,
+                       double* traj_dP_dV_ray, torj_counters* counters) {
+    if (!c) FAIL("torj_trace_plasmas: ctx is NULL");
+    // refused before the workspace is touched; the bundle's beams are those torj_bundle_set_beams will set
+    if (int rc = check_plasma_set("torj_trace_plasmas", c, n_plasmas, plasmas, beam_plasma, (beam_id && n_beams > 1) ? n_beams : 1))
+        return rc;
+    return trace_oneshot(c, n_plasmas, plasmas, beam_plasma, opt, n_rays, pos, dir, weight, freq_hz, mode, per_ray_fm, s_max, n_psi,
+                         psi_edges, n_beams, beam_id, dP_dV, deposited_power, P_final, P_dep, n_points, status, traj_first,
+                         traj_count, traj_max_pts, traj_s, traj_xyz, traj_P, traj_dP_ds, traj_dP_dV_ray, counters);
 }
 
 // ---- single-process multi-GPU front end (what a Julia make_beam on an 8-GPU box calls) -------------------------

@@ -8,6 +8,8 @@
 #include "torj_device.cuh"
 #include "torj_warm.cuh"
 
+#include <type_traits>
+
 namespace torj {
 
 // Runge-Kutta tableaux (OrdinaryDiffEq Tsit5 / OwrenZen3; SURVEY.md A.2), uploaded once per context
@@ -46,6 +48,20 @@ struct TrajDev {
     int max_pts;
     double *s, *xyz, *P, *dP, *prof;  // [count][max], [count][3][max], [count][max], [count][max], [count][n_psi]
 };
+
+// Plasma set (torj_bundle_trace_plasmas): beam b is traced through plasma beam_plasma[b]. Every plasma of a set is on the
+// grid of the DevTables the kernels receive, so a ray's own plasma contributes only its table base and psi_prof_max.
+struct PlasmaSetDev {
+    const double2* const* A;    // [n_plasmas] table base of each plasma; NULL = one plasma, the DevTables passed
+    const DevTables* const* T;  // [n_plasmas] each plasma's DevTables in device memory (ray init, life prediction)
+    const int* beam_plasma;     // [n_beams]
+    const int* beam_id;         // [n_rays]
+};
+
+// the tables of ray i: T0 itself, or with a plasma set those of the ray's plasma (off the hot path: ray init, life prediction)
+__device__ __forceinline__ DevTables ray_tables(const DevTables& T0, const PlasmaSetDev& P, long long i) {
+    return P.T ? *P.T[P.beam_plasma[P.beam_id[i]]] : T0;
+}
 
 // ------------------------------------------------------------------------------------------------
 // ray initialisation
@@ -138,10 +154,11 @@ __device__ inline void refraction_equations(const double N[3], double X, double 
     }
 }
 
-__global__ void k_ray_init(DevTables T, BundleDev B, SolverOpts O) {
+__global__ void k_ray_init(DevTables T0, BundleDev B, SolverOpts O, PlasmaSetDev P) {
     exp_tab_init();
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= B.n_rays) return;
+    const DevTables T = ray_tables(T0, P, i);
     const long long n = B.n_rays;
     double x0[3] = {B.pos[i], B.pos[n + i], B.pos[2 * n + i]};
     double N0[3] = {B.dir[i], B.dir[n + i], B.dir[2 * n + i]};
@@ -281,6 +298,7 @@ struct TraceArgs {
     // start first and all rays END together — no tail of a few long rays running alone. NULL = every ray starts in round 0
     const int* life;                  // [n] predicted cost of every ray in rounds (segments, those inside the absorbing layer weighted)
     const int* lmax;                  // max of life[]
+    PlasmaSetDev P;                   // k_trace<..., SET = true> only (last member: the other instantiations keep their layout)
 };
 #define TORJ_HAND_D 20
 #define TORJ_SEG_RETIRED 0x7fffffff
@@ -398,7 +416,9 @@ __device__ __forceinline__ void stage_sum_unrolled(const double* ks, double dt, 
 //   performs the side effects (bins, per-ray outputs, queue bookkeeping). For bundles below the resident lanes
 //   (37 888), where the time is one ray's latency, for the tail of a large bundle (`resume`), and for the warm model,
 //   whose alpha costs ~100x the rest of the RHS.
-template <int SCH, bool HIGH = false, int MODEL = 0, int LPR = 1>
+// SET = true: a plasma set (a.P). The grid comes from a.T as always; the table base is per lane, bound with the ray
+//   (a ray's plasma is that of its beam), so rays of several equilibria share one launch.
+template <int SCH, bool HIGH = false, int MODEL = 0, int LPR = 1, bool SET = false>
 __global__ void TORJ_TRACE_BOUNDS k_trace(TraceArgs a) {
     exp_tab_init();
     constexpr bool COOP = LPR == 32;
@@ -434,7 +454,7 @@ __global__ void TORJ_TRACE_BOUNDS k_trace(TraceArgs a) {
     if (threadIdx.x < 7) s_bt[threadIdx.x] = c_tab[SCH].bt[threadIdx.x];
     __syncthreads();
 
-    const DevTables T = a.T;
+    std::conditional_t<SET, DevTables, const DevTables> T = a.T;  // SET: T.A is rebound per ray
     const SolverOpts& O = a.O;
     const long long n = a.B.n_rays;
     const unsigned lane = threadIdx.x & 31u;
@@ -541,6 +561,7 @@ __global__ void TORJ_TRACE_BOUNDS k_trace(TraceArgs a) {
         int mode = a.B.per_ray_fm ? a.B.mode[idx] : a.B.mode[0];
         rc = make_ray_const(f, mode, O.te_min, O.max_harmonic, O.alpha_floor);
         if (a.n_beams > 1) beam_bins = a.bins + (size_t)a.beam_id[idx] * (n_psi + 2);
+        if constexpr (SET) T.A = a.P.A[a.P.beam_plasma[a.beam_id[idx]]];
         if (TORJ_FATAL(last_stat)) {  // a dead ray may have left NaN/Inf in the stage slots (0 * NaN != 0)
 #pragma unroll
             for (int j = 0; j < S; ++j)
@@ -1038,13 +1059,14 @@ __global__ void TORJ_TRACE_BOUNDS k_trace(TraceArgs a) {
 // kernel draws 32 consecutive items, and they must be all real or all void — lanes that each skip ahead to their own next
 // real item would end up with rays from all over the bundle, and neighbouring rays on neighbouring lanes is what keeps
 // the stencil loads and the absorbing layer coherent (a random ray order costs 40 %, DESIGN.md §8).
-__global__ void k_predict_life(DevTables T, BundleDev B, SolverOpts O, double harm_cost, int* __restrict__ life,
-                               int* __restrict__ lmax) {
+__global__ void k_predict_life(DevTables T0, BundleDev B, SolverOpts O, PlasmaSetDev P, double harm_cost,
+                               int* __restrict__ life, int* __restrict__ lmax) {
     exp_tab_init();
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;  // blockDim.x is a multiple of 32: warp = ray block
     const long long n = B.n_rays;
     double cost = 1.0;
     if (i < n && B.status[i] == 0) {
+        const DevTables T = ray_tables(T0, P, i);
         const double f = B.per_ray_fm ? B.freq[i] : B.freq[0];
         const int mode = B.per_ray_fm ? B.mode[i] : B.mode[0];
         const RayConst rc = make_ray_const(f, mode, O.te_min, O.max_harmonic, O.alpha_floor);
@@ -1072,11 +1094,13 @@ __global__ void k_predict_life(DevTables T, BundleDev B, SolverOpts O, double ha
     if ((threadIdx.x & 31) == 0) atomicMax(lmax, L);
 }
 
-// dP_dV[j] = bins[j] / (V(psi_{j+1}) - V(psi_j)); last entry 0 (reference src/plasma.jl:103,141)
-__global__ void k_finalize(const double* bins, const double* dV, int n_psi, int n_beams, double* profile) {
+// dP_dV[j] = bins[j] / (V(psi_{j+1}) - V(psi_j)); last entry 0 (reference src/plasma.jl:103,141). dV: one row for all beams,
+// or one row per beam (dV_per_beam: a plasma set, each beam normalised by its own plasma's volume)
+__global__ void k_finalize(const double* bins, const double* dV, int n_psi, int n_beams, int dV_per_beam, double* profile) {
     long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (g >= (long long)n_beams * (n_psi + 2)) return;
     int j = (int)(g % (n_psi + 2));
+    if (dV_per_beam) dV += (g / (n_psi + 2)) * n_psi;
     if (j < n_psi - 1) profile[g] = bins[g] / dV[j];
     else if (j == n_psi - 1) profile[g] = 0.0;
     else profile[g] = bins[g];

@@ -113,6 +113,27 @@ def plasma_from_dd(dd: dict, global_time=None, *, density_scale: float = 1.0, ma
                   a["Br_data"], a["Bz_data"], a["Bphi_data"], a["eqt1d_psi_norm"], a["eqt1d_volume"], build=build)
 
 
+def plasmas_from_dd(dd: dict, times=None, *, density_scale: float = 1.0, matrix_order: str = "auto",
+                    build: str = "host") -> list:
+    """One Plasma per equilibrium time slice — every slice (times=None) or the slice valid at each of `times` under the
+    causal lookup — each with the core_profiles slice valid at that slice's time: the plasma set of
+    trace_bundle / make_beams / make_beam_series. Raises ValueError when the slices' 2-D grids differ (a set shares one
+    (R,Z) grid; resample the equilibria first)."""
+    eq = dd["equilibrium"]
+    if times is None:
+        times = _times(eq, eq["time_slice"]) if eq["time_slice"] else []
+    times = [float(t) for t in np.atleast_1d(times)]
+    if not times:
+        raise ValueError("no time slices")
+    arrs = [plasma_arrays_from_dd(dd, t, density_scale=density_scale, matrix_order=matrix_order) for t in times]
+    for t, a in zip(times, arrs):
+        if not (np.array_equal(a["R_coords"], arrs[0]["R_coords"]) and np.array_equal(a["Z_coords"], arrs[0]["Z_coords"])):
+            raise ValueError(f"the (R,Z) grid of the slice at t = {t} differs from that at t = {times[0]}: "
+                             "a plasma set shares one grid")
+    return [Plasma(a["R_coords"], a["Z_coords"], a["psi_norm_data"], a["psi_prof"], a["ne_prof"], a["Te_prof"], a["Br_data"],
+                   a["Bz_data"], a["Bphi_data"], a["eqt1d_psi_norm"], a["eqt1d_volume"], build=build) for a in arrs]
+
+
 def plasma_from_imas_json(path: str, global_time=None, **kw) -> Plasma:
     """test/tests/setup.jl:31-55 in one call."""
     return plasma_from_dd(load_imas_json(path), global_time, **kw)

@@ -24,9 +24,11 @@ def _p(a):
     return a.ctypes.data_as(c_dp)
 
 
-def marshal_bundle(ray_positions, ray_directions, ray_weights, f, mode, psi_dP_dV, beam_id, n_beams):
+def marshal_bundle(ray_positions, ray_directions, ray_weights, f, mode, psi_dP_dV, beam_id, n_beams, *, n_plasmas=1,
+                   beam_plasma=None):
     """The host buffers torj_trace / torj_multi_trace take: component-major [3][n] rays (a Julia Matrix[n,3] as is),
-    per-ray or scalar frequency / mode, psi levels, beam ids, and the result arrays."""
+    per-ray or scalar frequency / mode, psi levels, beam ids, and the result arrays. With a plasma set (torj_trace_plasmas)
+    also the plasma of every beam, beam_plasma[n_beams] in [0, n_plasmas)."""
     pos = np.ascontiguousarray(np.asarray(ray_positions, dtype=np.float64).T)
     dr = np.ascontiguousarray(np.asarray(ray_directions, dtype=np.float64).T)
     n = pos.shape[1]
@@ -39,9 +41,29 @@ def marshal_bundle(ray_positions, ray_directions, ray_weights, f, mode, psi_dP_d
     bid = np.ascontiguousarray(beam_id, dtype=np.int32) if beam_id is not None else None
     if bid is not None and bid.shape != (n,):
         raise ValueError("beam_id must have one entry per ray")
+    bp = None
+    if beam_plasma is not None:
+        bp = np.ascontiguousarray(beam_plasma, dtype=np.int32)
+        if bp.shape != (n_beams,):
+            raise ValueError(f"beam_plasma must have one entry per beam (n_beams = {n_beams}), got shape {bp.shape}")
+        if bp.min() < 0 or bp.max() >= n_plasmas:
+            raise ValueError(f"beam_plasma must lie in [0, {n_plasmas}) (one index into the plasmas per beam)")
+        if n_plasmas > 1 and n_beams < 2:
+            raise ValueError("several plasmas need several beams (beam_id, n_beams): a profile row belongs to one plasma")
     out = dict(prof=np.zeros((n_beams, len(psi))), dep=np.zeros(n_beams), Pf=np.zeros(n), Pd=np.zeros(n),
                npts=np.zeros(n, dtype=np.int32), st=np.zeros(n, dtype=np.int32), cnt=_lib.TorjCounters())
-    return dict(pos=pos, dir=dr, n=n, w=wt, per_ray=per_ray, f=fr, mode=md, psi=psi, n_beams=n_beams, beam=bid, out=out)
+    return dict(pos=pos, dir=dr, n=n, w=wt, per_ray=per_ray, f=fr, mode=md, psi=psi, n_beams=n_beams, beam=bid,
+                beam_plasma=bp, out=out)
+
+
+def _plasma_list(plasma):
+    """trace_bundle's plasma argument: a Plasma (None returned) or a non-empty sequence of them."""
+    if isinstance(plasma, Plasma):
+        return None
+    pls = list(plasma)
+    if not pls or not all(isinstance(p, Plasma) for p in pls):
+        raise TypeError("plasma must be a Plasma or a non-empty sequence of Plasma")
+    return pls
 
 
 def bundle_result(m):
@@ -50,13 +72,21 @@ def bundle_result(m):
                 P_final=o["Pf"], P_deposited_ray=o["Pd"], n_points=o["npts"], status=o["st"], counters=o["cnt"].as_dict())
 
 
-def trace_bundle(plasma: Plasma, ray_positions, ray_directions, ray_weights, f, mode, s_max, psi_dP_dV, *,
-                 options=None, ctx=None, trajectories=None, traj_max_pts=None, beam_id=None, n_beams=1):
+def trace_bundle(plasma, ray_positions, ray_directions, ray_weights, f, mode, s_max, psi_dP_dV, *,
+                 options=None, ctx=None, trajectories=None, traj_max_pts=None, beam_id=None, n_beams=1, beam_plasma=None):
     """One torj_trace call on host buffers. trajectories: None or (first, count).
-    beam_id/n_beams: rays of several beams in one bundle -> dP_dV[n_beams, n_psi], deposited_power[n_beams]."""
+    beam_id/n_beams: rays of several beams in one bundle -> dP_dV[n_beams, n_psi], deposited_power[n_beams].
+    plasma: a Plasma, or a sequence of Plasma on one (R,Z) grid with beam_plasma[n_beams] naming the plasma of every beam
+    (torj_trace_plasmas; keep each beam's rays contiguous)."""
+    pls = _plasma_list(plasma)
+    if pls is None and beam_plasma is not None:
+        raise ValueError("beam_plasma needs a sequence of plasmas")
+    if pls is not None and beam_plasma is None:
+        raise ValueError("a sequence of plasmas needs beam_plasma (the plasma of every beam)")
+    m = marshal_bundle(ray_positions, ray_directions, ray_weights, f, mode, psi_dP_dV, beam_id, n_beams,
+                       n_plasmas=len(pls) if pls else 1, beam_plasma=beam_plasma)
     ctx = ctx or _lib.context()
     L = _lib.lib()
-    m = marshal_bundle(ray_positions, ray_directions, ray_weights, f, mode, psi_dP_dV, beam_id, n_beams)
     n, psi, o = m["n"], m["psi"], m["out"]
     opt = options or _lib.default_options()
     t_first, t_count = trajectories if trajectories else (0, 0)
@@ -65,11 +95,15 @@ def trace_bundle(plasma: Plasma, ray_positions, ray_directions, ray_weights, f, 
     tm = int(traj_max_pts or 0)
     ts = np.zeros((t_count, tm)); txyz = np.zeros((t_count, 3, tm)); tP = np.zeros((t_count, tm))
     tdP = np.zeros((t_count, tm)); tprof = np.zeros((t_count, len(psi)))
-    _lib.check(L.torj_trace(ctx, plasma.handle(ctx), C.byref(opt), n, _p(m["pos"]), _p(m["dir"]), _p(m["w"]), _p(m["f"]),
-                            m["mode"].ctypes.data_as(c_ip), m["per_ray"], float(s_max), len(psi), _p(psi), m["n_beams"],
-                            m["beam"].ctypes.data_as(c_ip) if m["beam"] is not None else None, _p(o["prof"]), _p(o["dep"]),
-                            _p(o["Pf"]), _p(o["Pd"]), o["npts"].ctypes.data_as(c_ip), o["st"].ctypes.data_as(c_ip), t_first,
-                            t_count, tm, _p(ts), _p(txyz), _p(tP), _p(tdP), _p(tprof), C.byref(o["cnt"])))
+    rest = (C.byref(opt), n, _p(m["pos"]), _p(m["dir"]), _p(m["w"]), _p(m["f"]), m["mode"].ctypes.data_as(c_ip), m["per_ray"],
+            float(s_max), len(psi), _p(psi), m["n_beams"], m["beam"].ctypes.data_as(c_ip) if m["beam"] is not None else None,
+            _p(o["prof"]), _p(o["dep"]), _p(o["Pf"]), _p(o["Pd"]), o["npts"].ctypes.data_as(c_ip), o["st"].ctypes.data_as(c_ip),
+            t_first, t_count, tm, _p(ts), _p(txyz), _p(tP), _p(tdP), _p(tprof), C.byref(o["cnt"]))
+    if pls is None:
+        _lib.check(L.torj_trace(ctx, plasma.handle(ctx), *rest))
+    else:
+        hs = (_lib.c_vp * len(pls))(*[p.handle(ctx).value for p in pls])
+        _lib.check(L.torj_trace_plasmas(ctx, len(pls), hs, m["beam_plasma"].ctypes.data_as(c_ip), *rest))
     res = bundle_result(m)
     res.update(traj_s=ts, traj_xyz=txyz, traj_P=tP, traj_dP_ds=tdP, traj_dP_dV_ray=tprof)
     return res
@@ -119,10 +153,27 @@ def make_beam(plasma: Plasma, r, phi, z, steering_angle_tor, steering_angle_pol,
     return arc, traj, powers, res["dP_dV"], res["deposited_power"], wts
 
 
+def _launcher_plasmas(plasma, launchers):
+    """(plasmas or None, beam_plasma or None) of make_beams: a launcher's optional "plasma" key indexes a sequence of plasmas."""
+    pls = _plasma_list(plasma)
+    idx = [q.get("plasma", 0) for q in launchers]
+    if pls is None:
+        if any(i != 0 for i in idx):
+            raise ValueError('a launcher names a "plasma" but make_beams got a single Plasma')
+        return None, None
+    bp = np.asarray(idx, dtype=np.int32)
+    if bp.min() < 0 or bp.max() >= len(pls):
+        raise ValueError(f'launcher "plasma" must lie in [0, {len(pls)})')
+    return pls, bp
+
+
 def _make_beams_device(plasma, launchers, s_max, psi_dP_dV, options, ctx, N_rings=3, min_azimuthal_points=5,
                        normalize_weight_sum=True):
     """Rays generated on the GPU (torj_bundle_create_from_launchers), traced and reduced there; only launcher
     parameters go in and profiles / per-ray scalars come out."""
+    pls, bp = _launcher_plasmas(plasma, launchers)
+    if pls is not None and len(pls) > 1 and len(launchers) < 2:
+        raise ValueError("several plasmas need several launchers: a profile row belongs to one plasma")
     ctx = ctx or _lib.context()
     L = _lib.lib()
     if N_rings < 2:
@@ -144,7 +195,12 @@ def _make_beams_device(plasma, launchers, s_max, psi_dP_dV, options, ctx, N_ring
         n = int(n.value)
         psi = np.ascontiguousarray(psi_dP_dV, dtype=np.float64)
         opt = options or _lib.default_options()
-        _lib.check(L.torj_bundle_trace(bh, plasma.handle(ctx), C.byref(opt), float(s_max), len(psi), _p(psi)))
+        if pls is None:
+            _lib.check(L.torj_bundle_trace(bh, plasma.handle(ctx), C.byref(opt), float(s_max), len(psi), _p(psi)))
+        else:
+            hs = (_lib.c_vp * len(pls))(*[p.handle(ctx).value for p in pls])
+            _lib.check(L.torj_bundle_trace_plasmas(bh, len(pls), hs, bp.ctypes.data_as(c_ip), C.byref(opt), float(s_max),
+                                                   len(psi), _p(psi)))
         prof = np.zeros((nl, len(psi))); dep = np.zeros(nl)
         Pf = np.zeros(n); Pd = np.zeros(n); npts = np.zeros(n, dtype=np.int32); st = np.zeros(n, dtype=np.int32)
         cnt = _lib.TorjCounters()
@@ -160,13 +216,16 @@ def _make_beams_device(plasma, launchers, s_max, psi_dP_dV, options, ctx, N_ring
     return prof, dep, [wt[i * per:(i + 1) * per] for i in range(nl)], [Pf[i * per:(i + 1) * per] for i in range(nl)], res
 
 
-def make_beams(plasma: Plasma, launchers, s_max, psi_dP_dV, *, options=None, ctx=None, device_launch=False, **kwargs):
+def make_beams(plasma, launchers, s_max, psi_dP_dV, *, options=None, ctx=None, device_launch=False, **kwargs):
     """Batched make_beam for scans: `launchers` is a sequence of dicts with the positional arguments of make_beam
     (r, phi, z, steering_angle_tor, steering_angle_pol, spot_size, inverse_curvature_radius, f, mode). All beams are
     traced in ONE device call; returns (dP_dV[n_beams, n_psi], deposited_power[n_beams], ray_weights per beam,
-    P_final per beam). Equivalent to a host loop over make_beam (reference src/solve.jl:209-242) without trajectories."""
+    P_final per beam). Equivalent to a host loop over make_beam (reference src/solve.jl:209-242) without trajectories.
+    `plasma` may be a sequence of Plasma on one (R,Z) grid: a launcher's "plasma" key (default 0) picks the one its beam
+    is traced through, and its profile row is normalised by that plasma's volume."""
     if device_launch:
         return _make_beams_device(plasma, launchers, s_max, psi_dP_dV, options, ctx, **kwargs)
+    pls, bp = _launcher_plasmas(plasma, launchers)
     P, D, W, F, M, B = [], [], [], [], [], []
     for b, L in enumerate(launchers):
         N0 = pol_tor_angles_2_vector(L["steering_angle_pol"], L["steering_angle_tor"])
@@ -175,8 +234,31 @@ def make_beams(plasma: Plasma, launchers, s_max, psi_dP_dV, *, options=None, ctx
         P.append(p); D.append(d); W.append(w)
         F.append(np.full(len(w), float(L["f"]))); M.append(np.full(len(w), int(L["mode"]), dtype=np.int32))
         B.append(np.full(len(w), b, dtype=np.int32))
-    res = trace_bundle(plasma, np.concatenate(P), np.concatenate(D), np.concatenate(W), np.concatenate(F), np.concatenate(M),
-                       s_max, psi_dP_dV, options=options, ctx=ctx, beam_id=np.concatenate(B), n_beams=len(launchers))
+    res = trace_bundle(pls if pls is not None else plasma, np.concatenate(P), np.concatenate(D), np.concatenate(W),
+                       np.concatenate(F), np.concatenate(M), s_max, psi_dP_dV, options=options, ctx=ctx,
+                       beam_id=np.concatenate(B), n_beams=len(launchers), beam_plasma=bp)
     off = np.cumsum([0] + [len(w) for w in W])
     dP = np.atleast_2d(res["dP_dV"]); dep = np.atleast_1d(res["deposited_power"])
     return dP, dep, W, [res["P_final"][off[i]:off[i + 1]] for i in range(len(W))], res
+
+
+def make_beam_series(plasmas, r, phi, z, steering_angle_tor, steering_angle_pol, spot_size, inverse_curvature_radius,
+                     f, mode, s_max, psi_dP_dV, *, options=None, ctx=None, trajectories=None, **kwargs):
+    """The reference's make_beam (src/solve.jl:209-242) of one launcher on each plasma of a sequence on one (R,Z) grid
+    (time slices, an uncertainty ensemble), in ONE device call (torj_trace_plasmas). The beam's rays go in once per
+    plasma, contiguous. Returns (dP_dV[n_plasmas, n_psi], deposited_power[n_plasmas], ray_weights, P_final[n_plasmas, n],
+    res) where res holds the per-ray arrays over the whole bundle (plasma k's rays at [k n, (k+1) n)). No trajectories
+    unless `trajectories` = (first, count) over that bundle: the window would otherwise hold n_plasmas beams."""
+    pls = _plasma_list(plasmas)
+    if pls is None:
+        pls = [plasmas]
+    K = len(pls)
+    N0 = pol_tor_angles_2_vector(steering_angle_pol, steering_angle_tor)
+    x0 = np.array([r * np.cos(phi), r * np.sin(phi), z])
+    pos, dirs, wts = launch_peripheral_rays(x0, N0, spot_size, inverse_curvature_radius, f, **kwargs)
+    n = len(wts)
+    res = trace_bundle(pls, np.tile(pos, (K, 1)), np.tile(dirs, (K, 1)), np.tile(wts, K), float(f), int(mode), s_max,
+                       psi_dP_dV, options=options, ctx=ctx, trajectories=trajectories,
+                       beam_id=np.repeat(np.arange(K, dtype=np.int32), n) if K > 1 else None, n_beams=K,
+                       beam_plasma=np.arange(K, dtype=np.int32))
+    return (np.atleast_2d(res["dP_dV"]), np.atleast_1d(res["deposited_power"]), wts, res["P_final"].reshape(K, n), res)
