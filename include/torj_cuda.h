@@ -48,7 +48,8 @@ enum {
 typedef struct torj_options {
     int32_t scheme;                /* 0 = Tsit5: what `solve(prob)` runs, the `OwrenZen3()` at src/solve.jl:156 being
                                       passed as the parameter object; 1 = OwrenZen3 (the scheme the source names) */
-    int32_t n_segments;            /* 100   src/solve.jl:145 */
+    int32_t n_segments;            /* 100   src/solve.jl:145; >= 1. The segment hand-off (schedule 2 / 3) takes at most 16000:
+                                      above that, schedule 0 traces whole rays and schedules 2 and 3 are refused */
     double dtmax;                  /* 1e-4  src/solve.jl:157 */
     double abstol;                 /* 1e-6  src/solve.jl:157 */
     double reltol;                 /* 1e-6  src/solve.jl:157 */
@@ -72,7 +73,8 @@ typedef struct torj_options {
                                       life-ordered: a pilot march (straight line, real fields and alpha, one point per
                                       segment) predicts every ray's life and the long-lived rays start first, so that all
                                       rays end together instead of the longest ones finishing alone;
-                                      3 = plain segment hand-off: every ray starts in round 0 */
+                                      3 = plain segment hand-off: every ray starts in round 0.
+                                      The hand-off needs n_segments <= 16000 (see n_segments) */
     int32_t absorption_model;      /* 0 = Albajar (reference src/absorption.jl:191-235, what the reference's gradΛ! calls);
                                       1 = warm-plasma damping: alpha = α(ω, X, Y, |N|, acos(N∥/|N|), Te, v_g_perp, mode)[2] of
                                       reference src/general_absorption.jl:1328-1337 (iwarm = 3, Larmor order lrm <= 5) in the

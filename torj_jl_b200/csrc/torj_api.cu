@@ -938,12 +938,14 @@ static int bundle_trace(torj_bundle* b, int32_t n_pl, const torj_plasma* const* 
     torj_options_default(&od);
     if (opt) od = *opt;
     if (od.scheme != 0 && od.scheme != 1) FAIL("torj_bundle_trace: scheme must be 0 (Tsit5) or 1 (OwrenZen3)");
-    if (od.n_segments < 1 || od.n_segments > 16000) FAIL("torj_bundle_trace: n_segments must be in 1..16000");
+    if (od.n_segments < 1) FAIL("torj_bundle_trace: n_segments must be >= 1");
     if (!(od.alpha_floor >= 0.0)) FAIL("torj_bundle_trace: alpha_floor must be >= 0");
     if (od.max_harmonic < 1 || od.max_harmonic > 16) FAIL("torj_bundle_trace: max_harmonic must be in 1..16 (1 = no absorption)");
     if (!(od.dtmax > 0.0) || !(od.abstol > 0.0) || !(od.reltol > 0.0)) FAIL("torj_bundle_trace: dtmax, abstol and reltol must be > 0");
     if (od.schedule < 0 || od.schedule > 3)
         FAIL("torj_bundle_trace: schedule must be 0 (automatic), 1 (whole rays), 2 (segment hand-off) or 3 (hand-off without tail stages)");
+    if ((od.schedule == 2 || od.schedule == 3) && od.n_segments > TORJ_SEG_MAX)
+        FAIL("torj_bundle_trace: the segment hand-off (schedule 2 or 3) takes n_segments <= 16000; schedules 0 and 1 trace whole rays above that");
     if (od.max_steps_per_segment < 1) FAIL("torj_bundle_trace: max_steps_per_segment < 1");
     if (od.absorption_model != 0 && od.absorption_model != 1) FAIL("torj_bundle_trace: absorption_model must be 0 (Albajar) or 1 (warm)");
     if (od.lanes_per_ray != 0 && od.lanes_per_ray != 1 && od.lanes_per_ray != 2 && od.lanes_per_ray != 4 && od.lanes_per_ray != 8 &&
@@ -1074,7 +1076,7 @@ static int bundle_trace(torj_bundle* b, int32_t n_pl, const torj_plasma* const* 
     // absorption coefficient on every trip (measured 3.1 s -> 2.4 s). Below one wave there is nothing to balance.
     const int64_t lanes = (int64_t)c->num_sms * bps * TORJ_TPB / lpr;  // rays in flight
     int interleave = od.schedule == 2 || od.schedule == 3 || (od.schedule == 0 && b->n > lanes);
-    if (od.n_segments < 2 || b->n > 0x7fffffff) interleave = 0;
+    if (od.n_segments < 2 || od.n_segments > TORJ_SEG_MAX || b->n > 0x7fffffff) interleave = 0;  // TORJ_SEG_MAX: the hand-off word's 15-bit fields
     a.interleave = interleave; a.hand = nullptr; a.seg_done = nullptr; a.rays_left = nullptr;
     if (interleave) {
         if (!b->d_hand) CK(cudaMalloc(&b->d_hand, (size_t)b->n * TORJ_HAND_D * sizeof(double)));

@@ -7,6 +7,7 @@
 #pragma once
 #include "torj_device.cuh"
 #include "torj_warm.cuh"
+#include "torj_handoff.cuh"
 
 #include <type_traits>
 
@@ -288,9 +289,8 @@ struct TraceArgs {
     // segments, so all rays advance together and the bundle ends after n/lanes ray-times instead of ceil(n/lanes)
     int interleave;
     double* hand;                     // [n][TORJ_HAND_D] ray state between two segments
-    int* seg_done;                    // [n] bits 0-14: segments completed, bits 15-29: 1 + the highest segment whose work item
-                                      // was drawn before it could start and therefore dropped (its holder continues
-                                      // instead); TORJ_SEG_RETIRED once the ray has ended
+    int* seg_done;                    // [n] the ray's hand-off word: segments completed, dropped items, whether a lane holds
+                                      // the ray, or TORJ_SEG_RETIRED (layout and transitions in torj_handoff.cuh)
     int* rays_left;                   // rays not yet retired
     const double2* warm_tab;          // [501] (t_i, exp(-t_i^2) dt): set_extv! tables of the warm-plasma model
     double* u_final;                  // [7][n] state of every ray at retirement, or NULL
@@ -301,9 +301,6 @@ struct TraceArgs {
     PlasmaSetDev P;                   // k_trace<..., SET = true> only (last member: the other instantiations keep their layout)
 };
 #define TORJ_HAND_D 20
-#define TORJ_SEG_RETIRED 0x7fffffff
-#define TORJ_SEG_DONE(w) ((w) & 0x7fff)
-#define TORJ_SEG_DROP(w) (((w) >> 15) & 0x7fff)
 
 __device__ __forceinline__ double eps_of(double x) {  // Julia eps(x)
     x = fabs(x);
@@ -633,20 +630,21 @@ __global__ void TORJ_TRACE_BOUNDS k_trace(TraceArgs a) {
     };
     // A freshly drawn item (ray idx, segment wseg). Nobody ever waits for an unfinished predecessor: if the ray's previous
     // segment is still running, the item is DROPPED and marked as such in the ray's word, and the lane that runs that segment
-    // finds the mark when it hands in and continues with the ray itself (ACT_END_SEGMENT). Both sides use one atomic on
-    // the same word, so exactly one of them runs the segment. (Idle lanes that ran ahead in the queue used to hold such
-    // items and block; with life-ordered rounds that would idle most lanes while the long rays start.)
+    // finds the mark when it hands in and continues with the ray itself (ACT_END_SEGMENT). A ready claim sets the word's
+    // RUNNING bit, and a claim that finds it set is void: the holder already continues with that segment. Claims and
+    // hand-ins change the word only through the transitions of torj_handoff.cuh, each in one compare-and-swap, so exactly
+    // one lane runs every segment. (Idle lanes that ran ahead in the queue used to hold such items and block; with
+    // life-ordered rounds that would idle most lanes while the long rays start.)
     auto claim = [&](long long idx, bool aligned) {
         ray = idx;
         int verdict = 0;  // 0 void, 1 ready
         if (writer) {
-            int w = atomicAdd(&a.seg_done[idx], 0);
+            int w = wseg;  // first guess: ready, nothing dropped (the usual case, then one CAS); a wrong guess reads the word
             for (;;) {
-                if (w == TORJ_SEG_RETIRED || TORJ_SEG_DONE(w) > wseg) break;  // retired / already run by its previous holder
-                if (TORJ_SEG_DONE(w) == wseg) { verdict = 1; break; }
-                const int drop = max(TORJ_SEG_DROP(w), wseg + 1);
-                const int old = atomicCAS(&a.seg_done[idx], w, TORJ_SEG_DONE(w) | (drop << 15));
-                if (old == w) break;  // dropped: the holder of the running segment will see the mark
+                const TorjSegMove m = torj_seg_claim(w, wseg);
+                if (m.w == w) break;  // void with nothing to mark: retired, already run, held, or already dropped
+                const int old = atomicCAS(&a.seg_done[idx], w, m.w);
+                if (old == w) { verdict = m.go; break; }
                 w = old;
             }
         }
@@ -970,11 +968,21 @@ __global__ void TORJ_TRACE_BOUNDS k_trace(TraceArgs a) {
                 } else if (a.interleave) {
                     // hand the segment in. The next one is a separate work item, usually taken by another lane — unless that
                     // item was drawn while this segment was still running and dropped (claim): then this lane keeps the ray
+                    // (the word is read before save_ray's stores and fence, which hide the load; a stale value costs one
+                    // more round, the CAS checks it)
+                    int w = writer ? __ldcg(&a.seg_done[ray]) : 0;
                     save_ray();
-                    int old = 0;
-                    if (writer) old = atomicAdd(&a.seg_done[ray], 1);
-                    if (LPR > 1) old = __shfl_sync(gmask, old, gleader);
-                    if (TORJ_SEG_DROP(old) >= seg + 1) {
+                    int go = 0;
+                    if (writer) {
+                        for (;;) {
+                            const TorjSegMove m = torj_seg_hand_in(w, seg);
+                            const int old = atomicCAS(&a.seg_done[ray], w, m.w);
+                            if (old == w) { go = m.go; break; }
+                            w = old;
+                        }
+                    }
+                    if (LPR > 1) go = __shfl_sync(gmask, go, gleader);
+                    if (go) {
                         wseg = seg;
                         own = true;
                         phase = PH_WAIT;  // next segment on the warp's next aligned trip
