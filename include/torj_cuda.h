@@ -257,9 +257,11 @@ int torj_multi_create(int32_t n_devices /* <= 0: all visible */, torj_multi** ou
 void torj_multi_destroy(torj_multi* m);
 int32_t torj_multi_device_count(const torj_multi* m);
 int torj_multi_configure(torj_multi* m, int32_t sharding, int64_t block_rays, int32_t reduction);
-/* 1 when the cross-device sum of the last torj_multi_trace went through ncclAllReduce, 0 for the host sum */
+/* 1 when the cross-device sum of the last torj_multi_trace(_plasmas) went through ncclAllReduce, 0 for the host sum */
 int32_t torj_multi_used_nccl(const torj_multi* m);
 int torj_multi_abs_init(torj_multi* m, int32_t n, const double* nodes, const double* weights);
+/* torj_ctx_last_trace_ms of device d's context: the k_trace time of its part of the last torj_multi_trace(_plasmas) */
+int torj_multi_last_trace_ms(torj_multi* m, int32_t device, double* ms);
 int torj_multi_plasma_create_from_data(torj_multi* m, const torj_grid* grid, const double* psi_norm, const double* psi_prof,
                                        const double* ne_prof, const double* Te_prof, int32_t n_prof, const double* BR,
                                        const double* BZ, const double* Bphi, const double* psi_1d, const double* vol_1d,
@@ -271,6 +273,21 @@ int torj_multi_trace(torj_multi* m, const torj_mplasma* mp, const torj_options* 
                      double* dP_dV, double* deposited_power, double* P_final, double* P_deposited_ray, int32_t* n_points,
                      int32_t* status, int64_t traj_first, int64_t traj_count, int32_t traj_max_pts, double* traj_s,
                      double* traj_xyz, double* traj_P, double* traj_dP_ds, double* traj_dP_dV_ray, torj_counters* counters);
+/* torj_multi_trace through a plasma set (torj_trace_plasmas sharded over the devices): beam b of beam_id is traced through
+ * plasmas[beam_plasma[b]] on whichever device holds its rays; device d traces through the copies {plasmas[k] on d}. Each
+ * device's profile rows are already divided by their beam's plasma volume, so the one all-reduce (or host sum) of
+ * n_beams * (n_psi + 2) doubles is the set's profile; a device holds zero rows for the beams it did not trace.
+ * Block-cyclic sharding with block_rays = rays per beam deals whole beams. Refused before anything is enqueued (non-zero,
+ * torj_last_error, every device's workspace left as it was): the refusals of torj_trace_plasmas on every device, and a
+ * plasma created by another torj_multi. n_plasmas = 1 is torj_multi_trace (beam_plasma unused). */
+int torj_multi_trace_plasmas(torj_multi* m, int32_t n_plasmas, const torj_mplasma* const* plasmas,
+                             const int32_t* beam_plasma /* [n_beams] */, const torj_options* opt, int64_t n_rays,
+                             const double* pos, const double* dir, const double* weight, const double* freq_hz,
+                             const int32_t* mode, int32_t per_ray_fm, double s_max, int32_t n_psi, const double* psi_edges,
+                             int32_t n_beams, const int32_t* beam_id, double* dP_dV, double* deposited_power, double* P_final,
+                             double* P_deposited_ray, int32_t* n_points, int32_t* status, int64_t traj_first,
+                             int64_t traj_count, int32_t traj_max_pts, double* traj_s, double* traj_xyz, double* traj_P,
+                             double* traj_dP_ds, double* traj_dP_dV_ray, torj_counters* counters);
 
 /* --- measurement ------------------------------------------------------------------------------------------- */
 /* Register-resident DFMA-chain microbenchmark: the FP64 roofline denominator (MEASURED_PEAKS.json has none). */

@@ -177,7 +177,56 @@ const _multi = Ref{Ptr{Cvoid}}(C_NULL)
 function torj_multi()
     if _multi[] == C_NULL
         torj_check(ccall((:torj_multi_create, libtorj), Cint, (Int32, Ref{Ptr{Cvoid}}), 0, _multi))
-        atexit(() -> ccall((:torj_multi_destroy, libtorj), Cvoid, (Ptr{Cvoid},), _multi[]))
+        atexit() do  # the per-device copies of the plasmas first: they live on the contexts of the torj_multi
+            foreach(h -> ccall((:torj_multi_plasma_destroy, libtorj), Cvoid, (Ptr{Cvoid},), h), _mplasmas)
+            empty!(_mplasmas)
+            ccall((:torj_multi_destroy, libtorj), Cvoid, (Ptr{Cvoid},), _multi[])
+        end
     end
     _multi[]
+end
+
+# torj_mplasma: one plasma's tables on every device of torj_multi(), built there from the arrays of the Plasma constructor
+# (src/plasma.jl:30-32: 2-D arrays [nR, nZ], profiles and the 1-D volume; route (b) above). Kept until the process exits.
+const _mplasmas = Ptr{Cvoid}[]
+function torj_mplasma(R, Z, psi_norm, psi_prof, ne, Te, BR, BZ, Bphi, psi1d, vol1d)
+    m = torj_multi()
+    g = TorjGrid(length(R), length(Z), R[1], R[end], Z[1], Z[end])
+    h = Ref{Ptr{Cvoid}}(C_NULL)
+    torj_check(ccall((:torj_multi_plasma_create_from_data, libtorj), Cint,
+        (Ptr{Cvoid}, Ref{TorjGrid}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Int32, Ptr{Float64}, Ptr{Float64},
+         Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Int32, Ref{Ptr{Cvoid}}),
+        m, g, Matrix{Float64}(psi_norm), Vector{Float64}(psi_prof), Vector{Float64}(ne), Vector{Float64}(Te), length(psi_prof),
+        Matrix{Float64}(BR), Matrix{Float64}(BZ), Matrix{Float64}(Bphi), Vector{Float64}(psi1d), Vector{Float64}(vol1d),
+        length(psi1d), h))
+    push!(_mplasmas, h[])
+    h[]
+end
+
+# make_beam_series on every GPU (torj_multi_trace_plasmas): the same call and result as make_beam_series above, with
+# torj_mplasma handles for the plasmas. The beam on each plasma is a whole block of n rays, and block-cyclic sharding with
+# block_rays = n deals whole plasmas round-robin over the devices; contiguous sharding is restored afterwards.
+function multi_make_beam_series(mplasmas::Vector{Ptr{Cvoid}}, r, phi, z, tor, pol, spot, invRc, f, mode::Integer,
+                                s_max::Float64, psi_dP_dV; options=torj_options(), kwargs...)
+    N0 = collect(IMAS.pol_tor_angles_2_vector(pol, tor)); x0 = [r * cos(phi), r * sin(phi), z]
+    pos, dir, w = launch_peripheral_rays(x0, N0, spot, invRc, f; kwargs...)
+    n = length(w); K = length(mplasmas); npsi = length(psi_dP_dV)
+    beam = Int32.(repeat(0:K-1, inner=n)); bp = Int32.(collect(0:K-1))
+    dP_dV = zeros(npsi, K); dep = zeros(K); Pf = zeros(n * K); Pd = zeros(n * K); npts = zeros(Int32, n * K); st = zeros(Int32, n * K)
+    cnt = Ref{TorjCounters}()
+    m = torj_multi()
+    torj_check(ccall((:torj_multi_configure, libtorj), Cint, (Ptr{Cvoid}, Int32, Int64, Int32), m, 1, n, 0))
+    try
+        torj_check(ccall((:torj_multi_trace_plasmas, libtorj), Cint,
+            (Ptr{Cvoid}, Int32, Ptr{Ptr{Cvoid}}, Ptr{Int32}, Ref{TorjOptions}, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+             Ref{Float64}, Ref{Int32}, Int32, Float64, Int32, Ptr{Float64}, Int32, Ptr{Int32}, Ptr{Float64}, Ptr{Float64},
+             Ptr{Float64}, Ptr{Float64}, Ptr{Int32}, Ptr{Int32}, Int64, Int64, Int32, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+             Ptr{Float64}, Ptr{Float64}, Ref{TorjCounters}),
+            m, K, mplasmas, bp, options, n * K, repeat(pos, K), repeat(dir, K), repeat(w, K), Float64(f), Int32(mode), 0, s_max,
+            npsi, psi_dP_dV, K, beam, dP_dV, dep, Pf, Pd, npts, st, 0, 0, 0, C_NULL, C_NULL, C_NULL, C_NULL, C_NULL, cnt))
+    finally
+        torj_check(ccall((:torj_multi_configure, libtorj), Cint, (Ptr{Cvoid}, Int32, Int64, Int32), m, 0, 1, 0))
+    end
+    all(ray_ok, st) || throw(AssertionError("ray status $(st)"))
+    return dP_dV, dep, w, reshape(Pf, n, K)
 end

@@ -88,12 +88,17 @@ SIGNATURES = {
     "torj_multi_configure": (C.c_int, [c_vp, C.c_int32, C.c_int64, C.c_int32]),
     "torj_multi_used_nccl": (C.c_int32, [c_vp]),
     "torj_multi_abs_init": (C.c_int, [c_vp, C.c_int32, c_dp, c_dp]),
+    "torj_multi_last_trace_ms": (C.c_int, [c_vp, C.c_int32, c_dp]),
     "torj_multi_plasma_create_from_data": (C.c_int, [c_vp, C.POINTER(TorjGrid), c_dp, c_dp, c_dp, c_dp, C.c_int32, c_dp, c_dp,
                                                      c_dp, c_dp, c_dp, C.c_int32, C.POINTER(c_vp)]),
     "torj_multi_plasma_destroy": (None, [c_vp]),
     "torj_multi_trace": (C.c_int, [c_vp, c_vp, C.POINTER(TorjOptions), C.c_int64, c_dp, c_dp, c_dp, c_dp, c_ip, C.c_int32,
                                    C.c_double, C.c_int32, c_dp, C.c_int32, c_ip, c_dp, c_dp, c_dp, c_dp, c_ip, c_ip, C.c_int64,
                                    C.c_int64, C.c_int32, c_dp, c_dp, c_dp, c_dp, c_dp, C.POINTER(TorjCounters)]),
+    "torj_multi_trace_plasmas": (C.c_int, [c_vp, C.c_int32, C.POINTER(c_vp), c_ip, C.POINTER(TorjOptions), C.c_int64, c_dp, c_dp,
+                                           c_dp, c_dp, c_ip, C.c_int32, C.c_double, C.c_int32, c_dp, C.c_int32, c_ip, c_dp, c_dp,
+                                           c_dp, c_dp, c_ip, c_ip, C.c_int64, C.c_int64, C.c_int32, c_dp, c_dp, c_dp, c_dp, c_dp,
+                                           C.POINTER(TorjCounters)]),
     "torj_fp64_peak": (C.c_int, [c_vp, C.c_int32, c_dp, c_dp]),
     "torj_fp64_latency": (C.c_int, [c_vp, C.c_int32, c_dp]),
     "torj_math_probe": (C.c_int, [c_vp, C.c_int64, c_dp, c_dp]),

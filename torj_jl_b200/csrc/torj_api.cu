@@ -1492,6 +1492,11 @@ int torj_multi_abs_init(torj_multi* m, int32_t n, const double* nodes, const dou
     return 0;
 }
 
+int torj_multi_last_trace_ms(torj_multi* m, int32_t device, double* ms) {
+    if (device < 0 || device >= (int)m->ctx.size()) FAIL("torj_multi_last_trace_ms: device outside the torj_multi");
+    return torj_ctx_last_trace_ms(m->ctx[device], ms);
+}
+
 int torj_multi_plasma_create_from_data(torj_multi* m, const torj_grid* g, const double* psi_norm, const double* psi_prof,
                                        const double* ne_prof, const double* Te_prof, int32_t n_prof, const double* BR,
                                        const double* BZ, const double* Bphi, const double* psi_1d, const double* vol_1d,
@@ -1530,20 +1535,45 @@ static void shard_indices(int64_t n_rays, int used, int d, int sharding, int64_t
     }
 }
 
-// Phase A on device d: gather the shard into pinned staging, upload, enqueue ray init + trace + finalize.
-// Phase B: (NCCL all-reduce of the device profile buffers, in place, one call per device thread;) results to the host.
-int torj_multi_trace(torj_multi* m, const torj_mplasma* mp, const torj_options* opt, int64_t n_rays, const double* pos,
-                     const double* dir, const double* weight, const double* freq_hz, const int32_t* mode, int32_t per_ray_fm,
-                     double s_max, int32_t n_psi, const double* psi_edges, int32_t n_beams, const int32_t* beam_id,
-                     double* dP_dV, double* deposited_power, double* P_final, double* P_dep, int32_t* n_points,
-                     int32_t* status, int64_t traj_first, int64_t traj_count, int32_t traj_max_pts, double* traj_s,
-                     double* traj_xyz, double* traj_P, double* traj_dP_ds, double* traj_dP_dV_ray, torj_counters* counters) {
+// torj_multi_trace (one plasma, called "plasma" in the refusals: set_api false) and torj_multi_trace_plasmas.
+// Every refusal comes before phase A, so a refused call enqueues nothing and leaves the devices' workspaces as they were.
+// Phase A on device d: gather the shard into pinned staging, upload, enqueue ray init + trace + finalize through the set's
+// copies on d. Phase B: (NCCL all-reduce of the device profile buffers, in place, one call per device thread;) results to
+// the host.
+static int multi_trace(torj_multi* m, const char* fn, bool set_api, int32_t n_pl, const torj_mplasma* const* mps,
+                       const int32_t* beam_plasma, const torj_options* opt, int64_t n_rays, const double* pos,
+                       const double* dir, const double* weight, const double* freq_hz, const int32_t* mode, int32_t per_ray_fm,
+                       double s_max, int32_t n_psi, const double* psi_edges, int32_t n_beams, const int32_t* beam_id,
+                       double* dP_dV, double* deposited_power, double* P_final, double* P_dep, int32_t* n_points,
+                       int32_t* status, int64_t traj_first, int64_t traj_count, int32_t traj_max_pts, double* traj_s,
+                       double* traj_xyz, double* traj_P, double* traj_dP_ds, double* traj_dP_dV_ray, torj_counters* counters) {
     const int nd = (int)m->ctx.size();
-    if ((int)mp->p.size() != nd) FAIL("torj_multi_trace: plasma was created on a different device set");
-    if (n_rays < 1) FAIL("torj_multi_trace: n_rays < 1");
+    char msg[256];
+    const bool have = n_pl >= 1 && mps;
+    for (int k = 0; have && k < n_pl; ++k) {  // every device holds its own copy of a plasma, made by this torj_multi
+        const torj_mplasma* mp = mps[k];
+        if (!mp) continue;  // check_plasma_set names it
+        char who[32] = "plasma";
+        if (set_api) snprintf(who, sizeof who, "plasmas[%d]", k);
+        if ((int)mp->p.size() != nd) { snprintf(msg, sizeof msg, "%s: %s was created on a different device set", fn, who); FAIL(msg); }
+        for (int d = 0; d < nd; ++d)
+            if (mp->p[d]->ctx != m->ctx[d]) {
+                snprintf(msg, sizeof msg, "%s: %s belongs to another torj_multi (its copy on device %d has another context)", fn,
+                         who, d);
+                FAIL(msg);
+            }
+    }
     if (n_beams < 1 || !beam_id) n_beams = 1;
-    if (traj_count < 0 || (traj_count > 0 && (traj_first < 0 || traj_first + traj_count > n_rays)))
-        FAIL("torj_multi_trace: trajectory window outside the bundle");
+    std::vector<std::vector<const torj_plasma*>> sets(nd, std::vector<const torj_plasma*>(have ? n_pl : 0, nullptr));
+    for (int d = 0; d < nd; ++d) {
+        for (int k = 0; have && k < n_pl; ++k) sets[d][k] = mps[k] ? mps[k]->p[d] : nullptr;
+        if (int rc = check_plasma_set(fn, m->ctx[d], n_pl, have ? sets[d].data() : nullptr, beam_plasma, n_beams)) return rc;
+    }
+    if (n_rays < 1) { snprintf(msg, sizeof msg, "%s: n_rays < 1", fn); FAIL(msg); }
+    if (traj_count < 0 || (traj_count > 0 && (traj_first < 0 || traj_first + traj_count > n_rays))) {
+        snprintf(msg, sizeof msg, "%s: trajectory window outside the bundle", fn);
+        FAIL(msg);
+    }
     int used = (int)std::min<int64_t>(nd, n_rays);
     if (m->sharding == 1) used = (int)std::min<int64_t>(used, (n_rays + m->block - 1) / m->block);
     std::vector<int> rcs(used, 0);
@@ -1590,7 +1620,7 @@ int torj_multi_trace(torj_multi* m, const torj_mplasma* mp, const torj_options* 
         if (wcnt[d] != b->traj_count || wlo[d] != b->traj_first || (wcnt[d] > 0 && traj_max_pts != b->traj_max))
             rc = torj_bundle_set_window(b, wlo[d], wcnt[d], traj_max_pts);
         if (!rc) rc = torj_bundle_set_beams(b, n_beams, n_beams > 1 ? S.beam : nullptr);
-        if (!rc) rc = torj_bundle_trace(b, mp->p[d], opt, s_max, n_psi, psi_edges);
+        if (!rc) rc = bundle_trace(b, n_pl, sets[d].data(), beam_plasma, opt, s_max, n_psi, psi_edges);
         if (rc) fail(rc);
     });
     bool all_ok = true;
@@ -1673,6 +1703,30 @@ int torj_multi_trace(torj_multi* m, const torj_mplasma* mp, const torj_options* 
         }
     }
     return 0;
+}
+
+int torj_multi_trace(torj_multi* m, const torj_mplasma* mp, const torj_options* opt, int64_t n_rays, const double* pos,
+                     const double* dir, const double* weight, const double* freq_hz, const int32_t* mode, int32_t per_ray_fm,
+                     double s_max, int32_t n_psi, const double* psi_edges, int32_t n_beams, const int32_t* beam_id,
+                     double* dP_dV, double* deposited_power, double* P_final, double* P_dep, int32_t* n_points,
+                     int32_t* status, int64_t traj_first, int64_t traj_count, int32_t traj_max_pts, double* traj_s,
+                     double* traj_xyz, double* traj_P, double* traj_dP_ds, double* traj_dP_dV_ray, torj_counters* counters) {
+    return multi_trace(m, "torj_multi_trace", false, 1, &mp, nullptr, opt, n_rays, pos, dir, weight, freq_hz, mode, per_ray_fm,
+                       s_max, n_psi, psi_edges, n_beams, beam_id, dP_dV, deposited_power, P_final, P_dep, n_points, status,
+                       traj_first, traj_count, traj_max_pts, traj_s, traj_xyz, traj_P, traj_dP_ds, traj_dP_dV_ray, counters);
+}
+
+int torj_multi_trace_plasmas(torj_multi* m, int32_t n_plasmas, const torj_mplasma* const* plasmas, const int32_t* beam_plasma,
+                             const torj_options* opt, int64_t n_rays, const double* pos, const double* dir, const double* weight,
+                             const double* freq_hz, const int32_t* mode, int32_t per_ray_fm, double s_max, int32_t n_psi,
+                             const double* psi_edges, int32_t n_beams, const int32_t* beam_id, double* dP_dV,
+                             double* deposited_power, double* P_final, double* P_dep, int32_t* n_points, int32_t* status,
+                             int64_t traj_first, int64_t traj_count, int32_t traj_max_pts, double* traj_s, double* traj_xyz,
+                             double* traj_P, double* traj_dP_ds, double* traj_dP_dV_ray, torj_counters* counters) {
+    return multi_trace(m, "torj_multi_trace_plasmas", true, n_plasmas, plasmas, beam_plasma, opt, n_rays, pos, dir, weight,
+                       freq_hz, mode, per_ray_fm, s_max, n_psi, psi_edges, n_beams, beam_id, dP_dV, deposited_power, P_final,
+                       P_dep, n_points, status, traj_first, traj_count, traj_max_pts, traj_s, traj_xyz, traj_P, traj_dP_ds,
+                       traj_dP_dV_ray, counters);
 }
 
 int torj_fp64_peak(torj_ctx* c, int32_t iters, double* tflops, double* ms) {

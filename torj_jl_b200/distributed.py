@@ -51,29 +51,57 @@ def _world():
     return 0, 1
 
 
-def trace_sharded(trace_fn, ray_positions, ray_directions, ray_weights, *, sharding="contiguous", block=1, device=None,
-                  gather_rays=True):
+def trace_sharded(trace_fn, ray_positions, ray_directions, ray_weights, *, n_beams=1, per_ray=None, sharding="contiguous",
+                  block=1, device=None, gather_rays=True):
     """make_beam's parallel region and reduction (reference src/solve.jl:219-240) over the ranks of the initialised process
     group. `trace_fn(pos, dirs, w)` traces this rank's rays — on a GPU box `lambda p, d, w: tj.trace_bundle(plasma, p, d, w,
     ...)` — and returns a dict with dP_dV [n_psi], deposited_power, P_final / n_points / status [n_local].
-    Returns the all-reduced dP_dV, deposited_power and sum of weights, this rank's `local` result and `idx`, and (when
-    gather_rays) the per-ray outputs of the WHOLE bundle in launch order, identical on every rank."""
+    per_ray: a dict of further per-ray arrays over the whole bundle (beam_id, f, mode, ...); each is cut to this rank's rays
+    and passed to trace_fn as a keyword argument of that name.
+    n_beams > 1: trace_fn returns dP_dV [n_beams, n_psi] and deposited_power [n_beams], per_ray holds "beam_id", and the
+    reduced vector is the device profile layout [n_beams][n_psi | deposited | sum w] with the weights summed per beam. A
+    plasma set then runs as `lambda p, d, w, beam_id: tj.trace_bundle(plasmas, p, d, w, ..., beam_id=beam_id, n_beams=K,
+    beam_plasma=bp)`.
+    Returns the all-reduced dP_dV, deposited_power and sum of weights (per beam when n_beams > 1), this rank's `local`
+    result and `idx`, and (when gather_rays) the per-ray outputs of the WHOLE bundle in launch order, identical on every
+    rank."""
     import torch
     import torch.distributed as dist
 
     rank, world = _world()
     pos, dirs, w = np.asarray(ray_positions), np.asarray(ray_directions), np.asarray(ray_weights)
     n = len(w)
+    per_ray = {k: np.asarray(v) for k, v in (per_ray or {}).items()}
+    for k, v in per_ray.items():
+        if len(v) != n:
+            raise ValueError(f"per_ray[{k!r}] must have one entry per ray ({n}), got {len(v)}")
+    n_beams = int(n_beams)
+    if n_beams > 1:
+        bid = per_ray.get("beam_id")
+        if bid is None:
+            raise ValueError("n_beams > 1 needs per_ray['beam_id'] (the beam of every ray)")
+        if n and (bid.min() < 0 or bid.max() >= n_beams):
+            raise ValueError(f"beam_id must lie in [0, {n_beams})")
     idx = shard_indices(n, rank, world, sharding, block)
-    local = trace_fn(pos[idx], dirs[idx], w[idx])
-    vec = np.concatenate([np.ravel(local["dP_dV"]), [float(local["deposited_power"]), float(np.sum(w[idx]))]])
+    local = trace_fn(pos[idx], dirs[idx], w[idx], **{k: v[idx] for k, v in per_ray.items()})
+    if n_beams > 1:
+        sw = np.bincount(per_ray["beam_id"][idx], weights=w[idx], minlength=n_beams)
+        vec = np.concatenate([np.reshape(local["dP_dV"], (n_beams, -1)), np.reshape(local["deposited_power"], (n_beams, 1)),
+                              sw[:, None]], axis=1).ravel()
+    else:
+        vec = np.concatenate([np.ravel(local["dP_dV"]), [float(local["deposited_power"]), float(np.sum(w[idx]))]])
     t = torch.from_numpy(vec.copy())
     if device is not None:
         t = t.to(device)
     allreduce_profile(t)
     vec_sum = t.cpu().numpy()
-    out = dict(dP_dV=vec_sum[:-2], deposited_power=float(vec_sum[-2]), sum_weights=float(vec_sum[-1]), local=local, idx=idx,
-               local_vector=vec)
+    if n_beams > 1:
+        rows = vec_sum.reshape(n_beams, -1)
+        out = dict(dP_dV=rows[:, :-2].copy(), deposited_power=rows[:, -2].copy(), sum_weights=rows[:, -1].copy(), local=local,
+                   idx=idx, local_vector=vec)
+    else:
+        out = dict(dP_dV=vec_sum[:-2], deposited_power=float(vec_sum[-2]), sum_weights=float(vec_sum[-1]), local=local, idx=idx,
+                   local_vector=vec)
     if gather_rays:
         mine = {k: np.asarray(local[k]) for k in ("P_final", "n_points", "status") if k in local}
         parts = [None] * world

@@ -23,12 +23,14 @@ class MultiGPU:
         _lib.check(_lib.lib().torj_multi_create(int(n_devices), C.byref(self.h)))
         self.n_devices = int(_lib.lib().torj_multi_device_count(self.h))
         self._plasmas = {}
+        self.config = dict(sharding="contiguous", block_rays=1, deterministic=False)  # torj_multi_create's state
 
     def configure(self, sharding="contiguous", block_rays=1, deterministic=False):
         """sharding: "contiguous" | "block_cyclic" (blocks of block_rays consecutive rays — one beam — dealt round-robin);
-        deterministic: host sum in device order instead of the NCCL all-reduce."""
+        deterministic: host sum in device order instead of the NCCL all-reduce. `config` holds the current state."""
         code = {"contiguous": 0, "block_cyclic": 1}[sharding]
         _lib.check(_lib.lib().torj_multi_configure(self.h, code, int(block_rays), int(bool(deterministic))))
+        self.config = dict(sharding=sharding, block_rays=int(block_rays), deterministic=bool(deterministic))
 
     @property
     def used_nccl(self) -> bool:
@@ -56,19 +58,46 @@ class MultiGPU:
         return self._plasmas[key][0]
 
     def trace_bundle(self, plasma, ray_positions, ray_directions, ray_weights, f, mode, s_max, psi_dP_dV, *, options=None,
-                     beam_id=None, n_beams=1):
-        """Same arguments and result keys as torj_jl_b200.trace_bundle (without trajectories)."""
-        from .solve import bundle_result, marshal_bundle
-        L = _lib.lib()
-        m = marshal_bundle(ray_positions, ray_directions, ray_weights, f, mode, psi_dP_dV, beam_id, n_beams)
+                     beam_id=None, n_beams=1, beam_plasma=None):
+        """Same arguments and result keys as torj_jl_b200.trace_bundle (without trajectories). A sequence of plasmas with
+        beam_plasma traces beam b through plasmas[beam_plasma[b]] on whichever device holds its rays
+        (torj_multi_trace_plasmas); each plasma's copies on the devices are made once and kept."""
+        from .solve import _plasma_set, bundle_result, marshal_bundle
+        pls = _plasma_set(plasma, beam_plasma)
+        m = marshal_bundle(ray_positions, ray_directions, ray_weights, f, mode, psi_dP_dV, beam_id, n_beams,
+                           n_plasmas=len(pls) if pls else 1, beam_plasma=beam_plasma)
         o, psi = m["out"], m["psi"]
+        L = _lib.lib()
         opt = options or _lib.default_options()
-        _lib.check(L.torj_multi_trace(self.h, self._plasma(plasma), C.byref(opt), m["n"], _p(m["pos"]), _p(m["dir"]), _p(m["w"]),
-                                      _p(m["f"]), m["mode"].ctypes.data_as(c_ip), m["per_ray"], float(s_max), len(psi), _p(psi),
-                                      m["n_beams"], m["beam"].ctypes.data_as(c_ip) if m["beam"] is not None else None,
-                                      _p(o["prof"]), _p(o["dep"]), _p(o["Pf"]), _p(o["Pd"]), o["npts"].ctypes.data_as(c_ip),
-                                      o["st"].ctypes.data_as(c_ip), 0, 0, 0, None, None, None, None, None, C.byref(o["cnt"])))
+        rest = (C.byref(opt), m["n"], _p(m["pos"]), _p(m["dir"]), _p(m["w"]), _p(m["f"]), m["mode"].ctypes.data_as(c_ip),
+                m["per_ray"], float(s_max), len(psi), _p(psi), m["n_beams"],
+                m["beam"].ctypes.data_as(c_ip) if m["beam"] is not None else None, _p(o["prof"]), _p(o["dep"]), _p(o["Pf"]),
+                _p(o["Pd"]), o["npts"].ctypes.data_as(c_ip), o["st"].ctypes.data_as(c_ip), 0, 0, 0, None, None, None, None,
+                None, C.byref(o["cnt"]))
+        if pls is None:
+            _lib.check(L.torj_multi_trace(self.h, self._plasma(plasma), *rest))
+        else:
+            hs = (c_vp * len(pls))(*[self._plasma(p).value for p in pls])
+            _lib.check(L.torj_multi_trace_plasmas(self.h, len(pls), hs, m["beam_plasma"].ctypes.data_as(c_ip), *rest))
         return bundle_result(m)
+
+    def make_beam_series(self, plasmas, r, phi, z, steering_angle_tor, steering_angle_pol, spot_size,
+                         inverse_curvature_radius, f, mode, s_max, psi_dP_dV, *, options=None, **kwargs):
+        """torj_jl_b200.make_beam_series over the devices (same arguments and result, without trajectories): the beam's
+        rays on every plasma are whole beams dealt round-robin (block-cyclic with block_rays = rays per beam), so each
+        device traces whole plasmas; `config` is restored afterwards."""
+        from .solve import beam_series
+        saved = dict(self.config)
+
+        def trace(pls, pos, dirs, w, *a, **k):
+            self.configure("block_cyclic", len(w) // len(pls), saved["deterministic"])
+            try:
+                return self.trace_bundle(pls, pos, dirs, w, *a, options=options, **k)
+            finally:
+                self.configure(**saved)
+
+        return beam_series(trace, plasmas, r, phi, z, steering_angle_tor, steering_angle_pol, spot_size,
+                           inverse_curvature_radius, f, mode, s_max, psi_dP_dV, **kwargs)
 
     def close(self):
         if self.h:

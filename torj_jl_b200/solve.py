@@ -66,6 +66,16 @@ def _plasma_list(plasma):
     return pls
 
 
+def _plasma_set(plasma, beam_plasma):
+    """trace_bundle's plasma and beam_plasma: None for a Plasma, the list for a sequence (which needs beam_plasma)."""
+    pls = _plasma_list(plasma)
+    if pls is None and beam_plasma is not None:
+        raise ValueError("beam_plasma needs a sequence of plasmas")
+    if pls is not None and beam_plasma is None:
+        raise ValueError("a sequence of plasmas needs beam_plasma (the plasma of every beam)")
+    return pls
+
+
 def bundle_result(m):
     o, nb = m["out"], m["n_beams"]
     return dict(dP_dV=o["prof"] if nb > 1 else o["prof"][0], deposited_power=o["dep"] if nb > 1 else float(o["dep"][0]),
@@ -78,11 +88,7 @@ def trace_bundle(plasma, ray_positions, ray_directions, ray_weights, f, mode, s_
     beam_id/n_beams: rays of several beams in one bundle -> dP_dV[n_beams, n_psi], deposited_power[n_beams].
     plasma: a Plasma, or a sequence of Plasma on one (R,Z) grid with beam_plasma[n_beams] naming the plasma of every beam
     (torj_trace_plasmas; keep each beam's rays contiguous)."""
-    pls = _plasma_list(plasma)
-    if pls is None and beam_plasma is not None:
-        raise ValueError("beam_plasma needs a sequence of plasmas")
-    if pls is not None and beam_plasma is None:
-        raise ValueError("a sequence of plasmas needs beam_plasma (the plasma of every beam)")
+    pls = _plasma_set(plasma, beam_plasma)
     m = marshal_bundle(ray_positions, ray_directions, ray_weights, f, mode, psi_dP_dV, beam_id, n_beams,
                        n_plasmas=len(pls) if pls else 1, beam_plasma=beam_plasma)
     ctx = ctx or _lib.context()
@@ -249,6 +255,16 @@ def make_beam_series(plasmas, r, phi, z, steering_angle_tor, steering_angle_pol,
     plasma, contiguous. Returns (dP_dV[n_plasmas, n_psi], deposited_power[n_plasmas], ray_weights, P_final[n_plasmas, n],
     res) where res holds the per-ray arrays over the whole bundle (plasma k's rays at [k n, (k+1) n)). No trajectories
     unless `trajectories` = (first, count) over that bundle: the window would otherwise hold n_plasmas beams."""
+    def trace(*a, **k):
+        return trace_bundle(*a, options=options, ctx=ctx, trajectories=trajectories, **k)
+
+    return beam_series(trace, plasmas, r, phi, z, steering_angle_tor, steering_angle_pol, spot_size, inverse_curvature_radius,
+                       f, mode, s_max, psi_dP_dV, **kwargs)
+
+
+def beam_series(trace, plasmas, r, phi, z, steering_angle_tor, steering_angle_pol, spot_size, inverse_curvature_radius, f,
+                mode, s_max, psi_dP_dV, **kwargs):
+    """make_beam_series through `trace`, a function with trace_bundle's arguments (tj.trace_bundle, MultiGPU.trace_bundle)."""
     pls = _plasma_list(plasmas)
     if pls is None:
         pls = [plasmas]
@@ -257,8 +273,7 @@ def make_beam_series(plasmas, r, phi, z, steering_angle_tor, steering_angle_pol,
     x0 = np.array([r * np.cos(phi), r * np.sin(phi), z])
     pos, dirs, wts = launch_peripheral_rays(x0, N0, spot_size, inverse_curvature_radius, f, **kwargs)
     n = len(wts)
-    res = trace_bundle(pls, np.tile(pos, (K, 1)), np.tile(dirs, (K, 1)), np.tile(wts, K), float(f), int(mode), s_max,
-                       psi_dP_dV, options=options, ctx=ctx, trajectories=trajectories,
-                       beam_id=np.repeat(np.arange(K, dtype=np.int32), n) if K > 1 else None, n_beams=K,
-                       beam_plasma=np.arange(K, dtype=np.int32))
+    res = trace(pls, np.tile(pos, (K, 1)), np.tile(dirs, (K, 1)), np.tile(wts, K), float(f), int(mode), s_max, psi_dP_dV,
+                beam_id=np.repeat(np.arange(K, dtype=np.int32), n) if K > 1 else None, n_beams=K,
+                beam_plasma=np.arange(K, dtype=np.int32))
     return (np.atleast_2d(res["dP_dV"]), np.atleast_1d(res["deposited_power"]), wts, res["P_final"].reshape(K, n), res)
