@@ -35,7 +35,7 @@ src = open(os.path.join(root, "torj_jl_b200", "csrc", "torj_device.cuh")).read()
 find = lambda s: next(i + 1 for i, l in enumerate(src) if s in l)
 marks = [("rcp/rsqrt/sqrt", find("rcp_fast(double") - 8), ("bs_weights", find("bs_weights(") - 2), ("stencil", find("struct Fields")),
          ("fields misc", find("eval_field_ext(const DevTables T") - 8), ("dispersion", find("refractive_index_sq(") - 3),
-         ("polarisation", find("struct Pol")), ("exp_fast", find("__constant__ double c_exp") - 4),
+         ("polarisation", find("struct Pol")), ("exp_fast", find("// exp(x), branch-free")),
          ("bessel+node loop", find("bessel_JD(double hz") - 8), ("harmonic_alpha", find("harmonic_sum_large(const HarmCoef c") - 2),
          ("abs_albajar", find("double abs_albajar(") - 8), ("rhs body", find("struct PointVals") - 4),
          ("deposition", find("struct DepoState") - 2)]

@@ -286,13 +286,6 @@ int torj_ctx_create(int device, void* cuda_stream, torj_ctx** out) {
     for (int n = 0; n < 5; ++n)
         for (int k = 0; k < TORJ_BESS_K; ++k) bd[n][k] = (double)(n + 2 * k) * bc[n][k];
     CK(cudaMemcpyToSymbol(c_bessd, bd, sizeof bd));
-    {   // exp_fast: range reduction constants and Taylor coefficients 1/13! ... 1/2!, 1/1!, 1/0!
-        double ce[17] = {1.4426950408889634074, -6.93147180369123816490e-01, -1.90821492927058770002e-10};
-        double fact = 1.0, inv[14];
-        for (int n = 0; n <= 13; ++n) { if (n > 0) fact *= (double)n; inv[n] = 1.0 / fact; }
-        for (int j = 0; j <= 13; ++j) ce[3 + j] = inv[13 - j];
-        CK(cudaMemcpyToSymbol(c_exp, ce, sizeof ce));
-    }
     if (int rc = upload_warm_constants(c)) return rc;
     {
         std::lock_guard<std::mutex> lk(g_gl.mu);
@@ -353,7 +346,6 @@ int torj_abs_init(torj_ctx* c, int32_t n, const double* nodes, const double* wei
     g.n = n;
     for (int i = 0; i < n; ++i) {
         g.t[i] = nodes[i];
-        g.w[i] = weights[i];
         g.sq[i] = std::sqrt(1.0 - nodes[i] * nodes[i]);
         g.wp[i] = (2 * i == n - 1) ? 0.5 * weights[i] : weights[i];
     }
@@ -1050,14 +1042,9 @@ static int bundle_trace(torj_bundle* b, int32_t n_pl, const torj_plasma* const* 
         if (model == 1) lpr = (b->n <= lanes_guess / 2) ? 32 : 1;
         else lpr = (b->n * 8 <= lanes_guess / 2) ? 8 : (b->n * 4 <= lanes_guess) ? 4 : (b->n * 2 <= lanes_guess) ? 2 : 1;
     }
-    size_t smem = (size_t)TORJ_BIN_WORDS(n_psi) * sizeof(double);
+    // k_trace's dynamic shared memory: stage derivatives, parked scalars and, for the warm model at one lane per ray, its stash
+    size_t smem = (size_t)(TORJ_K_WORDS + TORJ_PARK_SLOTS * TORJ_TPB) * sizeof(double);
     if (model == 1 && lpr == 1) smem += (size_t)TORJ_WARM_H * TORJ_TPB * sizeof(double);
-#if TORJ_K_SMEM
-    smem += (size_t)TORJ_K_WORDS * sizeof(double);
-#endif
-#if TORJ_PARK
-    smem += (size_t)TORJ_PARK_SLOTS * TORJ_TPB * sizeof(double);
-#endif
     int bps = 0;
     int64_t warps = (b->n * lpr + 31) / 32;
     int64_t blocks_needed = (warps + (TORJ_TPB / 32) - 1) / (TORJ_TPB / 32);
@@ -1068,7 +1055,7 @@ static int bundle_trace(torj_bundle* b, int32_t n_pl, const torj_plasma* const* 
     kern = pick_trace_kernel(od.scheme, high, model, lpr, set);
     CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, kern, TORJ_TPB, smem));
-    if (bps < 1) FAIL("torj_bundle_trace: trace kernel does not fit on an SM (n_psi too large for shared memory)");
+    if (bps < 1) FAIL("torj_bundle_trace: trace kernel does not fit on an SM");
     int64_t grid = std::min<int64_t>((int64_t)c->num_sms * bps, blocks_needed);  // persistent: resident CTAs only
     // Segment hand-off whenever the bundle exceeds the resident lanes. It removes the partly filled last wave (65 543
     // rays on 37 888 lanes: 1.73 ray-times instead of 2) and keeps the lanes of a warp in step: with whole rays per lane

@@ -330,41 +330,15 @@ struct Scheme;
 template <> struct Scheme<0> { static constexpr int S = 7; static constexpr int ORDER = 5; };
 template <> struct Scheme<1> { static constexpr int S = 4; static constexpr int ORDER = 3; };
 
-#ifndef TORJ_TPB
 #define TORJ_TPB 128
-#endif
-#ifndef TORJ_SMEM_BINS
-#define TORJ_SMEM_BINS 0  // 1: single-profile bundles book into block-local shared-memory bins flushed at the end (round 1).
-#endif                    //    Measured SLOWER than booking straight into global memory (119.6 against 117.8 ms on the 65 543-ray
-                          //    beam): a shared-memory FP64 atomicAdd is a CAS loop, a global one is a fire-and-forget RED.ADD.F64.
-#define TORJ_BIN_WORDS(n_psi) (TORJ_SMEM_BINS ? (((n_psi) + 1) & ~1) : 0)
-#ifndef TORJ_K_PAIRS
-#define TORJ_K_PAIRS 1  // 1 (with TORJ_K_SMEM): stage derivatives stored as 4 double2 per stage and thread (8th slot unused), so a
-#endif                  //    stage is read with 4 LDS.128 instead of 7 LDS.64
-#define TORJ_K_WORDS ((TORJ_K_PAIRS ? 56 : 49) * TORJ_TPB)  // doubles of stage storage per CTA
-#ifndef TORJ_K_SMEM
-#define TORJ_K_SMEM 1  // 1: Runge-Kutta stage derivatives k[S][7] live in shared memory instead of (L1-backed) local memory
-#endif
-#ifndef TORJ_PARK
-#define TORJ_PARK 1  // 1: per-segment / per-ray scalars of the integrator live in shared memory
-#endif
-#define TORJ_PARK_SLOTS 9  // doubles per thread reserved when TORJ_PARK (7 doubles + 3 ints, rounded up)
-#ifndef TORJ_ROLL_J
-#define TORJ_ROLL_J 1  // 1: the stage-combination and error-estimate sums run as real loops over the stages: 170 hot instructions
-                       // less against a 32 KB instruction cache (measured 132.0 -> 126.7 ms); 0 = fully unrolled
-#endif
-#ifndef TORJ_ST_BOUND
-#define TORJ_ST_BOUND 1  // 1 (with TORJ_ROLL_J): the stage combination sums the st stages that exist instead of all S-1 zero-padded
-                         // ones (the cadence keeps the lanes of a warp at the same stage): 121.9 -> 119.8 ms
-#endif
-#ifndef TORJ_LIFE_HARM_COST
+// Runge-Kutta stage derivatives k[S][7] live in shared memory, not in (L1-backed) local memory, stored as 4 double2 per
+// stage and thread (8th slot unused), so that a stage is read with 4 LDS.128 instead of 7 LDS.64
+#define TORJ_K_WORDS (56 * TORJ_TPB)  // doubles of stage storage per CTA
+#define TORJ_PARK_SLOTS 9  // doubles per thread of parked per-segment / per-ray scalars (7 doubles + 3 ints, rounded up)
 #define TORJ_LIFE_HARM_COST 0.25  // k_predict_life: rounds one evaluated harmonic integral per pilot point adds to a ray's predicted
                                   // cost (segments inside the absorbing layer take longer). 1/16 and 1/8 shards of the 1 M-ray sweep:
                                   // 0 -> 174.8 / 299.2 ms, 0.25 -> 166.7 / 288.9, 0.5 -> 168.1 / 291.0, 0.75 -> 176.3 / 295.3; beam unchanged
-#endif
-#ifndef TORJ_MINB
 #define TORJ_MINB 2  // resident CTAs per SM the register allocation is bounded for (2 -> 255 regs, 3 -> 168, 4 -> 128)
-#endif
 // per-ray status codes of include/torj_cuda.h: everything but OK(0), LEFT_GRID(3) and TRAJ_TRUNCATED(6) ends the ray
 #define TORJ_FATAL(s) ((s) != 0 && (s) != 6 && (s) != 3)
 
@@ -375,33 +349,6 @@ template <> struct Scheme<1> { static constexpr int S = 4; static constexpr int 
 // another lane / has just loaded a ray's state. Phases >= PH_SEED evaluate the RHS.
 enum { PH_IDLE = 0, PH_WAIT = 1, PH_RESUME = 2, PH_SEED = 3, PH_INITDT = 4, PH_STAGE = 5, PH_CALLBACK = 6 };
 enum { ACT_NONE = 0, ACT_BEGIN_SEGMENT = 1, ACT_BEGIN_STEP = 2, ACT_END_SEGMENT = 3, ACT_AFTER_ACCEPT = 4 };
-
-#ifndef TORJ_STAGE_SWITCH
-#define TORJ_STAGE_SWITCH 0  // 1: the stage combination as a switch over the stage with exact-length unrolled sums and
-#endif                       //    constant-bank coefficients (no loop control, no coefficient loads), at +250 static instructions
-#if TORJ_K_PAIRS
-#define TORJ_KK_AT(ks, j, i) (ks)[((j) * 4 + ((i) >> 1)) * 2 * TORJ_TPB + ((i) & 1)]
-#else
-#define TORJ_KK_AT(ks, j, i) (ks)[((j) * 7 + (i)) * TORJ_TPB]
-#endif
-template <int SCH, int ST>
-__device__ __forceinline__ void stage_sum_unrolled(const double* ks, double dt, const double* u, double* tmp) {
-    double acc[7];
-#pragma unroll
-    for (int j = 0; j < ST; ++j) {
-        const double aj = c_tab[SCH].a[ST][j];
-#pragma unroll
-        for (int i = 0; i < 7; ++i) acc[i] = j == 0 ? aj * TORJ_KK_AT(ks, 0, i) : fma(aj, TORJ_KK_AT(ks, j, i), acc[i]);
-    }
-#pragma unroll
-    for (int i = 0; i < 7; ++i) tmp[i] = fma(dt, acc[i], u[i]);
-}
-
-#ifdef TORJ_MAXNREG
-#define TORJ_TRACE_BOUNDS __maxnreg__(TORJ_MAXNREG)
-#else
-#define TORJ_TRACE_BOUNDS __launch_bounds__(TORJ_TPB, TORJ_MINB)
-#endif
 
 // HIGH = true: harmonics above the third enabled (torj_options.max_harmonic > 3); see abs_albajar
 // MODEL: 0 = Albajar absorption (reference src/absorption.jl), 1 = warm-plasma damping (src/general_absorption.jl α,
@@ -416,35 +363,19 @@ __device__ __forceinline__ void stage_sum_unrolled(const double* ks, double dt, 
 // SET = true: a plasma set (a.P). The grid comes from a.T as always; the table base is per lane, bound with the ray
 //   (a ray's plasma is that of its beam), so rays of several equilibria share one launch.
 template <int SCH, bool HIGH = false, int MODEL = 0, int LPR = 1, bool SET = false>
-__global__ void TORJ_TRACE_BOUNDS k_trace(TraceArgs a) {
+__global__ void __launch_bounds__(TORJ_TPB, TORJ_MINB) k_trace(TraceArgs a) {
     exp_tab_init();
     constexpr bool COOP = LPR == 32;
     constexpr int S = Scheme<SCH>::S;
     constexpr int ORDER = Scheme<SCH>::ORDER;
     extern __shared__ __align__(16) double smem[];
-#if TORJ_SMEM_BINS
-    double* s_bins = smem;                                 // [n_psi] block-local deposition bins
-#endif
     const double* __restrict__ s_edges = a.psi_edges;      // psi levels: read-only, through L1 (__ldg)
-#if TORJ_K_SMEM
-#if TORJ_K_PAIRS
-    double* ks = smem + TORJ_BIN_WORDS(a.n_psi) + 2 * threadIdx.x;         // KK(j, 2p + q) at ks[(j*4+p)*2*TORJ_TPB + q]: 16-byte pairs
+    double* ks = smem + 2 * threadIdx.x;                   // KK(j, 2p + q) at ks[(j*4+p)*2*TORJ_TPB + q]: 16-byte pairs
 #define KK(j, i) ks[((j) * 4 + ((i) >> 1)) * 2 * TORJ_TPB + ((i) & 1)]
-#else
-    double* ks = smem + TORJ_BIN_WORDS(a.n_psi) + threadIdx.x;             // KK(j, i) at ks[(j*7+i)*TORJ_TPB]: conflict-free
-#define KK(j, i) ks[((j) * 7 + (i)) * TORJ_TPB]
-#endif
-#else
-    double k_loc[S][7];
-#define KK(j, i) k_loc[j][i]
-#endif
     __shared__ unsigned long long s_cnt[8];
     __shared__ double s_tot[2];
     __shared__ double s_a[7][7], s_bt[7];
     const int n_psi = a.n_psi;
-#if TORJ_SMEM_BINS
-    for (int j = threadIdx.x; j < n_psi; j += blockDim.x) s_bins[j] = 0.0;
-#endif
     if (threadIdx.x < 8) s_cnt[threadIdx.x] = 0ull;
     if (threadIdx.x < 2) s_tot[threadIdx.x] = 0.0;
     if (threadIdx.x < 49) s_a[threadIdx.x / 7][threadIdx.x % 7] = c_tab[SCH].a[threadIdx.x / 7][threadIdx.x % 7];
@@ -471,12 +402,11 @@ __global__ void TORJ_TRACE_BOUNDS k_trace(TraceArgs a) {
     const double s_step = O.s_max / (double)O.n_segments;
 
     // per-lane ray state
-#if TORJ_PARK
     // Scalars touched once per segment or per ray live in shared memory ([slot][thread], conflict-free): the kernel
     // sits at the 255-register limit and the compiler, not knowing trip frequencies, otherwise spills values that
     // every RHS evaluation touches (ray constants, counters) to local memory (122 -> 72 bytes of spills, -1 % time;
     // parking the once-per-step scalars as well removes the spills altogether but gains nothing more).
-    double* pk = smem + TORJ_BIN_WORDS(a.n_psi) + (TORJ_K_SMEM ? TORJ_K_WORDS : 0) + threadIdx.x;
+    double* pk = smem + TORJ_K_WORDS + threadIdx.x;
 #define PK(k) pk[(k) * TORJ_TPB]
     long long& ray = *reinterpret_cast<long long*>(&PK(0));
     long long& tj = *reinterpret_cast<long long*>(&PK(1));  // index into the trajectory window or -1
@@ -491,16 +421,8 @@ __global__ void TORJ_TRACE_BOUNDS k_trace(TraceArgs a) {
     int& last_stat = PKI(1);
     unsigned int& rays_ok = *reinterpret_cast<unsigned int*>(&PKI(2));
     ray = -1; tj = -1; s0 = 0.0; dt0 = 0.0; d1 = 0.0; tot_dep = 0.0; tot_w = 0.0; seg = 0; last_stat = 0; rays_ok = 0;
-#else
-    long long ray = -1;
-    long long tj = -1;  // index into the trajectory window or -1
-    double s0 = 0.0, dt0 = 0.0, d1 = 0.0;
-    double tot_dep = 0.0, tot_w = 0.0;
-    int seg = 0, last_stat = 0;
-    unsigned int rays_ok = 0;
-#endif
     // warm model, one ray per lane: shared-memory slots where a lane's quadrature sums wait for the serial solve
-    double* wstash = smem + TORJ_BIN_WORDS(a.n_psi) + (TORJ_K_SMEM ? TORJ_K_WORDS : 0) + (TORJ_PARK ? TORJ_PARK_SLOTS * TORJ_TPB : 0) + threadIdx.x;
+    double* wstash = smem + TORJ_K_WORDS + TORJ_PARK_SLOTS * TORJ_TPB + threadIdx.x;
     int phase = PH_IDLE, st = 0;
     bool exhausted = false;
     double u[7], tmp[7];
@@ -526,11 +448,7 @@ __global__ void TORJ_TRACE_BOUNDS k_trace(TraceArgs a) {
     auto sink = [&](int shell, double dP) {
         pdep += dP;
         if (!writer) return;
-#if TORJ_SMEM_BINS
-        if (a.n_beams == 1) atomicAdd(&s_bins[shell], wgt * dP);
-        else
-#endif
-            atomicAdd(&beam_bins[shell], wgt * dP);
+        atomicAdd(&beam_bins[shell], wgt * dP);
         if (tj >= 0) atomicAdd(&a.J.prof[tj * n_psi + shell], dP);  // (a ray may change SMs between segments)
     };
     auto put_point = [&](double s, const double* xx, double P, double dP) {
@@ -746,36 +664,24 @@ __global__ void TORJ_TRACE_BOUNDS k_trace(TraceArgs a) {
 #pragma unroll
                 for (int i = 0; i < 7; ++i) KK(st, i) = out[i];
                 st++;
-                // u + dt * sum_j a[st][j] k_j over ALL S-1 earlier slots: the tableau rows are zero-padded and
-                // stale slots hold finite values of the previous step, so the trip count is lane-independent
-#if TORJ_STAGE_SWITCH && TORJ_K_SMEM
-                switch (st) {
-                    case 2: stage_sum_unrolled<SCH, 2>(ks, dt, u, tmp); break;
-                    case 3: stage_sum_unrolled<SCH, 3>(ks, dt, u, tmp); break;
-                    case 4: stage_sum_unrolled<SCH, (S > 4 ? 4 : 2)>(ks, dt, u, tmp); break;
-                    case 5: stage_sum_unrolled<SCH, (S > 5 ? 5 : 2)>(ks, dt, u, tmp); break;
-                    default: stage_sum_unrolled<SCH, (S > 6 ? 6 : 2)>(ks, dt, u, tmp); break;
-                }
-#else
+                // u + dt * sum_j a[st][j] k_j over the st stages computed so far. The cadence keeps the lanes of a warp
+                // at the same stage, so the trip count is warp-uniform. A real loop, not unrolled: together with the
+                // rolled error sum below, 170 hot instructions less against a 32 KB instruction cache (132.0 -> 126.7 ms);
+                // bounded by st rather than summing all S-1 zero-padded rows: 121.9 -> 119.8 ms
                 double acc[7];
                 {
                     const double a0 = s_a[st][0];  // st >= 2 here: the first term initialises the sums
 #pragma unroll
                     for (int i = 0; i < 7; ++i) acc[i] = a0 * KK(0, i);
                 }
-#if TORJ_ROLL_J
 #pragma unroll 1
-#else
-#pragma unroll
-#endif
-                for (int j = 1; j < ((TORJ_ST_BOUND && TORJ_ROLL_J) ? st : S - 1); ++j) {
+                for (int j = 1; j < st; ++j) {
                     const double aj = s_a[st][j];
 #pragma unroll
                     for (int i = 0; i < 7; ++i) acc[i] = fma(aj, KK(j, i), acc[i]);
                 }
 #pragma unroll
                 for (int i = 0; i < 7; ++i) tmp[i] = fma(dt, acc[i], u[i]);
-#endif
             }
         } else if (phase == PH_STAGE) {
             {
@@ -787,29 +693,16 @@ __global__ void TORJ_TRACE_BOUNDS k_trace(TraceArgs a) {
                 dpsi_new = out[8];
                 double at[7];
                 bool bad = false;
-#if TORJ_ROLL_J
                 double utv[7] = {0, 0, 0, 0, 0, 0, 0};
-#if TORJ_STAGE_SWITCH
-#pragma unroll
-#else
 #pragma unroll 1
-#endif
                 for (int j = 0; j < S; ++j) {
-                    const double bj = TORJ_STAGE_SWITCH ? c_tab[SCH].bt[j] : s_bt[j];
+                    const double bj = s_bt[j];
 #pragma unroll
                     for (int i = 0; i < 7; ++i) utv[i] = fma(bj, KK(j, i), utv[i]);
                 }
-#endif
 #pragma unroll
                 for (int i = 0; i < 7; ++i) {
-#if TORJ_ROLL_J
-                    double ut = utv[i];
-#else
-                    double ut = 0.0;
-#pragma unroll
-                    for (int j = 0; j < S; ++j) ut = fma(s_bt[j], KK(j, i), ut);
-#endif
-                    ut *= dt;
+                    const double ut = utv[i] * dt;
                     const double au = fabs(u[i]), an = fabs(tmp[i]);
                     at[i] = ut * rcp_fast(O.abstol + (au > an ? au : an) * O.reltol);
                     if (!(tmp[i] == tmp[i])) bad = true;
@@ -1045,17 +938,11 @@ __global__ void TORJ_TRACE_BOUNDS k_trace(TraceArgs a) {
         for (int q = 0; q < 8; ++q) atomicAdd(&s_cnt[q], c6[q]);
     }
     __syncthreads();
-#if TORJ_SMEM_BINS
-    for (int j = threadIdx.x; j < n_psi; j += blockDim.x)
-        if (s_bins[j] != 0.0) atomicAdd(&a.bins[j], s_bins[j]);
-#endif
     if (threadIdx.x < 2) atomicAdd(&a.bins[n_psi + threadIdx.x], s_tot[threadIdx.x]);
     if (threadIdx.x < 8) atomicAdd(&a.counters[threadIdx.x], s_cnt[threadIdx.x]);
 #undef KK
-#if TORJ_PARK
 #undef PK
 #undef PKI
-#endif
 }
 
 // Predicted life of every ray in segments, for the order of the hand-off rounds only (never for a result): a straight march
