@@ -121,6 +121,18 @@ int torj_ctx_sync(torj_ctx* ctx);
 int64_t torj_ctx_launch_count(const torj_ctx* ctx);
 /* device duration (CUDA events on the context stream) of the most recent trace-kernel launch; synchronises on it */
 int torj_ctx_last_trace_ms(torj_ctx* ctx, double* ms);
+/* Exact deposition sums, for every later torj_trace(_plasmas) and torj_bundle_trace(_plasmas) on bundles of ctx.
+ * on = 0 (default): each booking into a profile bin is a floating-point atomicAdd, whose order changes from run to run, so
+ * dP_dV and deposited_power may differ in their last bits (the per-ray results never do).
+ * on = 1: each booking (w dP, w P_deposited_ray, w; rounded once to a double, as with 0) is rounded to 2^-160 and summed
+ * without error in a fixed-point integer accumulator; the profile is the correctly rounded value of that exact sum over
+ * dV. It is bit-identical under any schedule, ray order, sharding and device count, at a fixed lanes_per_ray (the per-ray
+ * arithmetic depends on it). Weights must satisfy |w| <= 2^40 (else the trace is refused); a booking of |w dP| >= 2^64 or
+ * NaN, or more than 2^34 bookings in one trace, makes torj_bundle_results fail (the device profile is then NaN).
+ * Other values of `on` are refused. The mode is state of the context and persists until the next call: a caller that
+ * shares a context with code that may have turned it on (the Python package's per-device context, for example) sets it
+ * explicitly before tracing, as every Python entry point does. */
+int torj_ctx_set_exact_sum(torj_ctx* ctx, int32_t on);
 
 /* abs_Al_init(N) — reference src/absorption.jl:1-7: Gauss-Legendre nodes/weights on [-1,1] (n <= 64), ascending and
  * symmetric (t[k] = -t[n-1-k], w[k] = w[n-1-k], as gausslegendre(N) returns them; anything else is refused: the kernel
@@ -206,9 +218,11 @@ int torj_bundle_trace_plasmas(torj_bundle* b, int32_t n_plasmas, const torj_plas
                               const int32_t* beam_plasma /* [n_beams] */, const torj_options* opt, double s_max,
                               int32_t n_psi, const double* psi_edges);
 /* Device pointer to n_beams x (n_psi+2) doubles: dP_dV[n_psi], deposited_power, sum of weights per beam — for a caller-side
- * NCCL all-reduce (sum) across GPUs; valid after torj_bundle_trace, ordered on the context stream. */
+ * NCCL all-reduce (sum) across GPUs; valid after torj_bundle_trace, ordered on the context stream. With exact sums each
+ * device's profile is exact, but a double all-reduce of several devices' profiles is not. */
 void* torj_bundle_device_profile(torj_bundle* b);
-/* Synchronises and copies results to the host (any pointer may be NULL). For a ray that failed initialisation
+/* Synchronises and copies results to the host (any pointer may be NULL); fails after an exact-sum trace whose accumulator
+ * overflowed or refused a booking (torj_ctx_set_exact_sum). For a ray that failed initialisation
  * (status 1 or 2) P_final and P_deposited_ray are 0 and n_points is minus the failing check's number (-1 no grid entry,
  * -2 no psi bracket, -3/-4 asserts of src/solve.jl:32,138, -5..-7 Newton, -8 assert :141, -9 cut-off :55-59). */
 int torj_bundle_results(torj_bundle* b, double* dP_dV, double* deposited_power, double* P_final,
@@ -248,7 +262,10 @@ int torj_trace_plasmas(torj_ctx* ctx, int32_t n_plasmas, const torj_plasma* cons
  * replicated). The weighted sum of reference src/solve.jl:233-240 across devices is ONE ncclAllReduce(sum, double,
  * n_beams * (n_psi + 2)) over NVLink on the devices' profile buffers (communicators from ncclCommInitAll at
  * torj_multi_create; libnccl.so.2 is loaded at run time), or — reduction = 1, and whenever NCCL is unavailable — a
- * host sum in device order, bit-reproducible for a given device count.
+ * host sum in device order. Neither is bit-reproducible by default: each device's own profile carries the noise of its
+ * floating-point atomics. With torj_multi_set_exact_sum(m, 1) both sum the devices' integer accumulators instead (an
+ * ncclInt64 all-reduce or a host integer sum) and convert once, which gives the bits of one device tracing the whole
+ * bundle, whatever the device count and sharding (at a fixed lanes_per_ray).
  * sharding: 0 = contiguous ray blocks; 1 = block-cyclic, blocks of `block_rays` consecutive rays (one beam) dealt
  * round-robin, which balances scans whose beams differ in ray length. */
 typedef struct torj_multi torj_multi;
@@ -260,6 +277,8 @@ int torj_multi_configure(torj_multi* m, int32_t sharding, int64_t block_rays, in
 /* 1 when the cross-device sum of the last torj_multi_trace(_plasmas) went through ncclAllReduce, 0 for the host sum */
 int32_t torj_multi_used_nccl(const torj_multi* m);
 int torj_multi_abs_init(torj_multi* m, int32_t n, const double* nodes, const double* weights);
+/* torj_ctx_set_exact_sum on every device's context: exact sums for every later torj_multi_trace(_plasmas); 0 or 1 */
+int torj_multi_set_exact_sum(torj_multi* m, int32_t on);
 /* torj_ctx_last_trace_ms of device d's context: the k_trace time of its part of the last torj_multi_trace(_plasmas) */
 int torj_multi_last_trace_ms(torj_multi* m, int32_t device, double* ms);
 int torj_multi_plasma_create_from_data(torj_multi* m, const torj_grid* grid, const double* psi_norm, const double* psi_prof,

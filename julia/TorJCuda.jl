@@ -27,6 +27,11 @@ function torj_ctx()
     _ctx[]
 end
 
+# Exact deposition sums for every later call on this context (torj_ctx_set_exact_sum): dP_dV and deposited_power then
+# come out bit-identical under any schedule, ray order and device count, like the reference's serial sum is run to run.
+# Weights |w| <= 2^40. Off (false) is the default and today's floating-point atomics.
+set_exact_sum!(on::Bool) = torj_check(ccall((:torj_ctx_set_exact_sum, libtorj), Cint, (Ptr{Cvoid}, Int32), torj_ctx(), Int32(on)))
+
 # Options: the reference's hard-coded constants (torj_options_default) with keyword overrides, e.g.
 # torj_options(absorption_model = 1) for the warm-plasma damping of src/general_absorption.jl.
 function torj_options(; kw...)
@@ -185,6 +190,11 @@ function torj_multi()
     end
     _multi[]
 end
+
+# Exact sums on every device of torj_multi() (torj_multi_set_exact_sum): the devices' integer accumulators are summed
+# (ncclInt64 all-reduce or on the host) before one conversion, giving the bits of one device tracing the whole bundle.
+multi_set_exact_sum!(on::Bool) =
+    torj_check(ccall((:torj_multi_set_exact_sum, libtorj), Cint, (Ptr{Cvoid}, Int32), torj_multi(), Int32(on)))
 
 # torj_mplasma: one plasma's tables on every device of torj_multi(), built there from the arrays of the Plasma constructor
 # (src/plasma.jl:30-32: 2-D arrays [nR, nZ], profiles and the 1-D volume; route (b) above). Kept until the process exits.

@@ -49,6 +49,7 @@ SIGNATURES = {
     "torj_ctx_sync": (C.c_int, [c_vp]),
     "torj_ctx_launch_count": (C.c_int64, [c_vp]),
     "torj_ctx_last_trace_ms": (C.c_int, [c_vp, c_dp]),
+    "torj_ctx_set_exact_sum": (C.c_int, [c_vp, C.c_int32]),
     "torj_abs_init": (C.c_int, [c_vp, C.c_int32, c_dp, c_dp]),
     "torj_warm_alpha": (C.c_int, [c_vp, C.c_int64, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp, C.c_int32, c_dp, c_dp, c_ip, c_ip]),
     "torj_bspline_prefilter_2d": (C.c_int, [C.c_int32, C.c_int32, c_dp, c_dp]),
@@ -88,6 +89,7 @@ SIGNATURES = {
     "torj_multi_configure": (C.c_int, [c_vp, C.c_int32, C.c_int64, C.c_int32]),
     "torj_multi_used_nccl": (C.c_int32, [c_vp]),
     "torj_multi_abs_init": (C.c_int, [c_vp, C.c_int32, c_dp, c_dp]),
+    "torj_multi_set_exact_sum": (C.c_int, [c_vp, C.c_int32]),
     "torj_multi_last_trace_ms": (C.c_int, [c_vp, C.c_int32, c_dp]),
     "torj_multi_plasma_create_from_data": (C.c_int, [c_vp, C.POINTER(TorjGrid), c_dp, c_dp, c_dp, c_dp, C.c_int32, c_dp, c_dp,
                                                      c_dp, c_dp, c_dp, C.c_int32, C.POINTER(c_vp)]),

@@ -49,6 +49,7 @@ struct torj_ctx {
     bool ev_valid = false;
     struct torj_bundle* ws = nullptr;  // workspace of the one-shot torj_trace call, kept between calls
     double2* d_warm_tab = nullptr;     // set_extv! tables of the warm-plasma model (reference src/general_absorption.jl:8-13)
+    int exact_sum = 0;                 // torj_ctx_set_exact_sum: later traces book profiles exactly (torj_exactsum.cuh)
 };
 
 // The Gauss-Legendre table lives in ONE __constant__ symbol per device (like the reference's module globals,
@@ -112,6 +113,11 @@ struct torj_bundle {
     const void** d_set = nullptr;
     int* d_beam_plasma = nullptr;
     int dV_rows = 1;  // rows of d_dV the last trace used
+    // exact-sum mode (allocated on first use): the words of every bin and the status words, torj_xs_buffer_words(bins)
+    long long* d_xs = nullptr;
+    size_t xs_words = 0;
+    bool xs_last = false;  // the last trace booked exactly: results check the status words
+    double w_max = 0.0;    // max |weight| of the host weights (infinite for a NaN); -1: weights made on the device
 };
 
 // Error paths: temporaries are owned by dev_ptr, objects under construction by a guard that destroys them unless the
@@ -313,6 +319,13 @@ int torj_ctx_sync(torj_ctx* c) {
 }
 
 int64_t torj_ctx_launch_count(const torj_ctx* c) { return c->launches; }
+
+int torj_ctx_set_exact_sum(torj_ctx* c, int32_t on) {
+    if (!c) FAIL("torj_ctx_set_exact_sum: ctx is NULL");
+    if (on != 0 && on != 1) FAIL("torj_ctx_set_exact_sum: on must be 0 (floating-point atomics) or 1 (exact sum)");
+    c->exact_sum = on;
+    return 0;
+}
 
 int torj_ctx_last_trace_ms(torj_ctx* c, double* ms) {
     if (!c->ev_valid) FAIL("torj_ctx_last_trace_ms: no trace launched yet");
@@ -581,21 +594,24 @@ static double volume_at(const torj_plasma* p, double x) {
 
 typedef void (*trace_kernel_t)(TraceArgs);
 extern "C++" {  // (inside the extern "C" block)
-template <bool SET>
+template <bool SET, bool XS>
 static trace_kernel_t pick_trace_kernel_set(int scheme, bool high, int model, int lpr) {
     const bool z3 = scheme == 1;
-    if (model == 1) return lpr == 32 ? (z3 ? k_trace<1, false, 1, 32, SET> : k_trace<0, false, 1, 32, SET>)
-                                     : (z3 ? k_trace<1, false, 1, 1, SET> : k_trace<0, false, 1, 1, SET>);
-    if (lpr == 32) return high ? (z3 ? k_trace<1, true, 0, 32, SET> : k_trace<0, true, 0, 32, SET>) : (z3 ? k_trace<1, false, 0, 32, SET> : k_trace<0, false, 0, 32, SET>);
-    if (lpr == 8) return high ? (z3 ? k_trace<1, true, 0, 8, SET> : k_trace<0, true, 0, 8, SET>) : (z3 ? k_trace<1, false, 0, 8, SET> : k_trace<0, false, 0, 8, SET>);
-    if (lpr == 4) return high ? (z3 ? k_trace<1, true, 0, 4, SET> : k_trace<0, true, 0, 4, SET>) : (z3 ? k_trace<1, false, 0, 4, SET> : k_trace<0, false, 0, 4, SET>);
-    if (lpr == 2) return high ? (z3 ? k_trace<1, true, 0, 2, SET> : k_trace<0, true, 0, 2, SET>) : (z3 ? k_trace<1, false, 0, 2, SET> : k_trace<0, false, 0, 2, SET>);
-    return high ? (z3 ? k_trace<1, true, 0, 1, SET> : k_trace<0, true, 0, 1, SET>) : (z3 ? k_trace<1, false, 0, 1, SET> : k_trace<0, false, 0, 1, SET>);
+    if (model == 1) return lpr == 32 ? (z3 ? k_trace<1, false, 1, 32, SET, XS> : k_trace<0, false, 1, 32, SET, XS>)
+                                     : (z3 ? k_trace<1, false, 1, 1, SET, XS> : k_trace<0, false, 1, 1, SET, XS>);
+    if (lpr == 32) return high ? (z3 ? k_trace<1, true, 0, 32, SET, XS> : k_trace<0, true, 0, 32, SET, XS>) : (z3 ? k_trace<1, false, 0, 32, SET, XS> : k_trace<0, false, 0, 32, SET, XS>);
+    if (lpr == 8) return high ? (z3 ? k_trace<1, true, 0, 8, SET, XS> : k_trace<0, true, 0, 8, SET, XS>) : (z3 ? k_trace<1, false, 0, 8, SET, XS> : k_trace<0, false, 0, 8, SET, XS>);
+    if (lpr == 4) return high ? (z3 ? k_trace<1, true, 0, 4, SET, XS> : k_trace<0, true, 0, 4, SET, XS>) : (z3 ? k_trace<1, false, 0, 4, SET, XS> : k_trace<0, false, 0, 4, SET, XS>);
+    if (lpr == 2) return high ? (z3 ? k_trace<1, true, 0, 2, SET, XS> : k_trace<0, true, 0, 2, SET, XS>) : (z3 ? k_trace<1, false, 0, 2, SET, XS> : k_trace<0, false, 0, 2, SET, XS>);
+    return high ? (z3 ? k_trace<1, true, 0, 1, SET, XS> : k_trace<0, true, 0, 1, SET, XS>) : (z3 ? k_trace<1, false, 0, 1, SET, XS> : k_trace<0, false, 0, 1, SET, XS>);
 }
 }
 // set: the plasma-set instantiations (torj_bundle_trace_plasmas with more than one plasma)
-static trace_kernel_t pick_trace_kernel(int scheme, bool high, int model, int lpr, bool set) {
-    return set ? pick_trace_kernel_set<true>(scheme, high, model, lpr) : pick_trace_kernel_set<false>(scheme, high, model, lpr);
+// xs: the exact-sum instantiations (a template parameter: a never-taken out-of-line call in the float kernels measured 0.7 %
+// on the bench beam and on the warm model at one lane per ray, profiles/README.md)
+static trace_kernel_t pick_trace_kernel(int scheme, bool high, int model, int lpr, bool set, bool xs) {
+    if (xs) return set ? pick_trace_kernel_set<true, true>(scheme, high, model, lpr) : pick_trace_kernel_set<false, true>(scheme, high, model, lpr);
+    return set ? pick_trace_kernel_set<true, false>(scheme, high, model, lpr) : pick_trace_kernel_set<false, false>(scheme, high, model, lpr);
 }
 
 static SolverOpts to_sopts(const torj_options* o, double s_max) {
@@ -695,6 +711,8 @@ static int bundle_upload(torj_bundle* b, const double* pos, const double* dir, c
     CK(cudaMemcpyAsync(b->d_pos, pos, 3 * n * sizeof(double), cudaMemcpyHostToDevice, c->stream));
     CK(cudaMemcpyAsync(b->d_dir, dir, 3 * n * sizeof(double), cudaMemcpyHostToDevice, c->stream));
     CK(cudaMemcpyAsync(b->d_w, weight, n * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    b->w_max = 0.0;
+    for (int64_t i = 0; i < n; ++i) b->w_max = std::isnan(weight[i]) ? INFINITY : std::max(b->w_max, std::fabs(weight[i]));
     CK(cudaMemcpyAsync(b->d_freq, freq_hz, nf * sizeof(double), cudaMemcpyHostToDevice, c->stream));
     CK(cudaMemcpyAsync(b->d_mode, mode, nf * sizeof(int), cudaMemcpyHostToDevice, c->stream));
     CK(cudaStreamSynchronize(c->stream));  // host buffers may be released by the caller on return
@@ -766,6 +784,7 @@ int torj_bundle_create_from_launchers(torj_ctx* c, int32_t n_launchers, const do
     torj_bundle* b = new torj_bundle();
     Guard<torj_bundle, torj_bundle_destroy> guard(b);
     b->ctx = c; b->n = n; b->per_ray_fm = 1;
+    b->w_max = -1.0;  // weights of order 1 made on the device; an exact booking out of range is refused there
     CK(cudaMalloc(&b->d_pos, 3 * n * sizeof(double)));
     CK(cudaMalloc(&b->d_dir, 3 * n * sizeof(double)));
     CK(cudaMalloc(&b->d_w, n * sizeof(double)));
@@ -838,7 +857,7 @@ void torj_bundle_destroy(torj_bundle* b) {
     cudaFree(b->d_s0); cudaFree(b->d_psil); cudaFree(b->d_Pf); cudaFree(b->d_Pdep); cudaFree(b->d_status); cudaFree(b->d_npts);
     cudaFree(b->d_hand); cudaFree(b->d_segdone); cudaFree(b->d_left); cudaFree(b->d_life);
     cudaFree(b->d_queue); cudaFree(b->d_counters); cudaFree(b->d_edges); cudaFree(b->d_bins); cudaFree(b->d_dV);
-    cudaFree(b->d_profile);
+    cudaFree(b->d_profile); cudaFree(b->d_xs);
     cudaFree(b->d_beam);
     cudaFree(b->d_set); cudaFree(b->d_beam_plasma);
     cudaFree(b->d_ufinal);
@@ -917,6 +936,8 @@ static int check_plasma_set(const char* fn, const torj_ctx* c, int32_t n_pl, con
     return 0;
 }
 
+static int finalize(torj_bundle* b);
+
 // torj_bundle_trace (one plasma) and torj_bundle_trace_plasmas: beam q through pls[beam_plasma[q]] when n_pl > 1
 static int bundle_trace(torj_bundle* b, int32_t n_pl, const torj_plasma* const* pls, const int32_t* beam_plasma,
                         const torj_options* opt, double s_max, int32_t n_psi, const double* psi_edges) {
@@ -947,6 +968,9 @@ static int bundle_trace(torj_bundle* b, int32_t n_pl, const torj_plasma* const* 
         FAIL("torj_bundle_trace: the warm model runs with 1 or 32 lanes per ray");
     if (od.absorption_model == 1 && od.max_harmonic > 3) FAIL("torj_bundle_trace: max_harmonic > 3 belongs to the Albajar model; the warm model takes its harmonics from larmornumber");
     if (!(s_max > 0.0)) FAIL("torj_bundle_trace: s_max must be > 0");
+    const bool xs = c->exact_sum != 0;
+    if (xs && b->w_max > TORJ_XS_WMAX)
+        FAIL("torj_bundle_trace: exact sum mode takes ray weights of magnitude <= 2^40 (and no NaN)");
     if (set_device(c)) return 1;
     cudaStream_t st = c->stream;
     if (b->n_psi != n_psi || b->prof_rows != b->n_beams) {
@@ -1013,6 +1037,18 @@ static int bundle_trace(torj_bundle* b, int32_t n_pl, const torj_plasma* const* 
         P.beam_plasma = b->d_beam_plasma; P.beam_id = b->d_beam;
     }
     CK(cudaMemsetAsync(b->d_bins, 0, (size_t)b->n_beams * (n_psi + 2) * sizeof(double), st));
+    const size_t xs_words = torj_xs_buffer_words((size_t)b->n_beams * (n_psi + 2));
+    b->xs_last = false;
+    if (xs) {
+        if (b->xs_words != xs_words) {
+            CK(cudaStreamSynchronize(st));
+            cudaFree(b->d_xs);
+            b->d_xs = nullptr; b->xs_words = 0;
+            CK(cudaMalloc(&b->d_xs, xs_words * sizeof(long long)));
+            b->xs_words = xs_words;
+        }
+        CK(cudaMemsetAsync(b->d_xs, 0, xs_words * sizeof(long long), st));
+    }
     CK(cudaMemsetAsync(b->d_queue, 0, sizeof(unsigned long long), st));
     CK(cudaMemsetAsync(b->d_counters, 0, 8 * sizeof(unsigned long long), st));
     if (b->traj_count > 0) CK(cudaMemsetAsync(b->d_tprof, 0, (size_t)b->traj_count * n_psi * sizeof(double), st));
@@ -1028,6 +1064,7 @@ static int bundle_trace(torj_bundle* b, int32_t n_pl, const torj_plasma* const* 
     a.J.s = b->d_ts; a.J.xyz = b->d_txyz; a.J.P = b->d_tP; a.J.dP = b->d_tdP; a.J.prof = b->d_tprof;
     a.n_psi = n_psi; a.n_beams = b->n_beams; a.beam_id = b->d_beam; a.psi_edges = b->d_edges; a.bins = b->d_bins; a.next_ray = b->d_queue; a.counters = b->d_counters;
     a.warm_tab = c->d_warm_tab; a.u_final = b->d_ufinal;
+    a.xs = xs ? b->d_xs + TORJ_XS_STAT : nullptr;
     const int model = od.absorption_model;
     // Several lanes per ray when the bundle cannot fill the GPU with one thread per ray — then the time is one ray's
     // latency, and splitting the quadrature nodes over the lanes of a group shortens exactly that. Measured
@@ -1052,7 +1089,7 @@ static int bundle_trace(torj_bundle* b, int32_t n_pl, const torj_plasma* const* 
     // default kernels do not carry the code
     void (*kern)(TraceArgs);
     const bool high = od.max_harmonic > 3;
-    kern = pick_trace_kernel(od.scheme, high, model, lpr, set);
+    kern = pick_trace_kernel(od.scheme, high, model, lpr, set, xs);
     CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, kern, TORJ_TPB, smem));
     if (bps < 1) FAIL("torj_bundle_trace: trace kernel does not fit on an SM");
@@ -1094,8 +1131,18 @@ static int bundle_trace(torj_bundle* b, int32_t n_pl, const torj_plasma* const* 
     CK(cudaGetLastError());
     CK(cudaEventRecord(c->ev1, st));
     c->ev_valid = true;
-    k_finalize<<<(unsigned)(((size_t)b->n_beams * (n_psi + 2) + 127) / 128), 128, 0, st>>>(b->d_bins, b->d_dV, n_psi, b->n_beams,
-                                                                                         (int)set, b->d_profile);
+    b->xs_last = xs;
+    return finalize(b);
+}
+
+// bins (or, after an exact-sum trace, the words) -> d_profile, normalised by the dV rows of the last trace
+static int finalize(torj_bundle* b) {
+    torj_ctx* c = b->ctx;
+    const unsigned grid = (unsigned)(((size_t)b->n_beams * (b->n_psi + 2) + 127) / 128);
+    if (b->xs_last)
+        k_finalize_exact<<<grid, 128, 0, c->stream>>>(b->d_xs + TORJ_XS_STAT, b->d_dV, b->n_psi, b->n_beams, (int)(b->dV_rows > 1), b->d_profile);
+    else
+        k_finalize<<<grid, 128, 0, c->stream>>>(b->d_bins, b->d_dV, b->n_psi, b->n_beams, (int)(b->dV_rows > 1), b->d_profile);
     c->launches++;
     CK(cudaGetLastError());
     return 0;
@@ -1132,7 +1179,20 @@ int torj_bundle_results(torj_bundle* b, double* dP_dV, double* deposited_power, 
     if (status) CK(cudaMemcpyAsync(status, b->d_status, b->n * sizeof(int), cudaMemcpyDeviceToHost, st));
     unsigned long long cn[8];
     CK(cudaMemcpyAsync(cn, b->d_counters, sizeof cn, cudaMemcpyDeviceToHost, st));
+    long long xst[TORJ_XS_STAT] = {0, 0};
+    if (b->xs_last)
+        CK(cudaMemcpyAsync(xst, b->d_xs, sizeof xst, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
+    if (!torj_xs_valid(xst[0], xst[1])) {
+        char msg[256];
+        if (xst[1])
+            snprintf(msg, sizeof msg, "torj_bundle_results: exact sum: %lld bookings outside the accumulator's range (|w dP| >= 2^64 "
+                     "or NaN); the profile is NaN", xst[1]);
+        else
+            snprintf(msg, sizeof msg, "torj_bundle_results: exact sum: %lld bookings exceed the accumulator's bound of 2^34; "
+                     "the profile is NaN", xst[0]);
+        FAIL(msg);
+    }
     for (int q = 0; q < b->n_beams; ++q) {
         if (dP_dV) memcpy(dP_dV + (size_t)q * b->n_psi, prof.data() + q * row, b->n_psi * sizeof(double));
         if (deposited_power) deposited_power[q] = prof[q * row + b->n_psi];
@@ -1473,6 +1533,13 @@ int torj_multi_configure(torj_multi* m, int32_t sharding, int64_t block_rays, in
     return 0;
 }
 
+int torj_multi_set_exact_sum(torj_multi* m, int32_t on) {
+    if (!m) FAIL("torj_multi_set_exact_sum: torj_multi is NULL");
+    if (on != 0 && on != 1) FAIL("torj_multi_set_exact_sum: on must be 0 (floating-point atomics) or 1 (exact sum)");
+    for (auto* c : m->ctx) c->exact_sum = on;
+    return 0;
+}
+
 int torj_multi_abs_init(torj_multi* m, int32_t n, const double* nodes, const double* weights) {
     for (auto* c : m->ctx)
         if (int rc = torj_abs_init(c, n, nodes, weights)) return rc;
@@ -1613,8 +1680,40 @@ static int multi_trace(torj_multi* m, const char* fn, bool set_api, int32_t n_pl
     bool all_ok = true;
     for (int d = 0; d < used; ++d) all_ok = all_ok && rcs[d] == 0;
 
-    // ---- phase B (the collective only when every device got through phase A: a missing rank would hang the others)
+    // Exact sum: the devices' words are summed as integers (status words included), before any conversion, so the profile
+    // is that of one device tracing the whole bundle. Without NCCL on the host; device 0 then converts the sum.
+    const bool xs = m->ctx[0]->exact_sum != 0;
     const bool do_nccl = all_ok && want_nccl;
+    if (all_ok && xs && !do_nccl && used > 1) {
+        const size_t nw = m->ctx[0]->ws->xs_words;
+        std::vector<std::vector<unsigned long long>> hw(used, std::vector<unsigned long long>(nw));
+        m->run(used, [&](int d) {
+            torj_ctx* c = m->ctx[d];
+            auto fail = [&](int rc) { rcs[d] = rc; errs[d] = g_err; };
+            if (set_device(c)) return fail(1);
+            cudaError_t e = cudaMemcpyAsync(hw[d].data(), c->ws->d_xs, nw * sizeof(long long), cudaMemcpyDeviceToHost, c->stream);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+            if (e != cudaSuccess) { g_err = std::string("exact sum: ") + cudaGetErrorString(e); return fail(1); }
+        });
+        for (int d = 0; d < used; ++d) all_ok = all_ok && rcs[d] == 0;
+        if (all_ok) {
+            for (int d = 1; d < used; ++d)
+                for (size_t k = 0; k < nw; ++k) hw[0][k] += hw[d][k];  // two's complement: a signed sum, in any order
+            torj_ctx* c0 = m->ctx[0];
+            torj_bundle* b0 = c0->ws;
+            int rc = set_device(c0);
+            if (!rc) {
+                cudaError_t e = cudaMemcpyAsync(b0->d_xs, hw[0].data(), nw * sizeof(long long), cudaMemcpyHostToDevice, c0->stream);
+                if (e == cudaSuccess) e = cudaStreamSynchronize(c0->stream);
+                if (e != cudaSuccess) { g_err = std::string("exact sum: ") + cudaGetErrorString(e); rc = 1; }
+            }
+            if (!rc) rc = finalize(b0);
+            if (rc) { rcs[0] = rc; errs[0] = g_err; all_ok = false; }
+        }
+    }
+
+    // ---- phase B (the collective only when every device got through phase A: a missing rank would hang the others)
+    const bool one = do_nccl || xs;  // every device's (or device 0's) profile is the whole bundle's
     if (all_ok) m->run(used, [&](int d) {
         torj_ctx* c = m->ctx[d];
         torj_bundle* b = c->ws;
@@ -1622,7 +1721,11 @@ static int multi_trace(torj_multi* m, const char* fn, bool set_api, int32_t n_pl
         auto fail = [&](int rc) { rcs[d] = rc; errs[d] = g_err; };
         if (set_device(c)) return fail(1);
         const int64_t n = b->n;
-        if (do_nccl) {
+        if (do_nccl && xs) {
+            ncclResult_t r = nccl_api().AllReduce(b->d_xs, b->d_xs, b->xs_words, ncclInt64, ncclSum, m->comm[d], c->stream);
+            if (r != ncclSuccess) { g_err = std::string("ncclAllReduce: ") + nccl_api().GetErrorString(r); return fail(3); }
+            if (int rc = finalize(b)) return fail(rc);
+        } else if (do_nccl) {
             ncclResult_t r = nccl_api().AllReduce(b->d_profile, b->d_profile, (size_t)n_beams * prow, ncclDouble, ncclSum,
                                                   m->comm[d], c->stream);
             if (r != ncclSuccess) { g_err = std::string("ncclAllReduce: ") + nccl_api().GetErrorString(r); return fail(3); }
@@ -1630,7 +1733,7 @@ static int multi_trace(torj_multi* m, const char* fn, bool set_api, int32_t n_pl
         memset(&cnts[d], 0, sizeof(torj_counters));
         prof[d].assign((size_t)n_beams * prow, 0.0);
         std::vector<double> pr((size_t)n_beams * n_psi), dp(n_beams);
-        int rc = torj_bundle_results(b, (!do_nccl || d == 0) ? pr.data() : nullptr, (!do_nccl || d == 0) ? dp.data() : nullptr,
+        int rc = torj_bundle_results(b, (!one || d == 0) ? pr.data() : nullptr, (!one || d == 0) ? dp.data() : nullptr,
                                      P_final ? S.Pf : nullptr, P_dep ? S.Pd : nullptr, n_points ? S.np : nullptr,
                                      status ? S.st : nullptr, &cnts[d]);
         if (rc) return fail(rc);
@@ -1675,8 +1778,8 @@ static int multi_trace(torj_multi* m, const char* fn, bool set_api, int32_t n_pl
     for (int q = 0; q < n_beams; ++q) {
         for (int j = 0; j < n_psi + 1; ++j) {
             double sum = 0.0;
-            if (do_nccl) sum = prof[0][q * prow + j];  // every device holds the all-reduced vector; device 0's copy is returned
-            else for (int d = 0; d < used; ++d) sum += prof[d][q * prow + j];  // device order: bit-reproducible
+            if (one) sum = prof[0][q * prow + j];  // device 0 holds the whole bundle's profile
+            else for (int d = 0; d < used; ++d) sum += prof[d][q * prow + j];  // device order (each device's own sums are not ordered)
             if (j < n_psi) { if (dP_dV) dP_dV[(size_t)q * n_psi + j] = sum; }
             else if (deposited_power) deposited_power[q] = sum;
         }

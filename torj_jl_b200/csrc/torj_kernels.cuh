@@ -8,6 +8,7 @@
 #include "torj_device.cuh"
 #include "torj_warm.cuh"
 #include "torj_handoff.cuh"
+#include "torj_exactsum.cuh"
 
 #include <type_traits>
 
@@ -299,6 +300,9 @@ struct TraceArgs {
     const int* life;                  // [n] predicted cost of every ray in rounds (segments, those inside the absorbing layer weighted)
     const int* lmax;                  // max of life[]
     PlasmaSetDev P;                   // k_trace<..., SET = true> only (last member: the other instantiations keep their layout)
+    // exact-sum mode (torj_exactsum.cuh), k_trace<..., XS = true> only: every booking goes, exactly, into
+    // xs[bin * TORJ_XS_WORDS ...] (bins as in `bins`); the buffer's status words are xs[-2], xs[-1]
+    long long* xs;
 };
 #define TORJ_HAND_D 20
 
@@ -334,13 +338,43 @@ template <> struct Scheme<1> { static constexpr int S = 4; static constexpr int 
 // Runge-Kutta stage derivatives k[S][7] live in shared memory, not in (L1-backed) local memory, stored as 4 double2 per
 // stage and thread (8th slot unused), so that a stage is read with 4 LDS.128 instead of 7 LDS.64
 #define TORJ_K_WORDS (56 * TORJ_TPB)  // doubles of stage storage per CTA
-#define TORJ_PARK_SLOTS 9  // doubles per thread of parked per-segment / per-ray scalars (7 doubles + 3 ints, rounded up)
+#define TORJ_PARK_SLOTS 9  // doubles per thread of parked per-segment / per-ray scalars (7 doubles + 4 ints)
 #define TORJ_LIFE_HARM_COST 0.25  // k_predict_life: rounds one evaluated harmonic integral per pilot point adds to a ray's predicted
                                   // cost (segments inside the absorbing layer take longer). 1/16 and 1/8 shards of the 1 M-ray sweep:
                                   // 0 -> 174.8 / 299.2 ms, 0.25 -> 166.7 / 288.9, 0.5 -> 168.1 / 291.0, 0.75 -> 176.3 / 295.3; beam unchanged
 #define TORJ_MINB 2  // resident CTAs per SM the register allocation is bounded for (2 -> 255 regs, 3 -> 168, 4 -> 128)
 // per-ray status codes of include/torj_cuda.h: everything but OK(0), LEFT_GRID(3) and TRAJ_TRUNCATED(6) ends the ray
 #define TORJ_FATAL(s) ((s) != 0 && (s) != 6 && (s) != 3)
+
+// The lane's count of exact bookings: k_trace's parked int slot PKI(3) (flushed into the status word before it can wrap,
+// the rest at the end of k_trace)
+__device__ __forceinline__ unsigned* xs_count_slot() {
+    extern __shared__ __align__(16) double smem[];
+    return reinterpret_cast<unsigned*>(smem + TORJ_K_WORDS + 7 * TORJ_TPB) + 3 * TORJ_TPB + threadIdx.x;
+}
+
+// One exact booking (exact-sum mode): v's digits into the words of bin `bin`, fire-and-forget integer REDs. Out of line and
+// with few arguments, by value, so the hot loop carries only the call. The status words precede the words.
+__device__ __noinline__ void xs_book(long long* xs, size_t bin, double v) {
+    unsigned long long* stat = reinterpret_cast<unsigned long long*>(xs - TORJ_XS_STAT);
+    unsigned* nb = xs_count_slot();
+    const TorjXsSplit s = torj_xs_split(v);
+    if (!s.ok) { atomicAdd(&stat[1], 1ull); return; }
+    unsigned long long* w = reinterpret_cast<unsigned long long*>(xs + bin * TORJ_XS_WORDS + s.k);
+#pragma unroll
+    for (int j = 0; j < 3; ++j)
+        if (s.d[j]) atomicAdd(&w[j], (unsigned long long)s.d[j]);  // two's complement: a signed add
+    const unsigned c = *nb + 1;
+    if (c == 0x80000000u) { atomicAdd(&stat[0], (unsigned long long)c); *nb = 0; }
+    else *nb = c;
+}
+
+// A retiring ray's two per-beam bookings, w P_dep and w, into the bins row_bin + n_psi, + n_psi + 1: one call site less
+// in k_trace
+__device__ __noinline__ void xs_book_ray(long long* xs, size_t row_bin, double w_pdep, double w) {
+    xs_book(xs, row_bin, w_pdep);
+    xs_book(xs, row_bin + 1, w);
+}
 
 // Integrator phases. Every trip of the kernel's main loop evaluates the RHS exactly once per lane that holds a
 // ray, whatever that lane's phase, so the expensive code is always warp-converged; the cheap phase-specific
@@ -362,7 +396,7 @@ enum { ACT_NONE = 0, ACT_BEGIN_SEGMENT = 1, ACT_BEGIN_STEP = 2, ACT_END_SEGMENT 
 //   whose alpha costs ~100x the rest of the RHS.
 // SET = true: a plasma set (a.P). The grid comes from a.T as always; the table base is per lane, bound with the ray
 //   (a ray's plasma is that of its beam), so rays of several equilibria share one launch.
-template <int SCH, bool HIGH = false, int MODEL = 0, int LPR = 1, bool SET = false>
+template <int SCH, bool HIGH = false, int MODEL = 0, int LPR = 1, bool SET = false, bool XS = false>
 __global__ void __launch_bounds__(TORJ_TPB, TORJ_MINB) k_trace(TraceArgs a) {
     exp_tab_init();
     constexpr bool COOP = LPR == 32;
@@ -421,6 +455,7 @@ __global__ void __launch_bounds__(TORJ_TPB, TORJ_MINB) k_trace(TraceArgs a) {
     int& last_stat = PKI(1);
     unsigned int& rays_ok = *reinterpret_cast<unsigned int*>(&PKI(2));
     ray = -1; tj = -1; s0 = 0.0; dt0 = 0.0; d1 = 0.0; tot_dep = 0.0; tot_w = 0.0; seg = 0; last_stat = 0; rays_ok = 0;
+    if constexpr (XS) PKI(3) = 0;  // exact-sum bookings of this lane (xs_count_slot)
     // warm model, one ray per lane: shared-memory slots where a lane's quadrature sums wait for the serial solve
     double* wstash = smem + TORJ_K_WORDS + TORJ_PARK_SLOTS * TORJ_TPB + threadIdx.x;
     int phase = PH_IDLE, st = 0;
@@ -448,7 +483,8 @@ __global__ void __launch_bounds__(TORJ_TPB, TORJ_MINB) k_trace(TraceArgs a) {
     auto sink = [&](int shell, double dP) {
         pdep += dP;
         if (!writer) return;
-        atomicAdd(&beam_bins[shell], wgt * dP);
+        if constexpr (XS) xs_book(a.xs, (size_t)(beam_bins - a.bins) + shell, wgt * dP);
+        else atomicAdd(&beam_bins[shell], wgt * dP);
         if (tj >= 0) atomicAdd(&a.J.prof[tj * n_psi + shell], dP);  // (a ray may change SMs between segments)
     };
     auto put_point = [&](double s, const double* xx, double P, double dP) {
@@ -841,7 +877,9 @@ __global__ void __launch_bounds__(TORJ_TPB, TORJ_MINB) k_trace(TraceArgs a) {
                         if (!TORJ_FATAL(rstat)) {
                             a.B.P_final[ray] = u[6];
                             a.B.P_dep[ray] = pdep;
-                            if (a.n_beams > 1) {
+                            if constexpr (XS) {  // per ray, also with one beam: the block sum below would round
+                                xs_book_ray(a.xs, (size_t)(beam_bins - a.bins) + n_psi, wgt * pdep, wgt);
+                            } else if (a.n_beams > 1) {
                                 atomicAdd(&beam_bins[n_psi], wgt * pdep);
                                 atomicAdd(&beam_bins[n_psi + 1], wgt);
                             } else {
@@ -938,8 +976,14 @@ __global__ void __launch_bounds__(TORJ_TPB, TORJ_MINB) k_trace(TraceArgs a) {
         for (int q = 0; q < 8; ++q) atomicAdd(&s_cnt[q], c6[q]);
     }
     __syncthreads();
-    if (threadIdx.x < 2) atomicAdd(&a.bins[n_psi + threadIdx.x], s_tot[threadIdx.x]);
+    if (threadIdx.x < 2 && !XS) atomicAdd(&a.bins[n_psi + threadIdx.x], s_tot[threadIdx.x]);  // exact mode booked per ray
     if (threadIdx.x < 8) atomicAdd(&a.counters[threadIdx.x], s_cnt[threadIdx.x]);
+    if constexpr (XS) {  // the bookings not yet flushed by xs_book
+        unsigned long long nb = (unsigned)PKI(3);
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) nb += __shfl_down_sync(FULL, nb, off);
+        if (lane == 0 && nb) atomicAdd(reinterpret_cast<unsigned long long*>(a.xs - TORJ_XS_STAT), nb);
+    }
 #undef KK
 #undef PK
 #undef PKI
@@ -999,6 +1043,22 @@ __global__ void k_finalize(const double* bins, const double* dV, int n_psi, int 
     if (j < n_psi - 1) profile[g] = bins[g] / dV[j];
     else if (j == n_psi - 1) profile[g] = 0.0;
     else profile[g] = bins[g];
+}
+
+// k_finalize of the exact-sum mode: bin g is the correctly rounded value of its words xs[g * 8 ..] (status words at xs[-2],
+// xs[-1]); same layout rules. An invalid buffer (a refused booking, or more bookings than the words' headroom allows)
+// yields NaN everywhere; the results call reports it.
+__global__ void k_finalize_exact(const long long* xs, const double* dV, int n_psi, int n_beams, int dV_per_beam, double* profile) {
+    long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const long long nb = (long long)n_beams * (n_psi + 2);
+    if (g >= nb) return;
+    int j = (int)(g % (n_psi + 2));
+    if (dV_per_beam) dV += (g / (n_psi + 2)) * n_psi;
+    const long long* st = xs - TORJ_XS_STAT;
+    const double v = torj_xs_valid(st[0], st[1]) ? torj_xs_to_double(xs + g * TORJ_XS_WORDS) : __longlong_as_double(0x7ff8000000000000ll);
+    if (j < n_psi - 1) profile[g] = v / dV[j];
+    else if (j == n_psi - 1) profile[g] = 0.0;
+    else profile[g] = v;
 }
 
 // ------------------------------------------------------------------------------------------------

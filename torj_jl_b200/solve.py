@@ -83,16 +83,20 @@ def bundle_result(m):
 
 
 def trace_bundle(plasma, ray_positions, ray_directions, ray_weights, f, mode, s_max, psi_dP_dV, *,
-                 options=None, ctx=None, trajectories=None, traj_max_pts=None, beam_id=None, n_beams=1, beam_plasma=None):
+                 options=None, ctx=None, trajectories=None, traj_max_pts=None, beam_id=None, n_beams=1, beam_plasma=None,
+                 exact_sum=False):
     """One torj_trace call on host buffers. trajectories: None or (first, count).
     beam_id/n_beams: rays of several beams in one bundle -> dP_dV[n_beams, n_psi], deposited_power[n_beams].
     plasma: a Plasma, or a sequence of Plasma on one (R,Z) grid with beam_plasma[n_beams] naming the plasma of every beam
-    (torj_trace_plasmas; keep each beam's rays contiguous)."""
+    (torj_trace_plasmas; keep each beam's rays contiguous).
+    exact_sum: book the profile in an exact fixed-point sum (torj_ctx_set_exact_sum), so dP_dV and deposited_power are
+    bit-identical under any schedule, ray order and device count; weights |w| <= 2^40."""
     pls = _plasma_set(plasma, beam_plasma)
     m = marshal_bundle(ray_positions, ray_directions, ray_weights, f, mode, psi_dP_dV, beam_id, n_beams,
                        n_plasmas=len(pls) if pls else 1, beam_plasma=beam_plasma)
     ctx = ctx or _lib.context()
     L = _lib.lib()
+    _lib.check(L.torj_ctx_set_exact_sum(ctx, int(bool(exact_sum))))
     n, psi, o = m["n"], m["psi"], m["out"]
     opt = options or _lib.default_options()
     t_first, t_count = trajectories if trajectories else (0, 0)
@@ -122,11 +126,13 @@ def cylindrical_state(xyz, P):
         return np.hypot(x, y), np.arctan2(y, x), -np.log(P)
 
 
-def make_ray(plasma: Plasma, x0, N_vacuum, f, mode, s_max, psi_dP_dV, *, options=None, ctx=None):
+def make_ray(plasma: Plasma, x0, N_vacuum, f, mode, s_max, psi_dP_dV, *, options=None, ctx=None, exact_sum=False):
     """make_ray(plasma, x0, N_vacuum, f, mode, s_max, psi_dP_dV) -> (s, u, P_beam, dP_dV_ray, deposited_power)
-    — reference src/solve.jl:135-136,180.  u is the list of positions (first two: launch point, plasma entry)."""
+    — reference src/solve.jl:135-136,180.  u is the list of positions (first two: launch point, plasma entry).
+    exact_sum: see trace_bundle."""
     r = trace_bundle(plasma, np.asarray(x0, dtype=np.float64)[None, :], np.asarray(N_vacuum, dtype=np.float64)[None, :],
-                     [1.0], float(f), int(mode), s_max, psi_dP_dV, options=options, ctx=ctx, trajectories=(0, 1))
+                     [1.0], float(f), int(mode), s_max, psi_dP_dV, options=options, ctx=ctx, trajectories=(0, 1),
+                     exact_sum=exact_sum)
     st = int(r["status"][0])
     if st not in (0, 3):
         # the reference raises AssertionError / MethodError at src/solve.jl:32,138,141
@@ -138,15 +144,16 @@ def make_ray(plasma: Plasma, x0, N_vacuum, f, mode, s_max, psi_dP_dV, *, options
 
 
 def make_beam(plasma: Plasma, r, phi, z, steering_angle_tor, steering_angle_pol, spot_size, inverse_curvature_radius,
-              f, mode, s_max, psi_dP_dV, *, options=None, ctx=None, **kwargs):
+              f, mode, s_max, psi_dP_dV, *, options=None, ctx=None, exact_sum=False, **kwargs):
     """make_beam(...) -> (arc_lengths, trajectories, ray_powers, dP_dV, deposited_power, ray_weights)
-    — reference src/solve.jl:209-210,241; kwargs go to launch_peripheral_rays (src/solve.jl:216-217)."""
+    — reference src/solve.jl:209-210,241; kwargs go to launch_peripheral_rays (src/solve.jl:216-217).
+    exact_sum: see trace_bundle."""
     N0 = pol_tor_angles_2_vector(steering_angle_pol, steering_angle_tor)  # src/solve.jl:211
     x0 = np.array([r * np.cos(phi), r * np.sin(phi), z])                  # src/solve.jl:212-215
     pos, dirs, wts = launch_peripheral_rays(x0, N0, spot_size, inverse_curvature_radius, f, **kwargs)
     n = len(wts)
     res = trace_bundle(plasma, pos, dirs, wts, float(f), int(mode), s_max, psi_dP_dV, options=options, ctx=ctx,
-                       trajectories=(0, n))
+                       trajectories=(0, n), exact_sum=exact_sum)
     bad = np.nonzero(~np.isin(res["status"], (0, 3)))[0]
     if len(bad):
         raise AssertionError(f"ray {int(bad[0])}: " + STATUS_TEXT.get(int(res['status'][bad[0]]), "failed"))
@@ -173,7 +180,7 @@ def _launcher_plasmas(plasma, launchers):
     return pls, bp
 
 
-def _make_beams_device(plasma, launchers, s_max, psi_dP_dV, options, ctx, N_rings=3, min_azimuthal_points=5,
+def _make_beams_device(plasma, launchers, s_max, psi_dP_dV, options, ctx, exact_sum, N_rings=3, min_azimuthal_points=5,
                        normalize_weight_sum=True):
     """Rays generated on the GPU (torj_bundle_create_from_launchers), traced and reduced there; only launcher
     parameters go in and profiles / per-ray scalars come out."""
@@ -201,6 +208,7 @@ def _make_beams_device(plasma, launchers, s_max, psi_dP_dV, options, ctx, N_ring
         n = int(n.value)
         psi = np.ascontiguousarray(psi_dP_dV, dtype=np.float64)
         opt = options or _lib.default_options()
+        _lib.check(L.torj_ctx_set_exact_sum(ctx, int(bool(exact_sum))))
         if pls is None:
             _lib.check(L.torj_bundle_trace(bh, plasma.handle(ctx), C.byref(opt), float(s_max), len(psi), _p(psi)))
         else:
@@ -222,15 +230,15 @@ def _make_beams_device(plasma, launchers, s_max, psi_dP_dV, options, ctx, N_ring
     return prof, dep, [wt[i * per:(i + 1) * per] for i in range(nl)], [Pf[i * per:(i + 1) * per] for i in range(nl)], res
 
 
-def make_beams(plasma, launchers, s_max, psi_dP_dV, *, options=None, ctx=None, device_launch=False, **kwargs):
+def make_beams(plasma, launchers, s_max, psi_dP_dV, *, options=None, ctx=None, device_launch=False, exact_sum=False, **kwargs):
     """Batched make_beam for scans: `launchers` is a sequence of dicts with the positional arguments of make_beam
     (r, phi, z, steering_angle_tor, steering_angle_pol, spot_size, inverse_curvature_radius, f, mode). All beams are
     traced in ONE device call; returns (dP_dV[n_beams, n_psi], deposited_power[n_beams], ray_weights per beam,
     P_final per beam). Equivalent to a host loop over make_beam (reference src/solve.jl:209-242) without trajectories.
     `plasma` may be a sequence of Plasma on one (R,Z) grid: a launcher's "plasma" key (default 0) picks the one its beam
-    is traced through, and its profile row is normalised by that plasma's volume."""
+    is traced through, and its profile row is normalised by that plasma's volume. exact_sum: see trace_bundle."""
     if device_launch:
-        return _make_beams_device(plasma, launchers, s_max, psi_dP_dV, options, ctx, **kwargs)
+        return _make_beams_device(plasma, launchers, s_max, psi_dP_dV, options, ctx, exact_sum, **kwargs)
     pls, bp = _launcher_plasmas(plasma, launchers)
     P, D, W, F, M, B = [], [], [], [], [], []
     for b, L in enumerate(launchers):
@@ -242,21 +250,22 @@ def make_beams(plasma, launchers, s_max, psi_dP_dV, *, options=None, ctx=None, d
         B.append(np.full(len(w), b, dtype=np.int32))
     res = trace_bundle(pls if pls is not None else plasma, np.concatenate(P), np.concatenate(D), np.concatenate(W),
                        np.concatenate(F), np.concatenate(M), s_max, psi_dP_dV, options=options, ctx=ctx,
-                       beam_id=np.concatenate(B), n_beams=len(launchers), beam_plasma=bp)
+                       beam_id=np.concatenate(B), n_beams=len(launchers), beam_plasma=bp, exact_sum=exact_sum)
     off = np.cumsum([0] + [len(w) for w in W])
     dP = np.atleast_2d(res["dP_dV"]); dep = np.atleast_1d(res["deposited_power"])
     return dP, dep, W, [res["P_final"][off[i]:off[i + 1]] for i in range(len(W))], res
 
 
 def make_beam_series(plasmas, r, phi, z, steering_angle_tor, steering_angle_pol, spot_size, inverse_curvature_radius,
-                     f, mode, s_max, psi_dP_dV, *, options=None, ctx=None, trajectories=None, **kwargs):
+                     f, mode, s_max, psi_dP_dV, *, options=None, ctx=None, trajectories=None, exact_sum=False, **kwargs):
     """The reference's make_beam (src/solve.jl:209-242) of one launcher on each plasma of a sequence on one (R,Z) grid
     (time slices, an uncertainty ensemble), in ONE device call (torj_trace_plasmas). The beam's rays go in once per
     plasma, contiguous. Returns (dP_dV[n_plasmas, n_psi], deposited_power[n_plasmas], ray_weights, P_final[n_plasmas, n],
     res) where res holds the per-ray arrays over the whole bundle (plasma k's rays at [k n, (k+1) n)). No trajectories
-    unless `trajectories` = (first, count) over that bundle: the window would otherwise hold n_plasmas beams."""
+    unless `trajectories` = (first, count) over that bundle: the window would otherwise hold n_plasmas beams.
+    exact_sum: see trace_bundle."""
     def trace(*a, **k):
-        return trace_bundle(*a, options=options, ctx=ctx, trajectories=trajectories, **k)
+        return trace_bundle(*a, options=options, ctx=ctx, trajectories=trajectories, exact_sum=exact_sum, **k)
 
     return beam_series(trace, plasmas, r, phi, z, steering_angle_tor, steering_angle_pol, spot_size, inverse_curvature_radius,
                        f, mode, s_max, psi_dP_dV, **kwargs)
