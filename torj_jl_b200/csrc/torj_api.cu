@@ -38,6 +38,42 @@ static thread_local std::string g_err;
 
 #define FAIL(msg) do { g_err = (msg); return 2; } while (0)
 
+// Owning array of size() T in device memory (dev_array) or page-locked host memory (pinned_array); it converts to its
+// pointer. The destructor frees it, so whoever destroys an owner makes the owning device current first.
+template <bool PINNED>
+struct CudaFree {
+    void operator()(void* p) const { PINNED ? cudaFreeHost(p) : cudaFree(p); }
+};
+template <class T, bool PINNED>
+class cuda_array {
+    std::unique_ptr<T, CudaFree<PINNED>> p_;
+    size_t n_ = 0;
+
+  public:
+    operator T*() const { return p_.get(); }
+    size_t size() const { return n_; }
+    // Unchanged size: nothing. Otherwise wait for st (a kernel or copy on it may still use the old buffer), free, then
+    // allocate. A failed allocation leaves the array empty.
+    cudaError_t resize(size_t count, cudaStream_t st) {
+        if (count == n_) return cudaSuccess;
+        cudaError_t e = p_ ? cudaStreamSynchronize(st) : cudaSuccess;
+        if (e != cudaSuccess) return e;
+        p_.reset();
+        n_ = 0;
+        if (count == 0) return cudaSuccess;
+        T* raw = nullptr;
+        e = PINNED ? cudaHostAlloc(&raw, count * sizeof(T), cudaHostAllocDefault) : cudaMalloc(&raw, count * sizeof(T));
+        if (e != cudaSuccess) return e;
+        p_.reset(raw);
+        n_ = count;
+        return cudaSuccess;
+    }
+};
+template <class T>
+using dev_array = cuda_array<T, false>;
+template <class T>
+using pinned_array = cuda_array<T, true>;
+
 struct torj_ctx {
     int device = 0;
     cudaStream_t stream = nullptr;
@@ -48,7 +84,7 @@ struct torj_ctx {
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;  // bracket the last k_trace launch
     bool ev_valid = false;
     struct torj_bundle* ws = nullptr;  // workspace of the one-shot torj_trace call, kept between calls
-    double2* d_warm_tab = nullptr;     // set_extv! tables of the warm-plasma model (reference src/general_absorption.jl:8-13)
+    dev_array<double2> d_warm_tab;     // set_extv! tables of the warm-plasma model (reference src/general_absorption.jl:8-13)
     int exact_sum = 0;                 // torj_ctx_set_exact_sum: later traces book profiles exactly (torj_exactsum.cuh)
 };
 
@@ -67,8 +103,8 @@ struct torj_plasma {
     torj_ctx* ctx = nullptr;
     uint64_t id = 0;  // unique per created plasma (addresses can be recycled)
     DevTables T{};
-    double2* dA = nullptr;  // [nodes][3]
-    DevTables* dT = nullptr;  // T mirrored in global memory
+    dev_array<double2> dA;  // [nodes][3]
+    dev_array<DevTables> dT;  // T mirrored in global memory
     // host copy of the V(psi_N) spline (reference src/plasma.jl:42-44)
     std::vector<double> vol_c;
     int n_vol = 0;
@@ -80,60 +116,45 @@ struct torj_bundle {
     int64_t n = 0;
     BundleDev B{};
     int per_ray_fm = 0;
-    // owned device buffers
-    double *d_pos = nullptr, *d_dir = nullptr, *d_w = nullptr, *d_freq = nullptr, *d_u0 = nullptr, *d_s0 = nullptr,
-           *d_psil = nullptr, *d_Pf = nullptr, *d_Pdep = nullptr;
-    int *d_mode = nullptr, *d_status = nullptr, *d_npts = nullptr;
-    double* d_ufinal = nullptr;  // [7][n] state at retirement
+    // per-ray device buffers
+    dev_array<double> d_pos, d_dir, d_w, d_freq, d_u0, d_s0, d_psil, d_Pf, d_Pdep;
+    dev_array<int> d_mode, d_status, d_npts;
+    dev_array<double> d_ufinal;  // [7][n] state at retirement
     // deposition
     int n_psi = 0;
-    double *d_edges = nullptr, *d_bins = nullptr, *d_dV = nullptr, *d_profile = nullptr;
-    unsigned long long *d_queue = nullptr, *d_counters = nullptr;
+    dev_array<double> d_edges, d_bins, d_dV, d_profile;
+    dev_array<unsigned long long> d_queue, d_counters;
     // segment hand-off (allocated on first use)
-    double* d_hand = nullptr;
-    int *d_segdone = nullptr, *d_left = nullptr;
+    dev_array<double> d_hand;
+    dev_array<int> d_segdone, d_left;
     int h_left = 0;  // source of the copy into d_left (outlives the call)
-    int *d_life = nullptr;                      // [n + 1]: predicted life of every ray in segments, then the maximum
-    // trajectory window
+    dev_array<int> d_life;                      // [n + 1]: predicted life of every ray in segments, then the maximum
+    // trajectory window; d_tprof is sized by the trace's n_psi
     int64_t traj_first = 0, traj_count = 0;
     int traj_max = 0;
-    double *d_ts = nullptr, *d_txyz = nullptr, *d_tP = nullptr, *d_tdP = nullptr, *d_tprof = nullptr;
-    int traj_prof_npsi = 0;
+    dev_array<double> d_ts, d_txyz, d_tP, d_tdP, d_tprof;
     // what the device copies of psi_edges / dV were computed from (skips the re-upload when unchanged): the edges and the
     // plasma of every dV row (one row, or one per beam for a plasma set)
     std::vector<double> h_edges;
     std::vector<uint64_t> dV_plasmas;
     // beams
     int n_beams = 1, prof_rows = 0;
-    int* d_beam = nullptr;
+    dev_array<int> d_beam;
     // plasma set of the last torj_bundle_trace_plasmas (n_plasmas > 1): table bases then DevTables pointers, and the plasma
     // of every beam, as last uploaded
     std::vector<const void*> h_set;
     std::vector<int> h_beam_plasma;
-    const void** d_set = nullptr;
-    int* d_beam_plasma = nullptr;
+    dev_array<const void*> d_set;
+    dev_array<int> d_beam_plasma;
     int dV_rows = 1;  // rows of d_dV the last trace used
     // exact-sum mode (allocated on first use): the words of every bin and the status words, torj_xs_buffer_words(bins)
-    long long* d_xs = nullptr;
-    size_t xs_words = 0;
+    dev_array<long long> d_xs;
     bool xs_last = false;  // the last trace booked exactly: results check the status words
     double w_max = 0.0;    // max |weight| of the host weights (infinite for a NaN); -1: weights made on the device
 };
 
-// Error paths: temporaries are owned by dev_ptr, objects under construction by a guard that destroys them unless the
+// Error paths: temporaries are owned by dev_array, objects under construction by a guard that destroys them unless the
 // function reaches its end (every CK / FAIL returns early).
-struct DevFree {
-    void operator()(void* p) const { cudaFree(p); }
-};
-template <class T>
-using dev_ptr = std::unique_ptr<T, DevFree>;
-template <class T>
-static cudaError_t dev_alloc(dev_ptr<T>& p, size_t count) {
-    T* raw = nullptr;
-    cudaError_t e = cudaMalloc(&raw, count * sizeof(T));
-    p.reset(raw);
-    return e;
-}
 template <class T, void (*Destroy)(T*)>
 struct Guard {
     T* p;
@@ -222,8 +243,9 @@ static int upload_warm_constants(torj_ctx* c) {
         const double t = -tmax + (i - 1) * dt;
         tab[i - 1] = make_double2(t, std::exp(-(t * t)) * dt);
     }
-    CK(cudaMalloc(&c->d_warm_tab, ntv * sizeof(double2)));
-    CK(cudaMemcpy(c->d_warm_tab, tab.data(), ntv * sizeof(double2), cudaMemcpyHostToDevice));
+    CK(c->d_warm_tab.resize(ntv, c->stream));
+    CK(cudaMemcpyAsync(c->d_warm_tab, tab.data(), ntv * sizeof(double2), cudaMemcpyHostToDevice, c->stream));
+    CK(cudaStreamSynchronize(c->stream));  // tab is a local
     double comb[6][6][6], fal[6], fct[8], igam[8];
     memset(comb, 0, sizeof comb);
     for (int l = 1; l <= 5; ++l) {
@@ -280,6 +302,7 @@ int torj_ctx_create(int device, void* cuda_stream, torj_ctx** out) {
     CK(cudaEventCreate(&c->ev1));
     Tableau t[2];
     fill_tableaux(t);
+    // cudaMemcpyToSymbol, not the stream: every context writes the same constants, so a running kernel never sees a change
     CK(cudaMemcpyToSymbol(c_tab, t, sizeof t));
     // Bessel series coefficients c[n][k] = (-1)^k n!/(k!(n+k)!)
     double bc[5][TORJ_BESS_K];
@@ -304,7 +327,6 @@ int torj_ctx_create(int device, void* cuda_stream, torj_ctx** out) {
 void torj_ctx_destroy(torj_ctx* c) {
     if (!c) return;
     cudaSetDevice(c->device);
-    cudaFree(c->d_warm_tab);
     if (c->ws) torj_bundle_destroy(c->ws);
     if (c->own_stream) cudaStreamDestroy(c->stream);
     if (c->ev0) cudaEventDestroy(c->ev0);
@@ -363,7 +385,7 @@ int torj_abs_init(torj_ctx* c, int32_t n, const double* nodes, const double* wei
         g.wp[i] = (2 * i == n - 1) ? 0.5 * weights[i] : weights[i];
     }
     CK(cudaDeviceSynchronize());  // no kernel of ANY context on this device may be reading the old table
-    CK(cudaMemcpyToSymbol(c_gl, &g, sizeof g));
+    CK(cudaMemcpyToSymbol(c_gl, &g, sizeof g));  // not a stream copy: the whole device is idle (above)
     g_gl.tab[c->device] = want;
     c->gl_set = true;
     return 0;
@@ -410,6 +432,23 @@ int torj_bspline_prefilter_2d(int32_t nR, int32_t nZ, const double* data, double
     return 0;
 }
 
+// The DevTables of a plasma whose node data are in p->dA, on grid g, and their copy p->dT
+static int plasma_tables(torj_plasma* p, const torj_grid* g, double psi_prof_max) {
+    cudaStream_t st = p->ctx->stream;
+    DevTables& T = p->T;
+    T.A = p->dA;
+    T.nR = g->nR; T.nZ = g->nZ; T.row = g->nR + 2;
+    T.r0 = g->R_first; T.z0 = g->Z_first;
+    double hr = (g->R_last - g->R_first) / (double)(g->nR - 1), hz = (g->Z_last - g->Z_first) / (double)(g->nZ - 1);
+    T.inv_hr = 1.0 / hr; T.inv_hz = 1.0 / hz;
+    T.rlast = g->R_first + hr * (g->nR - 1); T.zlast = g->Z_first + hz * (g->nZ - 1);
+    T.psi_prof_max = psi_prof_max;
+    CK(p->dT.resize(1, st));
+    CK(cudaMemcpyAsync(p->dT, &T, sizeof(DevTables), cudaMemcpyHostToDevice, st));
+    CK(cudaStreamSynchronize(st));  // a plasma set hands dT to the kernels of any context on the device
+    return 0;
+}
+
 int torj_plasma_create(torj_ctx* c, const torj_grid* g, const double* coef_psi, const double* coef_lnne,
                        const double* coef_lnTe, const double* coef_BR, const double* coef_BZ, const double* coef_Bphi,
                        const double* vol_coef, int32_t n_vol, double vol_psi0, double vol_dpsi, double psi_prof_max,
@@ -429,19 +468,10 @@ int torj_plasma_create(torj_ctx* c, const torj_grid* g, const double* coef_psi, 
         hA[3 * k + 1] = make_double2(coef_Bphi[k], coef_lnne[k]);
         hA[3 * k + 2] = make_double2(coef_lnTe[k], coef_psi[k]);
     }
-    CK(cudaMalloc(&p->dA, 3 * nodes * sizeof(double2)));
+    CK(p->dA.resize(3 * nodes, c->stream));
     CK(cudaMemcpyAsync(p->dA, hA.data(), 3 * nodes * sizeof(double2), cudaMemcpyHostToDevice, c->stream));
     CK(cudaStreamSynchronize(c->stream));
-    DevTables& T = p->T;
-    T.A = p->dA;
-    T.nR = g->nR; T.nZ = g->nZ; T.row = g->nR + 2;
-    T.r0 = g->R_first; T.z0 = g->Z_first;
-    double hr = (g->R_last - g->R_first) / (double)(g->nR - 1), hz = (g->Z_last - g->Z_first) / (double)(g->nZ - 1);
-    T.inv_hr = 1.0 / hr; T.inv_hz = 1.0 / hz;
-    T.rlast = g->R_first + hr * (g->nR - 1); T.zlast = g->Z_first + hz * (g->nZ - 1);
-    T.psi_prof_max = psi_prof_max;
-    CK(cudaMalloc(&p->dT, sizeof(DevTables)));
-    CK(cudaMemcpy(p->dT, &T, sizeof(DevTables), cudaMemcpyHostToDevice));
+    if (int rc = plasma_tables(p, g, psi_prof_max)) return rc;
     p->vol_c.assign(vol_coef, vol_coef + n_vol + 2);
     p->n_vol = n_vol; p->vol_x0 = vol_psi0; p->vol_h = vol_dpsi;
     *out = guard.release();
@@ -511,16 +541,16 @@ int torj_plasma_create_from_data(torj_ctx* c, const torj_grid* g, const double* 
     double psi_prof_max = psi_prof[0];
     for (int i = 1; i < n_prof; ++i) psi_prof_max = std::max(psi_prof_max, psi_prof[i]);
     // ---- device: node data of six fields, R pass, Z pass, pack
-    dev_ptr<double> o_raw, o_tmp, o_coef, o_c1, o_cpR, o_cpZ;
-    CK(dev_alloc(o_raw, 6 * npts));
-    CK(dev_alloc(o_tmp, (size_t)sr * nZ));
-    CK(dev_alloc(o_coef, 6 * nodes));
-    CK(dev_alloc(o_c1, 2 * (size_t)(n_prof + 2)));
+    dev_array<double> o_raw, o_tmp, o_coef, o_c1, o_cpR, o_cpZ;
+    CK(o_raw.resize(6 * npts, st));
+    CK(o_tmp.resize((size_t)sr * nZ, st));
+    CK(o_coef.resize(6 * nodes, st));
+    CK(o_c1.resize(2 * (size_t)(n_prof + 2), st));
     std::vector<double> cpR = thomas_pivots(nR), cpZ = thomas_pivots(nZ);
-    CK(dev_alloc(o_cpR, cpR.size()));
-    CK(dev_alloc(o_cpZ, cpZ.size()));
-    double *d_raw = o_raw.get(), *d_tmp = o_tmp.get(), *d_coef = o_coef.get(), *d_c1 = o_c1.get(), *d_cpR = o_cpR.get(),
-           *d_cpZ = o_cpZ.get();
+    CK(o_cpR.resize(cpR.size(), st));
+    CK(o_cpZ.resize(cpZ.size(), st));
+    double *d_raw = o_raw, *d_tmp = o_tmp, *d_coef = o_coef, *d_c1 = o_c1, *d_cpR = o_cpR,
+           *d_cpZ = o_cpZ;
     const double* src[6] = {psi_norm, nullptr, nullptr, BR, BZ, Bphi};  // field order: psi, lnne, lnTe, BR, BZ, Bphi
     for (int f = 0; f < 6; ++f)
         if (src[f]) CK(cudaMemcpyAsync(d_raw + f * npts, src[f], npts * sizeof(double), cudaMemcpyHostToDevice, st));
@@ -544,22 +574,13 @@ int torj_plasma_create_from_data(torj_ctx* c, const torj_grid* g, const double* 
     Guard<torj_plasma, torj_plasma_destroy> guard(p);
     p->ctx = c;
     p->id = ++g_plasma_serial;
-    CK(cudaMalloc(&p->dA, 3 * nodes * sizeof(double2)));
+    CK(p->dA.resize(3 * nodes, st));
     k_pack_tables<<<(unsigned)((nodes + 255) / 256), 256, 0, st>>>(d_coef, d_coef + nodes, d_coef + 2 * nodes, d_coef + 3 * nodes,
                                                                  d_coef + 4 * nodes, d_coef + 5 * nodes, (long long)nodes, p->dA);
     c->launches++;
     CK(cudaGetLastError());
     CK(cudaStreamSynchronize(st));
-    DevTables& T = p->T;
-    T.A = p->dA;
-    T.nR = nR; T.nZ = nZ; T.row = sr;
-    T.r0 = g->R_first; T.z0 = g->Z_first;
-    double hr = (g->R_last - g->R_first) / (double)(nR - 1), hz = (g->Z_last - g->Z_first) / (double)(nZ - 1);
-    T.inv_hr = 1.0 / hr; T.inv_hz = 1.0 / hz;
-    T.rlast = g->R_first + hr * (nR - 1); T.zlast = g->Z_first + hz * (nZ - 1);
-    T.psi_prof_max = psi_prof_max;
-    CK(cudaMalloc(&p->dT, sizeof(DevTables)));
-    CK(cudaMemcpy(p->dT, &T, sizeof(DevTables), cudaMemcpyHostToDevice));
+    if (int rc = plasma_tables(p, g, psi_prof_max)) return rc;
     p->vol_c = vc;
     p->n_vol = n_1d; p->vol_x0 = vr[0]; p->vol_h = (vr[n_1d - 1] - vr[0]) / (double)(n_1d - 1);
     *out = guard.release();
@@ -569,8 +590,6 @@ int torj_plasma_create_from_data(torj_ctx* c, const torj_grid* g, const double* 
 void torj_plasma_destroy(torj_plasma* p) {
     if (!p) return;
     cudaSetDevice(p->ctx->device);
-    cudaFree(p->dA);
-    cudaFree(p->dT);
     delete p;
 }
 
@@ -631,11 +650,11 @@ int torj_probe(torj_ctx* c, const torj_plasma* p, const torj_options* opt, int64
     if (!c->gl_set) FAIL("The weights and abscissae for the absorption were never initialized. Call `abs_Al_init` before using the absorption.");
     if (set_device(c)) return 1;
     SolverOpts so = to_sopts(opt, 1.0);
-    dev_ptr<double> o_x, o_N, o_out;
-    CK(dev_alloc(o_x, 3 * (size_t)n));
-    CK(dev_alloc(o_N, 3 * (size_t)n));
-    CK(dev_alloc(o_out, 11 * (size_t)n));
-    double *dx = o_x.get(), *dN = o_N.get(), *dout = o_out.get();
+    dev_array<double> o_x, o_N, o_out;
+    CK(o_x.resize(3 * (size_t)n, c->stream));
+    CK(o_N.resize(3 * (size_t)n, c->stream));
+    CK(o_out.resize(11 * (size_t)n, c->stream));
+    double *dx = o_x, *dN = o_N, *dout = o_out;
     CK(cudaMemcpyAsync(dx, x, 3 * n * sizeof(double), cudaMemcpyHostToDevice, c->stream));
     CK(cudaMemcpyAsync(dN, N, 3 * n * sizeof(double), cudaMemcpyHostToDevice, c->stream));
     const int model = opt ? opt->absorption_model : 0;
@@ -654,10 +673,10 @@ int torj_rhs(torj_ctx* c, const torj_plasma* p, const torj_options* opt, int64_t
     if (!c->gl_set) FAIL("The weights and abscissae for the absorption were never initialized. Call `abs_Al_init` before using the absorption.");
     if (set_device(c)) return 1;
     SolverOpts so = to_sopts(opt, 1.0);
-    dev_ptr<double> o_u, o_du;
-    CK(dev_alloc(o_u, 7 * (size_t)n));
-    CK(dev_alloc(o_du, 7 * (size_t)n));
-    double *d_u = o_u.get(), *d_du = o_du.get();
+    dev_array<double> o_u, o_du;
+    CK(o_u.resize(7 * (size_t)n, c->stream));
+    CK(o_du.resize(7 * (size_t)n, c->stream));
+    double *d_u = o_u, *d_du = o_du;
     CK(cudaMemcpyAsync(d_u, u, 7 * n * sizeof(double), cudaMemcpyHostToDevice, c->stream));
     const int model = opt ? opt->absorption_model : 0;
     if (model != 0 && model != 1) FAIL("torj_rhs: absorption_model must be 0 (Albajar) or 1 (warm)");
@@ -678,14 +697,14 @@ int torj_warm_alpha(torj_ctx* c, int64_t n, const double* omega, const double* X
     std::vector<double> in(7 * (size_t)n), out(5 * (size_t)n);
     const double* src[7] = {omega, X, Y, N_r, theta, te, v_g_perp};
     for (int q = 0; q < 7; ++q) memcpy(in.data() + q * n, src[q], n * sizeof(double));
-    dev_ptr<double> o_in, o_out;
-    CK(dev_alloc(o_in, in.size()));
-    CK(dev_alloc(o_out, out.size()));
-    CK(cudaMemcpyAsync(o_in.get(), in.data(), in.size() * sizeof(double), cudaMemcpyHostToDevice, c->stream));
-    k_warm_alpha<<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(n, o_in.get(), imod, c->d_warm_tab, o_out.get());
+    dev_array<double> o_in, o_out;
+    CK(o_in.resize(in.size(), c->stream));
+    CK(o_out.resize(out.size(), c->stream));
+    CK(cudaMemcpyAsync(o_in, in.data(), in.size() * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    k_warm_alpha<<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(n, o_in, imod, c->d_warm_tab, o_out);
     c->launches++;
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(out.data(), o_out.get(), out.size() * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaMemcpyAsync(out.data(), o_out, out.size() * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
     CK(cudaStreamSynchronize(c->stream));
     for (int64_t i = 0; i < n; ++i) {
         if (N_warm) N_warm[i] = out[i];
@@ -697,12 +716,6 @@ int torj_warm_alpha(torj_ctx* c, int64_t n, const double* omega, const double* X
 }
 
 // ---- bundle ---------------------------------------------------------------------------------------------------
-static void free_traj(torj_bundle* b) {
-    cudaFree(b->d_ts); cudaFree(b->d_txyz); cudaFree(b->d_tP); cudaFree(b->d_tdP); cudaFree(b->d_tprof);
-    b->d_ts = b->d_txyz = b->d_tP = b->d_tdP = b->d_tprof = nullptr;
-    b->traj_prof_npsi = 0;
-}
-
 static int bundle_upload(torj_bundle* b, const double* pos, const double* dir, const double* weight,
                          const double* freq_hz, const int32_t* mode) {
     torj_ctx* c = b->ctx;
@@ -719,33 +732,43 @@ static int bundle_upload(torj_bundle* b, const double* pos, const double* dir, c
     return 0;
 }
 
-int torj_bundle_create(torj_ctx* c, int64_t n, const double* pos, const double* dir, const double* weight,
-                       const double* freq_hz, const int32_t* mode, int32_t per_ray_fm, torj_bundle** out) {
-    if (!c || !out || n < 1) FAIL("torj_bundle_create: bad argument");
-    if (set_device(c)) return 1;
+// A new bundle of n rays on c (the current device): its per-ray device arrays and the BundleDev that points at them
+static int bundle_new(torj_ctx* c, int64_t n, int32_t per_ray_fm, torj_bundle** out) {
     torj_bundle* b = new torj_bundle();
     Guard<torj_bundle, torj_bundle_destroy> guard(b);
     b->ctx = c; b->n = n; b->per_ray_fm = per_ray_fm;
-    size_t nf = per_ray_fm ? (size_t)n : 1;
-    CK(cudaMalloc(&b->d_pos, 3 * n * sizeof(double)));
-    CK(cudaMalloc(&b->d_dir, 3 * n * sizeof(double)));
-    CK(cudaMalloc(&b->d_w, n * sizeof(double)));
-    CK(cudaMalloc(&b->d_freq, nf * sizeof(double)));
-    CK(cudaMalloc(&b->d_mode, nf * sizeof(int)));
-    CK(cudaMalloc(&b->d_u0, 7 * n * sizeof(double)));
-    CK(cudaMalloc(&b->d_s0, n * sizeof(double)));
-    CK(cudaMalloc(&b->d_psil, n * sizeof(double)));
-    CK(cudaMalloc(&b->d_Pf, n * sizeof(double)));
-    CK(cudaMalloc(&b->d_Pdep, n * sizeof(double)));
-    CK(cudaMalloc(&b->d_status, n * sizeof(int)));
-    CK(cudaMalloc(&b->d_npts, n * sizeof(int)));
-    CK(cudaMalloc(&b->d_queue, sizeof(unsigned long long)));
-    CK(cudaMalloc(&b->d_counters, 8 * sizeof(unsigned long long)));
-    CK(cudaMalloc(&b->d_ufinal, 7 * n * sizeof(double)));
+    const size_t nr = (size_t)n, nf = per_ray_fm ? nr : 1;
+    cudaStream_t st = c->stream;
+    CK(b->d_pos.resize(3 * nr, st));
+    CK(b->d_dir.resize(3 * nr, st));
+    CK(b->d_w.resize(nr, st));
+    CK(b->d_freq.resize(nf, st));
+    CK(b->d_mode.resize(nf, st));
+    CK(b->d_u0.resize(7 * nr, st));
+    CK(b->d_s0.resize(nr, st));
+    CK(b->d_psil.resize(nr, st));
+    CK(b->d_Pf.resize(nr, st));
+    CK(b->d_Pdep.resize(nr, st));
+    CK(b->d_status.resize(nr, st));
+    CK(b->d_npts.resize(nr, st));
+    CK(b->d_queue.resize(1, st));
+    CK(b->d_counters.resize(8, st));
+    CK(b->d_ufinal.resize(7 * nr, st));
     BundleDev& B = b->B;
     B.n_rays = n; B.pos = b->d_pos; B.dir = b->d_dir; B.weight = b->d_w; B.freq = b->d_freq; B.mode = b->d_mode;
     B.per_ray_fm = per_ray_fm; B.u0 = b->d_u0; B.s0 = b->d_s0; B.psi_launch = b->d_psil; B.status = b->d_status;
     B.P_final = b->d_Pf; B.P_dep = b->d_Pdep; B.n_points = b->d_npts;
+    *out = guard.release();
+    return 0;
+}
+
+int torj_bundle_create(torj_ctx* c, int64_t n, const double* pos, const double* dir, const double* weight,
+                       const double* freq_hz, const int32_t* mode, int32_t per_ray_fm, torj_bundle** out) {
+    if (!c || !out || n < 1) FAIL("torj_bundle_create: bad argument");
+    if (set_device(c)) return 1;
+    torj_bundle* b = nullptr;
+    if (int rc = bundle_new(c, n, per_ray_fm, &b)) return rc;
+    Guard<torj_bundle, torj_bundle_destroy> guard(b);
     if (bundle_upload(b, pos, dir, weight, freq_hz, mode)) return 1;
     *out = guard.release();
     return 0;
@@ -780,39 +803,19 @@ int torj_bundle_create_from_launchers(torj_ctx* c, int32_t n_launchers, const do
     const int n_per = start[N_rings];
     const int64_t n = (int64_t)n_launchers * n_per;
     // an empty bundle shell with device arrays, then the generator kernel fills pos/dir/weight/freq/mode/beam
-    std::vector<double> zero3(3, 0.0);
-    torj_bundle* b = new torj_bundle();
+    torj_bundle* b = nullptr;
+    if (int rc = bundle_new(c, n, 1, &b)) return rc;
     Guard<torj_bundle, torj_bundle_destroy> guard(b);
-    b->ctx = c; b->n = n; b->per_ray_fm = 1;
     b->w_max = -1.0;  // weights of order 1 made on the device; an exact booking out of range is refused there
-    CK(cudaMalloc(&b->d_pos, 3 * n * sizeof(double)));
-    CK(cudaMalloc(&b->d_dir, 3 * n * sizeof(double)));
-    CK(cudaMalloc(&b->d_w, n * sizeof(double)));
-    CK(cudaMalloc(&b->d_freq, n * sizeof(double)));
-    CK(cudaMalloc(&b->d_mode, n * sizeof(int)));
-    CK(cudaMalloc(&b->d_u0, 7 * n * sizeof(double)));
-    CK(cudaMalloc(&b->d_s0, n * sizeof(double)));
-    CK(cudaMalloc(&b->d_psil, n * sizeof(double)));
-    CK(cudaMalloc(&b->d_Pf, n * sizeof(double)));
-    CK(cudaMalloc(&b->d_Pdep, n * sizeof(double)));
-    CK(cudaMalloc(&b->d_status, n * sizeof(int)));
-    CK(cudaMalloc(&b->d_npts, n * sizeof(int)));
-    CK(cudaMalloc(&b->d_queue, sizeof(unsigned long long)));
-    CK(cudaMalloc(&b->d_counters, 8 * sizeof(unsigned long long)));
-    CK(cudaMalloc(&b->d_ufinal, 7 * n * sizeof(double)));
-    CK(cudaMalloc(&b->d_beam, n * sizeof(int)));
+    cudaStream_t st = c->stream;
+    CK(b->d_beam.resize(n, st));
     b->n_beams = n_launchers;
-    BundleDev& B = b->B;
-    B.n_rays = n; B.pos = b->d_pos; B.dir = b->d_dir; B.weight = b->d_w; B.freq = b->d_freq; B.mode = b->d_mode;
-    B.per_ray_fm = 1; B.u0 = b->d_u0; B.s0 = b->d_s0; B.psi_launch = b->d_psil; B.status = b->d_status;
-    B.P_final = b->d_Pf; B.P_dep = b->d_Pdep; B.n_points = b->d_npts;
     // launcher parameters to the device
     const size_t nl = n_launchers;
-    dev_ptr<double> o_par; dev_ptr<int> o_ipar;
-    CK(dev_alloc(o_par, 9 * nl + 2 * N_rings));
-    CK(dev_alloc(o_ipar, nl + N_rings + 1));
-    double* d_par = o_par.get(); int* d_ipar = o_ipar.get();
-    cudaStream_t st = c->stream;
+    dev_array<double> o_par; dev_array<int> o_ipar;
+    CK(o_par.resize(9 * nl + 2 * N_rings, st));
+    CK(o_ipar.resize(nl + N_rings + 1, st));
+    double* d_par = o_par; int* d_ipar = o_ipar;
     CK(cudaMemcpyAsync(d_par, x0, 3 * nl * sizeof(double), cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(d_par + 3 * nl, N0, 3 * nl * sizeof(double), cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(d_par + 6 * nl, w, nl * sizeof(double), cudaMemcpyHostToDevice, st));
@@ -853,30 +856,21 @@ void torj_bundle_destroy(torj_bundle* b) {
     if (!b) return;
     cudaSetDevice(b->ctx->device);
     cudaStreamSynchronize(b->ctx->stream);
-    cudaFree(b->d_pos); cudaFree(b->d_dir); cudaFree(b->d_w); cudaFree(b->d_freq); cudaFree(b->d_mode); cudaFree(b->d_u0);
-    cudaFree(b->d_s0); cudaFree(b->d_psil); cudaFree(b->d_Pf); cudaFree(b->d_Pdep); cudaFree(b->d_status); cudaFree(b->d_npts);
-    cudaFree(b->d_hand); cudaFree(b->d_segdone); cudaFree(b->d_left); cudaFree(b->d_life);
-    cudaFree(b->d_queue); cudaFree(b->d_counters); cudaFree(b->d_edges); cudaFree(b->d_bins); cudaFree(b->d_dV);
-    cudaFree(b->d_profile); cudaFree(b->d_xs);
-    cudaFree(b->d_beam);
-    cudaFree(b->d_set); cudaFree(b->d_beam_plasma);
-    cudaFree(b->d_ufinal);
-    free_traj(b);
     delete b;
 }
 
 int torj_bundle_set_window(torj_bundle* b, int64_t first, int64_t count, int32_t max_pts) {
     if (count > 0 && max_pts > 0 && (first < 0 || first + count > b->n)) FAIL("torj_bundle_set_window: window outside the bundle");
     if (set_device(b->ctx)) return 1;
-    CK(cudaStreamSynchronize(b->ctx->stream));
-    free_traj(b);
+    cudaStream_t st = b->ctx->stream;
     b->traj_first = 0; b->traj_count = 0; b->traj_max = 0;  // a failing allocation below leaves an EMPTY window, not a dangling one
-    if (count <= 0 || max_pts <= 0) return 0;
-    size_t m = (size_t)count * max_pts;
-    CK(cudaMalloc(&b->d_ts, m * sizeof(double)));
-    CK(cudaMalloc(&b->d_txyz, 3 * m * sizeof(double)));
-    CK(cudaMalloc(&b->d_tP, m * sizeof(double)));
-    CK(cudaMalloc(&b->d_tdP, m * sizeof(double)));
+    const size_t m = (count > 0 && max_pts > 0) ? (size_t)count * max_pts : 0;
+    CK(b->d_ts.resize(m, st));
+    CK(b->d_txyz.resize(3 * m, st));
+    CK(b->d_tP.resize(m, st));
+    CK(b->d_tdP.resize(m, st));
+    CK(b->d_tprof.resize(0, st));  // until a trace sizes it for its n_psi
+    if (m == 0) return 0;
     b->traj_first = first; b->traj_count = count; b->traj_max = max_pts;
     return 0;
 }
@@ -892,8 +886,9 @@ int torj_bundle_set_beams(torj_bundle* b, int32_t n_beams, const int32_t* beam_i
     }
     for (int64_t i = 0; i < b->n; ++i)
         if (beam_id[i] < 0 || beam_id[i] >= n_beams) FAIL("torj_bundle_set_beams: beam_id out of range");
-    if (!b->d_beam) CK(cudaMalloc(&b->d_beam, b->n * sizeof(int)));
-    CK(cudaMemcpy(b->d_beam, beam_id, b->n * sizeof(int), cudaMemcpyHostToDevice));
+    CK(b->d_beam.resize(b->n, c->stream));  // allocated on first use
+    CK(cudaMemcpyAsync(b->d_beam, beam_id, b->n * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+    CK(cudaStreamSynchronize(c->stream));  // beam_id belongs to the caller
     b->n_beams = n_beams;
     return 0;
 }
@@ -974,25 +969,16 @@ static int bundle_trace(torj_bundle* b, int32_t n_pl, const torj_plasma* const* 
     if (set_device(c)) return 1;
     cudaStream_t st = c->stream;
     if (b->n_psi != n_psi || b->prof_rows != b->n_beams) {
-        CK(cudaStreamSynchronize(st));
-        cudaFree(b->d_edges); cudaFree(b->d_bins); cudaFree(b->d_dV); cudaFree(b->d_profile);
-        b->d_edges = b->d_bins = b->d_dV = b->d_profile = nullptr;  // a failing allocation below must not leave them dangling
-        b->n_psi = 0; b->prof_rows = 0;
+        b->n_psi = 0; b->prof_rows = 0;  // a failing allocation below leaves the bundle untraced
         b->h_edges.clear();
-        CK(cudaMalloc(&b->d_edges, n_psi * sizeof(double)));
-        CK(cudaMalloc(&b->d_bins, (size_t)b->n_beams * (n_psi + 2) * sizeof(double)));
-        CK(cudaMalloc(&b->d_dV, (size_t)b->n_beams * n_psi * sizeof(double)));  // one row, or one per beam for a plasma set
-        CK(cudaMalloc(&b->d_profile, (size_t)b->n_beams * (n_psi + 2) * sizeof(double)));
+        CK(b->d_edges.resize(n_psi, st));
+        CK(b->d_bins.resize((size_t)b->n_beams * (n_psi + 2), st));
+        CK(b->d_dV.resize((size_t)b->n_beams * n_psi, st));  // one row, or one per beam for a plasma set
+        CK(b->d_profile.resize((size_t)b->n_beams * (n_psi + 2), st));
         b->n_psi = n_psi;
         b->prof_rows = b->n_beams;
     }
-    if (b->traj_count > 0 && b->traj_prof_npsi != n_psi) {
-        CK(cudaStreamSynchronize(st));
-        cudaFree(b->d_tprof);
-        b->d_tprof = nullptr; b->traj_prof_npsi = 0;
-        CK(cudaMalloc(&b->d_tprof, (size_t)b->traj_count * n_psi * sizeof(double)));
-        b->traj_prof_npsi = n_psi;
-    }
+    if (b->traj_count > 0) CK(b->d_tprof.resize((size_t)b->traj_count * n_psi, st));
     const int dV_rows = set ? b->n_beams : 1;
     std::vector<uint64_t> row_plasma(dV_rows);
     for (int q = 0; q < dV_rows; ++q) row_plasma[q] = pls[set ? beam_plasma[q] : 0]->id;
@@ -1017,36 +1003,24 @@ static int bundle_trace(torj_bundle* b, int32_t n_pl, const torj_plasma* const* 
         std::vector<int> hb(beam_plasma, beam_plasma + b->n_beams);
         if (hs != b->h_set || hb != b->h_beam_plasma) {
             CK(cudaStreamSynchronize(st));  // an earlier trace may still read them
-            if (hs.size() != b->h_set.size()) {
-                cudaFree(b->d_set);
-                b->d_set = nullptr; b->h_set.clear();
-                CK(cudaMalloc(&b->d_set, hs.size() * sizeof(void*)));
-            }
-            if (hb.size() != b->h_beam_plasma.size()) {
-                cudaFree(b->d_beam_plasma);
-                b->d_beam_plasma = nullptr; b->h_beam_plasma.clear();
-                CK(cudaMalloc(&b->d_beam_plasma, hb.size() * sizeof(int)));
-            }
+            b->h_set.clear(); b->h_beam_plasma.clear();  // until the copies below have completed
+            CK(b->d_set.resize(hs.size(), st));
+            CK(b->d_beam_plasma.resize(hb.size(), st));
             CK(cudaMemcpyAsync(b->d_set, hs.data(), hs.size() * sizeof(void*), cudaMemcpyHostToDevice, st));
             CK(cudaMemcpyAsync(b->d_beam_plasma, hb.data(), hb.size() * sizeof(int), cudaMemcpyHostToDevice, st));
             CK(cudaStreamSynchronize(st));  // hs and hb are locals
             b->h_set = hs; b->h_beam_plasma = hb;
         }
-        P.A = reinterpret_cast<const double2* const*>(b->d_set);
-        P.T = reinterpret_cast<const DevTables* const*>(b->d_set + n_pl);
+        const void** d_set = b->d_set;
+        P.A = reinterpret_cast<const double2* const*>(d_set);
+        P.T = reinterpret_cast<const DevTables* const*>(d_set + n_pl);
         P.beam_plasma = b->d_beam_plasma; P.beam_id = b->d_beam;
     }
     CK(cudaMemsetAsync(b->d_bins, 0, (size_t)b->n_beams * (n_psi + 2) * sizeof(double), st));
     const size_t xs_words = torj_xs_buffer_words((size_t)b->n_beams * (n_psi + 2));
     b->xs_last = false;
     if (xs) {
-        if (b->xs_words != xs_words) {
-            CK(cudaStreamSynchronize(st));
-            cudaFree(b->d_xs);
-            b->d_xs = nullptr; b->xs_words = 0;
-            CK(cudaMalloc(&b->d_xs, xs_words * sizeof(long long)));
-            b->xs_words = xs_words;
-        }
+        CK(b->d_xs.resize(xs_words, st));
         CK(cudaMemsetAsync(b->d_xs, 0, xs_words * sizeof(long long), st));
     }
     CK(cudaMemsetAsync(b->d_queue, 0, sizeof(unsigned long long), st));
@@ -1103,9 +1077,9 @@ static int bundle_trace(torj_bundle* b, int32_t n_pl, const torj_plasma* const* 
     if (od.n_segments < 2 || od.n_segments > TORJ_SEG_MAX || b->n > 0x7fffffff) interleave = 0;  // TORJ_SEG_MAX: the hand-off word's 15-bit fields
     a.interleave = interleave; a.hand = nullptr; a.seg_done = nullptr; a.rays_left = nullptr;
     if (interleave) {
-        if (!b->d_hand) CK(cudaMalloc(&b->d_hand, (size_t)b->n * TORJ_HAND_D * sizeof(double)));
-        if (!b->d_segdone) CK(cudaMalloc(&b->d_segdone, (size_t)b->n * sizeof(int)));
-        if (!b->d_left) CK(cudaMalloc(&b->d_left, sizeof(int)));
+        CK(b->d_hand.resize((size_t)b->n * TORJ_HAND_D, st));
+        CK(b->d_segdone.resize((size_t)b->n, st));
+        CK(b->d_left.resize(1, st));
         b->h_left = (int)b->n;
         CK(cudaMemsetAsync(b->d_segdone, 0, (size_t)b->n * sizeof(int), st));
         CK(cudaMemcpyAsync(b->d_left, &b->h_left, sizeof(int), cudaMemcpyHostToDevice, st));
@@ -1118,7 +1092,7 @@ static int bundle_trace(torj_bundle* b, int32_t n_pl, const torj_plasma* const* 
     // GPUs (profiles/). A pilot march predicts every ray's life; the rounds are shifted so that all rays END together and
     // the long ones start first, while idle lanes run ahead in the queue and start the short ones early.
     if (interleave && model == 0 && od.schedule != 3) {
-        if (!b->d_life) CK(cudaMalloc(&b->d_life, ((size_t)b->n + 1) * sizeof(int)));
+        CK(b->d_life.resize((size_t)b->n + 1, st));
         CK(cudaMemsetAsync(b->d_life + b->n, 0, sizeof(int), st));
         k_predict_life<<<(unsigned)((b->n + 127) / 128), 128, 0, st>>>(p->T, b->B, so, P, TORJ_LIFE_HARM_COST, b->d_life,
                                                                       b->d_life + b->n);
@@ -1222,8 +1196,10 @@ int torj_bundle_trajectories(torj_bundle* b, double* s, double* xyz, double* P, 
     if (dP_dV_ray) {  // shell power -> dP/dV per ray (reference src/plasma.jl:141), with the volume of the ray's plasma
         std::vector<double> dV((size_t)b->dV_rows * b->n_psi);
         std::vector<int> beam(b->dV_rows > 1 ? b->traj_count : 0);
-        CK(cudaMemcpy(dV.data(), b->d_dV, dV.size() * sizeof(double), cudaMemcpyDeviceToHost));
-        if (!beam.empty()) CK(cudaMemcpy(beam.data(), b->d_beam + b->traj_first, beam.size() * sizeof(int), cudaMemcpyDeviceToHost));
+        CK(cudaMemcpyAsync(dV.data(), b->d_dV, dV.size() * sizeof(double), cudaMemcpyDeviceToHost, st));
+        if (!beam.empty())
+            CK(cudaMemcpyAsync(beam.data(), b->d_beam + b->traj_first, beam.size() * sizeof(int), cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));  // dV and beam are locals
         for (int64_t r = 0; r < b->traj_count; ++r) {
             double* row = dP_dV_ray + (size_t)r * b->n_psi;
             const double* dVr = dV.data() + (beam.empty() ? 0 : (size_t)beam[r] * b->n_psi);
@@ -1263,7 +1239,8 @@ int torj_bundle_trajectories_cyl(torj_bundle* b, double* R, double* phi, double*
     std::vector<double> xyz(3 * m), P(m);
     if (int rc = torj_bundle_trajectories(b, nullptr, xyz.data(), P.data(), nullptr, nullptr)) return rc;
     std::vector<int> np(b->n);
-    CK(cudaMemcpy(np.data(), b->d_npts, b->n * sizeof(int), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpyAsync(np.data(), b->d_npts, b->n * sizeof(int), cudaMemcpyDeviceToHost, b->ctx->stream));
+    CK(cudaStreamSynchronize(b->ctx->stream));  // np is a local
     for (int64_t r = 0; r < b->traj_count; ++r) {
         const int cnt = std::min<int>(std::max(np[b->traj_first + r], 0), b->traj_max);
         const double* x = xyz.data() + (size_t)r * 3 * b->traj_max;
@@ -1280,22 +1257,25 @@ int torj_bundle_trajectories_cyl(torj_bundle* b, double* R, double* phi, double*
 
 }  // extern "C"
 
-// torj_trace (one plasma) and torj_trace_plasmas
-static int trace_oneshot(torj_ctx* c, int32_t n_pl, const torj_plasma* const* pls, const int32_t* beam_plasma,
-                         const torj_options* opt, int64_t n_rays, const double* pos, const double* dir, const double* weight,
-                         const double* freq_hz, const int32_t* mode, int32_t per_ray_fm, double s_max, int32_t n_psi,
-                         const double* psi_edges, int32_t n_beams, const int32_t* beam_id, double* dP_dV, double* deposited_power,
-                         double* P_final, double* P_dep, int32_t* n_points, int32_t* status, int64_t traj_first, int64_t traj_count,
-                         int32_t traj_max_pts, double* traj_s, double* traj_xyz, double* traj_P, double* traj_dP_ds,
-                         double* traj_dP_dV_ray, torj_counters* counters) {
-    // the device workspace of the previous call is reused when the bundle shape is unchanged (no cudaMalloc/cudaFree
-    // on the repeated-call path of make_beam scans)
-    int rc = 0;
+static void drop_workspace(torj_ctx* c) {  // a workspace in an unknown state is not kept
+    torj_bundle_destroy(c->ws);
+    c->ws = nullptr;
+}
+
+// The one-shot calls (torj_trace*, torj_multi_trace*) trace through the context's workspace c->ws with this call's rays,
+// trajectory window and beams. The workspace of the previous call is reused when the bundle shape is unchanged (no
+// cudaMalloc/cudaFree on the repeated-call path of make_beam scans).
+static int workspace_trace(torj_ctx* c, int32_t n_pl, const torj_plasma* const* pls, const int32_t* beam_plasma,
+                           const torj_options* opt, int64_t n_rays, const double* pos, const double* dir, const double* weight,
+                           const double* freq_hz, const int32_t* mode, int32_t per_ray_fm, double s_max, int32_t n_psi,
+                           const double* psi_edges, int32_t n_beams, const int32_t* beam_id, int64_t traj_first,
+                           int64_t traj_count, int32_t traj_max_pts) {
     torj_bundle* b = c->ws;
     if (b && (b->n != n_rays || b->per_ray_fm != per_ray_fm)) {
-        torj_bundle_destroy(b);
-        b = c->ws = nullptr;
+        drop_workspace(c);
+        b = nullptr;
     }
+    int rc = 0;
     if (!b) {
         rc = torj_bundle_create(c, n_rays, pos, dir, weight, freq_hz, mode, per_ray_fm, &b);
         if (rc) return rc;
@@ -1309,12 +1289,23 @@ static int trace_oneshot(torj_ctx* c, int32_t n_pl, const torj_plasma* const* pl
         rc = torj_bundle_set_window(b, traj_first, traj_count, traj_max_pts);
     if (!rc) rc = torj_bundle_set_beams(b, n_beams, beam_id);
     if (!rc) rc = bundle_trace(b, n_pl, pls, beam_plasma, opt, s_max, n_psi, psi_edges);
+    return rc;
+}
+
+// torj_trace (one plasma) and torj_trace_plasmas
+static int trace_oneshot(torj_ctx* c, int32_t n_pl, const torj_plasma* const* pls, const int32_t* beam_plasma,
+                         const torj_options* opt, int64_t n_rays, const double* pos, const double* dir, const double* weight,
+                         const double* freq_hz, const int32_t* mode, int32_t per_ray_fm, double s_max, int32_t n_psi,
+                         const double* psi_edges, int32_t n_beams, const int32_t* beam_id, double* dP_dV, double* deposited_power,
+                         double* P_final, double* P_dep, int32_t* n_points, int32_t* status, int64_t traj_first, int64_t traj_count,
+                         int32_t traj_max_pts, double* traj_s, double* traj_xyz, double* traj_P, double* traj_dP_ds,
+                         double* traj_dP_dV_ray, torj_counters* counters) {
+    int rc = workspace_trace(c, n_pl, pls, beam_plasma, opt, n_rays, pos, dir, weight, freq_hz, mode, per_ray_fm, s_max, n_psi,
+                             psi_edges, n_beams, beam_id, traj_first, traj_count, traj_max_pts);
+    torj_bundle* b = c->ws;
     if (!rc) rc = torj_bundle_results(b, dP_dV, deposited_power, P_final, P_dep, n_points, status, counters);
     if (!rc && traj_count > 0) rc = torj_bundle_trajectories(b, traj_s, traj_xyz, traj_P, traj_dP_ds, traj_dP_dV_ray);
-    if (rc) {  // do not keep a workspace in an unknown state
-        torj_bundle_destroy(b);
-        c->ws = nullptr;
-    }
+    if (rc) drop_workspace(c);
     return rc;
 }
 
@@ -1422,28 +1413,17 @@ struct MultiWorker {
 // Pinned host staging of one device's shard, grown on demand and kept between calls
 struct MultiStage {
     size_t cap = 0;
-    double *pos = nullptr, *dir = nullptr, *w = nullptr, *freq = nullptr, *Pf = nullptr, *Pd = nullptr;
-    int *mode = nullptr, *beam = nullptr, *np = nullptr, *st = nullptr;
+    pinned_array<double> pos, dir, w, freq, Pf, Pd;
+    pinned_array<int> mode, beam, np, st;
     std::vector<int64_t> gidx;  // global ray index of local ray j
-    void release() {
-        cudaFreeHost(pos); cudaFreeHost(dir); cudaFreeHost(w); cudaFreeHost(freq); cudaFreeHost(Pf); cudaFreeHost(Pd);
-        cudaFreeHost(mode); cudaFreeHost(beam); cudaFreeHost(np); cudaFreeHost(st);
-        pos = dir = w = freq = Pf = Pd = nullptr; mode = beam = np = st = nullptr; cap = 0;
-    }
-    cudaError_t reserve(size_t n) {
+    cudaError_t reserve(size_t n, cudaStream_t s) {
         if (n <= cap) return cudaSuccess;
-        release();
+        cap = 0;
         cudaError_t e;
-        if ((e = cudaHostAlloc(&pos, 3 * n * sizeof(double), cudaHostAllocDefault))) return e;
-        if ((e = cudaHostAlloc(&dir, 3 * n * sizeof(double), cudaHostAllocDefault))) return e;
-        if ((e = cudaHostAlloc(&w, n * sizeof(double), cudaHostAllocDefault))) return e;
-        if ((e = cudaHostAlloc(&freq, n * sizeof(double), cudaHostAllocDefault))) return e;
-        if ((e = cudaHostAlloc(&Pf, n * sizeof(double), cudaHostAllocDefault))) return e;
-        if ((e = cudaHostAlloc(&Pd, n * sizeof(double), cudaHostAllocDefault))) return e;
-        if ((e = cudaHostAlloc(&mode, n * sizeof(int), cudaHostAllocDefault))) return e;
-        if ((e = cudaHostAlloc(&beam, n * sizeof(int), cudaHostAllocDefault))) return e;
-        if ((e = cudaHostAlloc(&np, n * sizeof(int), cudaHostAllocDefault))) return e;
-        if ((e = cudaHostAlloc(&st, n * sizeof(int), cudaHostAllocDefault))) return e;
+        if ((e = pos.resize(3 * n, s)) || (e = dir.resize(3 * n, s)) || (e = w.resize(n, s)) || (e = freq.resize(n, s)) ||
+            (e = Pf.resize(n, s)) || (e = Pd.resize(n, s)) || (e = mode.resize(n, s)) || (e = beam.resize(n, s)) ||
+            (e = np.resize(n, s)) || (e = st.resize(n, s)))
+            return e;
         cap = n;
         return cudaSuccess;
     }
@@ -1452,7 +1432,7 @@ struct MultiStage {
 struct torj_multi {
     std::vector<torj_ctx*> ctx;
     std::vector<std::unique_ptr<MultiWorker>> worker;
-    std::vector<MultiStage> stage;
+    std::vector<std::unique_ptr<MultiStage>> stage;  // freed with its device current
     std::vector<ncclComm_t> comm;  // empty when NCCL is unavailable
     int sharding = 0;              // 0 contiguous, 1 block-cyclic
     int64_t block = 1;
@@ -1486,8 +1466,8 @@ int torj_multi_create(int32_t n_devices, torj_multi** out) {
         if (int rc = torj_ctx_create(d, nullptr, &c)) return rc;
         m->ctx.push_back(c);
     }
-    m->stage.resize(n_devices);
     for (int d = 0; d < n_devices; ++d) {
+        m->stage.emplace_back(new MultiStage());
         m->worker.emplace_back(new MultiWorker());
         MultiWorker* w = m->worker.back().get();
         w->th = std::thread([w] { w->loop(); });
@@ -1516,7 +1496,7 @@ void torj_multi_destroy(torj_multi* m) {
     for (size_t d = 0; d < m->comm.size(); ++d) nccl_api().CommDestroy(m->comm[d]);
     for (size_t d = 0; d < m->stage.size(); ++d) {
         if (d < m->ctx.size()) cudaSetDevice(m->ctx[d]->device);
-        m->stage[d].release();
+        m->stage[d].reset();
     }
     for (auto* c : m->ctx) torj_ctx_destroy(c);
     delete m;
@@ -1641,12 +1621,12 @@ static int multi_trace(torj_multi* m, const char* fn, bool set_api, int32_t n_pl
     // ---- phase A
     m->run(used, [&](int d) {
         torj_ctx* c = m->ctx[d];
-        MultiStage& S = m->stage[d];
+        MultiStage& S = *m->stage[d];
         auto fail = [&](int rc) { rcs[d] = rc; errs[d] = g_err; };  // g_err is thread-local
         if (set_device(c)) return fail(1);
         shard_indices(n_rays, used, d, m->sharding, m->block, S.gidx);
         const int64_t n = (int64_t)S.gidx.size();
-        if (cudaError_t e = S.reserve((size_t)n)) { g_err = std::string("pinned staging: ") + cudaGetErrorString(e); return fail(1); }
+        if (cudaError_t e = S.reserve((size_t)n, c->stream)) { g_err = std::string("pinned staging: ") + cudaGetErrorString(e); return fail(1); }
         for (int64_t j = 0; j < n; ++j) {
             const int64_t g = S.gidx[j];
             for (int q = 0; q < 3; ++q) { S.pos[q * n + j] = pos[q * n_rays + g]; S.dir[q * n + j] = dir[q * n_rays + g]; }
@@ -1661,21 +1641,10 @@ static int multi_trace(torj_multi* m, const char* fn, bool set_api, int32_t n_pl
             for (int64_t j = 0; j < n; ++j)
                 if (S.gidx[j] >= traj_first && S.gidx[j] < traj_first + traj_count) { lo = std::min(lo, j); ++cntw; }
         wlo[d] = cntw ? lo : 0; wcnt[d] = cntw;  // contiguous in local order for both shardings
-        torj_bundle* b = c->ws;
-        if (b && (b->n != n || b->per_ray_fm != per_ray_fm)) { torj_bundle_destroy(b); b = c->ws = nullptr; }
-        int rc = 0;
-        if (!b) {
-            rc = torj_bundle_create(c, n, S.pos, S.dir, S.w, S.freq, S.mode, per_ray_fm, &b);
-            if (rc) return fail(rc);
-            c->ws = b;
-        } else if ((rc = bundle_upload(b, S.pos, S.dir, S.w, S.freq, S.mode))) {
-            return fail(rc);
-        }
-        if (wcnt[d] != b->traj_count || wlo[d] != b->traj_first || (wcnt[d] > 0 && traj_max_pts != b->traj_max))
-            rc = torj_bundle_set_window(b, wlo[d], wcnt[d], traj_max_pts);
-        if (!rc) rc = torj_bundle_set_beams(b, n_beams, n_beams > 1 ? S.beam : nullptr);
-        if (!rc) rc = bundle_trace(b, n_pl, sets[d].data(), beam_plasma, opt, s_max, n_psi, psi_edges);
-        if (rc) fail(rc);
+        if (int rc = workspace_trace(c, n_pl, sets[d].data(), beam_plasma, opt, n, S.pos, S.dir, S.w,
+                                     S.freq, S.mode, per_ray_fm, s_max, n_psi, psi_edges, n_beams,
+                                     S.beam, wlo[d], wcnt[d], traj_max_pts))
+            fail(rc);
     });
     bool all_ok = true;
     for (int d = 0; d < used; ++d) all_ok = all_ok && rcs[d] == 0;
@@ -1685,7 +1654,7 @@ static int multi_trace(torj_multi* m, const char* fn, bool set_api, int32_t n_pl
     const bool xs = m->ctx[0]->exact_sum != 0;
     const bool do_nccl = all_ok && want_nccl;
     if (all_ok && xs && !do_nccl && used > 1) {
-        const size_t nw = m->ctx[0]->ws->xs_words;
+        const size_t nw = m->ctx[0]->ws->d_xs.size();
         std::vector<std::vector<unsigned long long>> hw(used, std::vector<unsigned long long>(nw));
         m->run(used, [&](int d) {
             torj_ctx* c = m->ctx[d];
@@ -1717,12 +1686,12 @@ static int multi_trace(torj_multi* m, const char* fn, bool set_api, int32_t n_pl
     if (all_ok) m->run(used, [&](int d) {
         torj_ctx* c = m->ctx[d];
         torj_bundle* b = c->ws;
-        MultiStage& S = m->stage[d];
+        MultiStage& S = *m->stage[d];
         auto fail = [&](int rc) { rcs[d] = rc; errs[d] = g_err; };
         if (set_device(c)) return fail(1);
         const int64_t n = b->n;
         if (do_nccl && xs) {
-            ncclResult_t r = nccl_api().AllReduce(b->d_xs, b->d_xs, b->xs_words, ncclInt64, ncclSum, m->comm[d], c->stream);
+            ncclResult_t r = nccl_api().AllReduce(b->d_xs, b->d_xs, b->d_xs.size(), ncclInt64, ncclSum, m->comm[d], c->stream);
             if (r != ncclSuccess) { g_err = std::string("ncclAllReduce: ") + nccl_api().GetErrorString(r); return fail(3); }
             if (int rc = finalize(b)) return fail(rc);
         } else if (do_nccl) {
@@ -1734,8 +1703,9 @@ static int multi_trace(torj_multi* m, const char* fn, bool set_api, int32_t n_pl
         prof[d].assign((size_t)n_beams * prow, 0.0);
         std::vector<double> pr((size_t)n_beams * n_psi), dp(n_beams);
         int rc = torj_bundle_results(b, (!one || d == 0) ? pr.data() : nullptr, (!one || d == 0) ? dp.data() : nullptr,
-                                     P_final ? S.Pf : nullptr, P_dep ? S.Pd : nullptr, n_points ? S.np : nullptr,
-                                     status ? S.st : nullptr, &cnts[d]);
+                                     P_final ? static_cast<double*>(S.Pf) : nullptr, P_dep ? static_cast<double*>(S.Pd) : nullptr,
+                                     n_points ? static_cast<int*>(S.np) : nullptr, status ? static_cast<int*>(S.st) : nullptr,
+                                     &cnts[d]);
         if (rc) return fail(rc);
         for (int q = 0; q < n_beams; ++q) {
             memcpy(prof[d].data() + q * prow, pr.data() + (size_t)q * n_psi, n_psi * sizeof(double));
@@ -1768,9 +1738,7 @@ static int multi_trace(torj_multi* m, const char* fn, bool set_api, int32_t n_pl
     });
     for (int d = 0; d < used; ++d)
         if (rcs[d]) {
-            // a workspace in an unknown state is not kept
-            for (int q = 0; q < used; ++q)
-                if (m->ctx[q]->ws) { cudaSetDevice(m->ctx[q]->device); torj_bundle_destroy(m->ctx[q]->ws); m->ctx[q]->ws = nullptr; }
+            for (int q = 0; q < used; ++q) drop_workspace(m->ctx[q]);
             g_err = "device " + std::to_string(d) + ": " + errs[d];
             return rcs[d];
         }
@@ -1821,9 +1789,9 @@ int torj_multi_trace_plasmas(torj_multi* m, int32_t n_plasmas, const torj_mplasm
 
 int torj_fp64_peak(torj_ctx* c, int32_t iters, double* tflops, double* ms) {
     if (set_device(c)) return 1;
-    dev_ptr<double> o_d;
-    CK(dev_alloc(o_d, 1));
-    double* d = o_d.get();
+    dev_array<double> o_d;
+    CK(o_d.resize(1, c->stream));
+    double* d = o_d;
     struct Ev {
         cudaEvent_t e = nullptr;
         ~Ev() { if (e) cudaEventDestroy(e); }
@@ -1850,10 +1818,10 @@ int torj_fp64_peak(torj_ctx* c, int32_t iters, double* tflops, double* ms) {
 // cycles per dependent DFMA (single warp, single chain)
 int torj_fp64_latency(torj_ctx* c, int32_t iters, double* cycles_per_dfma) {
     if (set_device(c)) return 1;
-    dev_ptr<double> o_d; dev_ptr<long long> o_dc;
-    CK(dev_alloc(o_d, 1));
-    CK(dev_alloc(o_dc, 1));
-    double* d = o_d.get(); long long* dc = o_dc.get();
+    dev_array<double> o_d; dev_array<long long> o_dc;
+    CK(o_d.resize(1, c->stream));
+    CK(o_dc.resize(1, c->stream));
+    double* d = o_d; long long* dc = o_dc;
     k_dfma_latency<<<1, 32, 0, c->stream>>>(iters, 1.0, d, dc);
     c->launches++;
     long long cyc = 0;
@@ -1867,10 +1835,10 @@ int torj_fp64_latency(torj_ctx* c, int32_t iters, double* cycles_per_dfma) {
 int torj_math_probe(torj_ctx* c, int64_t n, const double* x, double* out) {
     if (!c || n < 1 || !x || !out) FAIL("torj_math_probe: bad argument");
     if (set_device(c)) return 1;
-    dev_ptr<double> o_x, o_out;
-    CK(dev_alloc(o_x, (size_t)n));
-    CK(dev_alloc(o_out, 4 * (size_t)n));
-    double *dx = o_x.get(), *dout = o_out.get();
+    dev_array<double> o_x, o_out;
+    CK(o_x.resize((size_t)n, c->stream));
+    CK(o_out.resize(4 * (size_t)n, c->stream));
+    double *dx = o_x, *dout = o_out;
     CK(cudaMemcpyAsync(dx, x, n * sizeof(double), cudaMemcpyHostToDevice, c->stream));
     k_math_probe<<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(n, dx, dout);
     c->launches++;
