@@ -219,8 +219,21 @@ int torj_bundle_trace_plasmas(torj_bundle* b, int32_t n_plasmas, const torj_plas
                               int32_t n_psi, const double* psi_edges);
 /* Device pointer to n_beams x (n_psi+2) doubles: dP_dV[n_psi], deposited_power, sum of weights per beam — for a caller-side
  * NCCL all-reduce (sum) across GPUs; valid after torj_bundle_trace, ordered on the context stream. With exact sums each
- * device's profile is exact, but a double all-reduce of several devices' profiles is not. */
+ * device's profile is exact, but a double all-reduce of several devices' profiles is not: sum the integer words instead
+ * (torj_bundle_device_exact_words, then torj_bundle_finalize_exact). */
 void* torj_bundle_device_profile(torj_bundle* b);
+/* After an exact-sum torj_bundle_trace(_plasmas): device pointer to the bundle's accumulator, TORJ_XS_STAT (2) status words
+ * followed by n_beams x (n_psi+2) x 8 int64 words, and its length. Ordered on the context stream. Valid until the next
+ * trace or destroy. A caller may add other processes' buffers of the same length into it, word by word, as signed 64-bit
+ * integers (status words included; an integer all-reduce with sum), then call torj_bundle_finalize_exact: the profile is
+ * then that of one device tracing every process's rays, bit for bit (at a fixed lanes_per_ray). Refused (non-zero,
+ * torj_last_error) for a NULL bundle, before any trace, and when the last trace was not in exact mode. */
+int torj_bundle_device_exact_words(torj_bundle* b, void** words, int64_t* n_words);
+/* Converts the (summed) words again into the device profile, normalised by the dV rows of the last trace, on the context
+ * stream; returns without synchronising. torj_bundle_results then checks the summed status words: an out-of-range booking
+ * on any process, or more than 2^34 bookings in the sum, makes it fail on every process. Same refusals as
+ * torj_bundle_device_exact_words. */
+int torj_bundle_finalize_exact(torj_bundle* b);
 /* Synchronises and copies results to the host (any pointer may be NULL); fails after an exact-sum trace whose accumulator
  * overflowed or refused a booking (torj_ctx_set_exact_sum). For a ray that failed initialisation
  * (status 1 or 2) P_final and P_deposited_ray are 0 and n_points is minus the failing check's number (-1 no grid entry,

@@ -174,6 +174,48 @@ function α(omega::Real, X::Real, Y::Real, N_r::Real, theta::Real, te::Real, v_g
     return Nw[], al[]
 end
 
+# ---- one process per GPU (MPI.jl + CUDA.jl): exact sums across ranks -------------------------------------------------
+# After an exact-sum trace the bundle's integer accumulator is summed over the ranks word by word (MPI.Allreduce! of Int64
+# with +), then converted once: dP_dV and the deposited power are the bits of one trace of every rank's rays, at a fixed
+# lanes_per_ray. The agreement first (ok and the word count, MIN) makes every rank throw when one rank's trace failed or
+# the lengths differ, instead of leaving the others waiting in the sum. This sketch needs n >= 1 rays on every rank.
+exact_words(b) = (p = Ref{Ptr{Cvoid}}(C_NULL); n = Ref{Int64}(0);
+                  torj_check(ccall((:torj_bundle_device_exact_words, libtorj), Cint, (Ptr{Cvoid}, Ref{Ptr{Cvoid}}, Ref{Int64}), b, p, n));
+                  (p[], n[]))
+finalize_exact!(b) = torj_check(ccall((:torj_bundle_finalize_exact, libtorj), Cint, (Ptr{Cvoid},), b))
+function torj_trace_exact_mpi(hp, pos::Matrix{Float64}, dir::Matrix{Float64}, w::Vector{Float64}, f, mode, s_max, psi, comm;
+                              options=torj_options())
+    set_exact_sum!(true)
+    n = length(w); npsi = length(psi); b = Ref{Ptr{Cvoid}}(C_NULL)
+    dP_dV = zeros(npsi); dep = Ref(0.0); Pf = zeros(n); Pd = zeros(n); npts = zeros(Int32, n); st = zeros(Int32, n)
+    try
+        words, nw = C_NULL, 0
+        try
+            torj_check(ccall((:torj_bundle_create, libtorj), Cint, (Ptr{Cvoid}, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+                Ref{Float64}, Ref{Int32}, Int32, Ref{Ptr{Cvoid}}), torj_ctx(), n, pos, dir, w, Float64(f), Int32(mode), 0, b))
+            torj_check(ccall((:torj_bundle_trace, libtorj), Cint, (Ptr{Cvoid}, Ptr{Cvoid}, Ref{TorjOptions}, Float64, Int32,
+                Ptr{Float64}), b[], hp, options, s_max, npsi, psi))
+            words, nw = exact_words(b[])
+        catch
+            MPI.Allreduce(Int64[0, typemax(Int64), typemax(Int64)], min, comm)   # join the agreement as failed
+            rethrow()
+        end
+        ok, lo, neg_hi = MPI.Allreduce(Int64[1, nw, -nw], min, comm)
+        ok == 1 || error("torj_trace_exact_mpi: the trace failed on another rank")
+        lo == -neg_hi || error("torj_trace_exact_mpi: the ranks' accumulators differ in length ($lo to $(-neg_hi) words)")
+        torj_check(ccall((:torj_ctx_sync, libtorj), Cint, (Ptr{Cvoid},), torj_ctx()))
+        buf = unsafe_wrap(CuArray, CuPtr{Int64}(UInt(words)), nw)   # the library's buffer, no copy (CUDA-aware MPI)
+        MPI.Allreduce!(buf, +, comm)
+        CUDA.synchronize()
+        finalize_exact!(b[])
+        torj_check(ccall((:torj_bundle_results, libtorj), Cint, (Ptr{Cvoid}, Ptr{Float64}, Ref{Float64}, Ptr{Float64},
+            Ptr{Float64}, Ptr{Int32}, Ptr{Int32}, Ptr{Cvoid}), b[], dP_dV, dep, Pf, Pd, npts, st, C_NULL))
+    finally
+        ccall((:torj_bundle_destroy, libtorj), Cvoid, (Ptr{Cvoid},), b[])
+    end
+    (; dP_dV, deposited = dep[], Pf, Pd, npts, st)
+end
+
 # ---- several GPUs from this one Julia process: bind torj_multi_* instead (same arguments as torj_trace) ---------------
 # torj_multi_create opens every visible device and the NCCL communicators (ncclCommInitAll); torj_multi_trace shards the
 # rays (contiguous, or beams dealt round-robin after torj_multi_configure(m, 1, rays_per_beam, 0)), traces every shard on

@@ -72,6 +72,8 @@ SIGNATURES = {
     "torj_bundle_trace_plasmas": (C.c_int, [c_vp, C.c_int32, C.POINTER(c_vp), c_ip, C.POINTER(TorjOptions), C.c_double,
                                             C.c_int32, c_dp]),
     "torj_bundle_device_profile": (c_vp, [c_vp]),
+    "torj_bundle_device_exact_words": (C.c_int, [c_vp, C.POINTER(c_vp), C.POINTER(C.c_int64)]),
+    "torj_bundle_finalize_exact": (C.c_int, [c_vp]),
     "torj_bundle_results": (C.c_int, [c_vp, c_dp, c_dp, c_dp, c_dp, c_ip, c_ip, C.POINTER(TorjCounters)]),
     "torj_bundle_trajectories": (C.c_int, [c_vp, c_dp, c_dp, c_dp, c_dp, c_dp]),
     "torj_bundle_final_state": (C.c_int, [c_vp, c_dp, c_dp, c_dp, c_dp]),

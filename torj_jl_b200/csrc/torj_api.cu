@@ -1138,6 +1138,36 @@ int torj_bundle_trace_plasmas(torj_bundle* b, int32_t n_plasmas, const torj_plas
 
 void* torj_bundle_device_profile(torj_bundle* b) { return b->d_profile; }
 
+}  // extern "C"
+
+// The refusals of the exact-word pair: the words exist only after a trace that booked them
+static int check_exact_words(const torj_bundle* b, const char* fn) {
+    char msg[256];
+    if (!b) { snprintf(msg, sizeof msg, "%s: bundle is NULL", fn); FAIL(msg); }
+    if (b->n_psi == 0) { snprintf(msg, sizeof msg, "%s: nothing traced yet", fn); FAIL(msg); }
+    if (!b->xs_last) {
+        snprintf(msg, sizeof msg, "%s: the last trace did not book exact sums (torj_ctx_set_exact_sum(ctx, 1) before it)", fn);
+        FAIL(msg);
+    }
+    return 0;
+}
+
+extern "C" {
+
+int torj_bundle_device_exact_words(torj_bundle* b, void** words, int64_t* n_words) {
+    if (int rc = check_exact_words(b, "torj_bundle_device_exact_words")) return rc;
+    if (!words || !n_words) FAIL("torj_bundle_device_exact_words: words and n_words must not be NULL");
+    *words = static_cast<long long*>(b->d_xs);
+    *n_words = (int64_t)b->d_xs.size();
+    return 0;
+}
+
+int torj_bundle_finalize_exact(torj_bundle* b) {
+    if (int rc = check_exact_words(b, "torj_bundle_finalize_exact")) return rc;
+    if (set_device(b->ctx)) return 1;
+    return finalize(b);
+}
+
 int torj_bundle_results(torj_bundle* b, double* dP_dV, double* deposited_power, double* P_final, double* P_dep,
                         int32_t* n_points, int32_t* status, torj_counters* counters) {
     torj_ctx* c = b->ctx;

@@ -51,8 +51,114 @@ def _world():
     return 0, 1
 
 
+class _ExactReduction:
+    """trace_sharded(exact_sum=True): the integer all-reduce of the ranks' exact words, between each rank's trace and its
+    conversion (trace_bundle's reduce_exact). Every rank makes the same collective calls in the same order whether it
+    traced, had no rays or failed, so a failure on one rank makes every rank raise instead of leaving the others waiting:
+      1. agreement, one all-reduce (MIN) of [ok, n_words, -n_words, rank if traced, -empty]: all ranks reached the sum,
+         the shortest and longest accumulator, the lowest rank that traced, whether some rank had no rays;
+      2. the integer sum (SUM, int64) of the words; a rank without rays adds zeros of the agreed length;
+      3. a second agreement [ok] after every rank's conversion and results;
+      4. only when some rank had no rays: a broadcast of the converted vector from the lowest rank that traced (a copy of
+         bits; an empty rank has no bundle to convert)."""
+    _NONE = 1 << 62  # neutral under MIN
+
+    def __init__(self, rank, world, device):
+        import torch
+        import torch.distributed as dist
+
+        self.torch, self.dist, self.rank = torch, dist, rank
+        self.on = world > 1
+        self.nccl = self.on and dist.get_backend() == "nccl"
+        if self.nccl:
+            self.dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+        else:
+            self.dev = torch.device("cpu")
+        self.entered = self.summed = False
+        self.agreed = None
+
+    def _min(self, vals):
+        t = self.torch.tensor(vals, dtype=self.torch.int64, device=self.dev)
+        if self.on:
+            self.dist.all_reduce(t, op=self.dist.ReduceOp.MIN)
+        return t.tolist()
+
+    def _agree(self, ok, n_words=None, empty=False):
+        N = self._NONE
+        ok_all, lo, neg_hi, src, neg_empty = self._min([int(ok), N if n_words is None else n_words,
+                                                        N if n_words is None else -n_words, N if empty else self.rank,
+                                                        -int(empty)])
+        if not ok_all:
+            raise RuntimeError("trace_sharded(exact_sum=True): trace_fn failed on a rank before the exact sum (that rank "
+                               "raised its own error); no rank summed")
+        if lo != -neg_hi:
+            raise RuntimeError(f"trace_sharded(exact_sum=True): the ranks' exact accumulators differ in length ({lo} to "
+                               f"{-neg_hi} words): every rank must trace with the same psi levels and n_beams")
+        self.agreed = (lo, src, neg_empty < 0)
+
+    def _agree_after(self, ok):
+        if not self._min([int(ok)])[0]:
+            raise RuntimeError("trace_sharded(exact_sum=True): a rank failed after the exact sum, converting it or reading "
+                               "its results (that rank raised its own error)")
+
+    def _sum(self, words):
+        if not self.on:
+            return
+        if self.nccl:
+            self.dist.all_reduce(words, op=self.dist.ReduceOp.SUM)
+        else:
+            h = words.cpu()
+            self.dist.all_reduce(h, op=self.dist.ReduceOp.SUM)
+            words.copy_(h)
+
+    def reduce_exact(self, words):
+        self.entered = True
+        self._agree(1, int(words.numel()))
+        self._sum(words)
+        self.summed = True
+
+    def run(self, trace_fn, args, per_ray, n_beams):
+        """(local result, this rank's exact vector, the reduced vector) of trace_fn on this rank's rays args"""
+        torch = self.torch
+        if len(args[2]) == 0:
+            self._agree(1, empty=True)
+            n_words, src, _ = self.agreed
+            self._sum(torch.zeros(n_words, dtype=torch.int64, device=self.dev))
+            self._agree_after(1)
+            vec = np.zeros((n_words - 2) // 8)  # a buffer's 2 status words, then 8 words per bin
+            out = torch.zeros(len(vec), dtype=torch.float64, device=self.dev)
+            self.dist.broadcast(out, src)
+            local = dict(P_final=np.zeros(0), P_deposited_ray=np.zeros(0), n_points=np.zeros(0, dtype=np.int32),
+                         status=np.zeros(0, dtype=np.int32))
+            return local, vec, out.cpu().numpy()
+        try:
+            local = trace_fn(*args, **per_ray, reduce_exact=self.reduce_exact)
+            if not self.summed:
+                raise RuntimeError("trace_sharded(exact_sum=True): trace_fn did not call reduce_exact; pass it on as "
+                                   "trace_bundle(..., exact_sum=True, reduce_exact=reduce_exact)")
+        except BaseException:
+            if not self.entered:
+                try:
+                    self._agree(0)
+                except RuntimeError:
+                    pass  # every rank learns of the failure; this one raises its own error
+            elif self.summed:
+                try:
+                    self._agree_after(0)
+                except RuntimeError:
+                    pass
+            raise
+        self._agree_after(1)
+        vec_sum = np.concatenate([np.reshape(local["dP_dV"], (n_beams, -1)), np.reshape(local["deposited_power"], (n_beams, 1)),
+                                  np.reshape(local["sum_weights"], (n_beams, 1))], axis=1).ravel()
+        if self.agreed[2]:
+            t = torch.from_numpy(vec_sum.copy()).to(self.dev)
+            self.dist.broadcast(t, self.agreed[1])
+        return local, np.asarray(local["local_vector"]), vec_sum
+
+
 def trace_sharded(trace_fn, ray_positions, ray_directions, ray_weights, *, n_beams=1, per_ray=None, sharding="contiguous",
-                  block=1, device=None, gather_rays=True):
+                  block=1, device=None, gather_rays=True, exact_sum=False):
     """make_beam's parallel region and reduction (reference src/solve.jl:219-240) over the ranks of the initialised process
     group. `trace_fn(pos, dirs, w)` traces this rank's rays — on a GPU box `lambda p, d, w: tj.trace_bundle(plasma, p, d, w,
     ...)` — and returns a dict with dP_dV [n_psi], deposited_power, P_final / n_points / status [n_local].
@@ -64,7 +170,15 @@ def trace_sharded(trace_fn, ray_positions, ray_directions, ray_weights, *, n_bea
     beam_plasma=bp)`.
     Returns the all-reduced dP_dV, deposited_power and sum of weights (per beam when n_beams > 1), this rank's `local`
     result and `idx`, and (when gather_rays) the per-ray outputs of the WHOLE bundle in launch order, identical on every
-    rank."""
+    rank.
+    exact_sum=True: the ranks' exact deposition sums are added as integers, not as finished double profiles, so dP_dV,
+    deposited_power and sum_weights are bit-identical for any world size and either sharding, at a fixed lanes_per_ray
+    (the automatic width depends on the shard's size), and equal those of one trace_bundle(..., exact_sum=True) of the
+    whole bundle. trace_fn then receives one more keyword argument, `reduce_exact`, and must pass it on:
+    `lambda p, d, w, reduce_exact: tj.trace_bundle(plasma, p, d, w, ..., exact_sum=True, reduce_exact=reduce_exact)`; its
+    result must carry trace_bundle's `sum_weights` and `local_vector`, which is then this rank's own exact vector. A rank
+    whose shard is empty (block-cyclic sharding with fewer blocks than ranks) does not call trace_fn. If trace_fn raises on
+    any rank, or the ranks' accumulators differ in length, every rank raises; none waits forever in a collective."""
     import torch
     import torch.distributed as dist
 
@@ -83,18 +197,24 @@ def trace_sharded(trace_fn, ray_positions, ray_directions, ray_weights, *, n_bea
         if n and (bid.min() < 0 or bid.max() >= n_beams):
             raise ValueError(f"beam_id must lie in [0, {n_beams})")
     idx = shard_indices(n, rank, world, sharding, block)
-    local = trace_fn(pos[idx], dirs[idx], w[idx], **{k: v[idx] for k, v in per_ray.items()})
-    if n_beams > 1:
-        sw = np.bincount(per_ray["beam_id"][idx], weights=w[idx], minlength=n_beams)
-        vec = np.concatenate([np.reshape(local["dP_dV"], (n_beams, -1)), np.reshape(local["deposited_power"], (n_beams, 1)),
-                              sw[:, None]], axis=1).ravel()
+    if exact_sum:
+        if n == 0:
+            raise ValueError("trace_sharded(exact_sum=True) needs at least one ray")
+        local, vec, vec_sum = _ExactReduction(rank, world, device).run(
+            trace_fn, (pos[idx], dirs[idx], w[idx]), {k: v[idx] for k, v in per_ray.items()}, n_beams)
     else:
-        vec = np.concatenate([np.ravel(local["dP_dV"]), [float(local["deposited_power"]), float(np.sum(w[idx]))]])
-    t = torch.from_numpy(vec.copy())
-    if device is not None:
-        t = t.to(device)
-    allreduce_profile(t)
-    vec_sum = t.cpu().numpy()
+        local = trace_fn(pos[idx], dirs[idx], w[idx], **{k: v[idx] for k, v in per_ray.items()})
+        if n_beams > 1:
+            sw = np.bincount(per_ray["beam_id"][idx], weights=w[idx], minlength=n_beams)
+            vec = np.concatenate([np.reshape(local["dP_dV"], (n_beams, -1)), np.reshape(local["deposited_power"], (n_beams, 1)),
+                                  sw[:, None]], axis=1).ravel()
+        else:
+            vec = np.concatenate([np.ravel(local["dP_dV"]), [float(local["deposited_power"]), float(np.sum(w[idx]))]])
+        t = torch.from_numpy(vec.copy())
+        if device is not None:
+            t = t.to(device)
+        allreduce_profile(t)
+        vec_sum = t.cpu().numpy()
     if n_beams > 1:
         rows = vec_sum.reshape(n_beams, -1)
         out = dict(dP_dV=rows[:, :-2].copy(), deposited_power=rows[:, -2].copy(), sum_weights=rows[:, -1].copy(), local=local,

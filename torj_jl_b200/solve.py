@@ -82,15 +82,34 @@ def bundle_result(m):
                 P_final=o["Pf"], P_deposited_ray=o["Pd"], n_points=o["npts"], status=o["st"], counters=o["cnt"].as_dict())
 
 
+def device_tensor(ptr, n, typestr):
+    """A torch CUDA tensor over n elements of a device buffer the library owns (no copy; torch finds the device from the
+    pointer). It is valid only as long as that buffer."""
+    import torch
+
+    class _DevBuf:
+        __cuda_array_interface__ = {"shape": (int(n),), "typestr": typestr, "version": 2, "data": (int(ptr or 0), False)}
+    return torch.as_tensor(_DevBuf())
+
+
 def trace_bundle(plasma, ray_positions, ray_directions, ray_weights, f, mode, s_max, psi_dP_dV, *,
                  options=None, ctx=None, trajectories=None, traj_max_pts=None, beam_id=None, n_beams=1, beam_plasma=None,
-                 exact_sum=False):
+                 exact_sum=False, reduce_exact=None):
     """One torj_trace call on host buffers. trajectories: None or (first, count).
     beam_id/n_beams: rays of several beams in one bundle -> dP_dV[n_beams, n_psi], deposited_power[n_beams].
     plasma: a Plasma, or a sequence of Plasma on one (R,Z) grid with beam_plasma[n_beams] naming the plasma of every beam
     (torj_trace_plasmas; keep each beam's rays contiguous).
     exact_sum: book the profile in an exact fixed-point sum (torj_ctx_set_exact_sum), so dP_dV and deposited_power are
-    bit-identical under any schedule, ray order and device count; weights |w| <= 2^40."""
+    bit-identical under any schedule, ray order and device count; weights |w| <= 2^40.
+    reduce_exact (needs exact_sum): fn(words), called between the trace and the conversion of the profile. `words` is the
+    bundle's exact accumulator as an int64 torch CUDA tensor (the library's buffer itself, torj_bundle_device_exact_words);
+    fn must leave in it the word-by-word integer sum over every process that traced a part of the bundle (an all-reduce
+    with SUM; distributed.trace_sharded(..., exact_sum=True) passes one). dP_dV and deposited_power are then the profile of
+    the summed words: the bits of one trace of all the processes' rays, at a fixed lanes_per_ray. The result also holds
+    `sum_weights` (of the sum; per beam when n_beams > 1) and `local_vector`, this process's own converted vector
+    [n_beams][n_psi | deposited | sum w]."""
+    if reduce_exact is not None and not exact_sum:
+        raise ValueError("reduce_exact needs exact_sum=True: only the exact accumulator sums across processes without rounding")
     pls = _plasma_set(plasma, beam_plasma)
     m = marshal_bundle(ray_positions, ray_directions, ray_weights, f, mode, psi_dP_dV, beam_id, n_beams,
                        n_plasmas=len(pls) if pls else 1, beam_plasma=beam_plasma)
@@ -105,6 +124,9 @@ def trace_bundle(plasma, ray_positions, ray_directions, ray_weights, f, mode, s_
     tm = int(traj_max_pts or 0)
     ts = np.zeros((t_count, tm)); txyz = np.zeros((t_count, 3, tm)); tP = np.zeros((t_count, tm))
     tdP = np.zeros((t_count, tm)); tprof = np.zeros((t_count, len(psi)))
+    traj = dict(traj_s=ts, traj_xyz=txyz, traj_P=tP, traj_dP_ds=tdP, traj_dP_dV_ray=tprof)
+    if reduce_exact is not None:
+        return _trace_reduced(L, ctx, plasma, pls, m, opt, s_max, (t_first, t_count, tm), traj, reduce_exact)
     rest = (C.byref(opt), n, _p(m["pos"]), _p(m["dir"]), _p(m["w"]), _p(m["f"]), m["mode"].ctypes.data_as(c_ip), m["per_ray"],
             float(s_max), len(psi), _p(psi), m["n_beams"], m["beam"].ctypes.data_as(c_ip) if m["beam"] is not None else None,
             _p(o["prof"]), _p(o["dep"]), _p(o["Pf"]), _p(o["Pd"]), o["npts"].ctypes.data_as(c_ip), o["st"].ctypes.data_as(c_ip),
@@ -115,7 +137,50 @@ def trace_bundle(plasma, ray_positions, ray_directions, ray_weights, f, mode, s_
         hs = (_lib.c_vp * len(pls))(*[p.handle(ctx).value for p in pls])
         _lib.check(L.torj_trace_plasmas(ctx, len(pls), hs, m["beam_plasma"].ctypes.data_as(c_ip), *rest))
     res = bundle_result(m)
-    res.update(traj_s=ts, traj_xyz=txyz, traj_P=tP, traj_dP_ds=tdP, traj_dP_dV_ray=tprof)
+    res.update(traj)
+    return res
+
+
+def _trace_reduced(L, ctx, plasma, pls, m, opt, s_max, window, traj, reduce_exact):
+    """trace_bundle with reduce_exact: the same trace on a resident bundle, whose exact words reduce_exact sums across
+    processes before they are converted (torj_bundle_device_exact_words / torj_bundle_finalize_exact)."""
+    import torch
+
+    n, psi, o, nb = m["n"], m["psi"], m["out"], m["n_beams"]
+    t_first, t_count, tm = window
+    bh = _lib.c_vp()
+    _lib.check(L.torj_bundle_create(ctx, n, _p(m["pos"]), _p(m["dir"]), _p(m["w"]), _p(m["f"]), m["mode"].ctypes.data_as(c_ip),
+                                    m["per_ray"], C.byref(bh)))
+    try:
+        _lib.check(L.torj_bundle_set_beams(bh, nb, m["beam"].ctypes.data_as(c_ip) if m["beam"] is not None else None))
+        _lib.check(L.torj_bundle_set_window(bh, t_first, t_count, tm))
+        if pls is None:
+            _lib.check(L.torj_bundle_trace(bh, plasma.handle(ctx), C.byref(opt), float(s_max), len(psi), _p(psi)))
+        else:
+            hs = (_lib.c_vp * len(pls))(*[p.handle(ctx).value for p in pls])
+            _lib.check(L.torj_bundle_trace_plasmas(bh, len(pls), hs, m["beam_plasma"].ctypes.data_as(c_ip), C.byref(opt),
+                                                   float(s_max), len(psi), _p(psi)))
+        ptr, n_words = _lib.c_vp(), C.c_int64()
+        _lib.check(L.torj_bundle_device_exact_words(bh, C.byref(ptr), C.byref(n_words)))
+        n_vec = nb * (len(psi) + 2)
+        # the library works on its context's stream, the reduction on torch's current one: each waits for the other
+        _lib.check(L.torj_ctx_sync(ctx))
+        local_vector = device_tensor(L.torj_bundle_device_profile(bh), n_vec, "<f8").cpu().numpy()
+        words = device_tensor(ptr.value, n_words.value, "<i8")
+        reduce_exact(words)
+        if words.is_cuda:
+            torch.cuda.current_stream(words.device).synchronize()
+        _lib.check(L.torj_bundle_finalize_exact(bh))
+        _lib.check(L.torj_bundle_results(bh, _p(o["prof"]), _p(o["dep"]), _p(o["Pf"]), _p(o["Pd"]), o["npts"].ctypes.data_as(c_ip),
+                                         o["st"].ctypes.data_as(c_ip), C.byref(o["cnt"])))
+        if t_count:
+            _lib.check(L.torj_bundle_trajectories(bh, *(_p(traj[k]) for k in ("traj_s", "traj_xyz", "traj_P", "traj_dP_ds",
+                                                                             "traj_dP_dV_ray"))))
+        sw = device_tensor(L.torj_bundle_device_profile(bh), n_vec, "<f8").cpu().numpy().reshape(nb, -1)[:, -1]
+    finally:
+        L.torj_bundle_destroy(bh)
+    res = bundle_result(m)
+    res.update(traj, sum_weights=sw.copy() if nb > 1 else float(sw[0]), local_vector=local_vector)
     return res
 
 
