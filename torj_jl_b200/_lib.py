@@ -5,6 +5,8 @@ from __future__ import annotations
 import ctypes as C
 import os
 
+import numpy as np
+
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("TORJ_CUDA_LIB") or os.path.join(_HERE, "libtorj_cuda.so")  # override: tuning experiments
 _LIB = None
@@ -12,6 +14,36 @@ _LIB = None
 c_dp = C.POINTER(C.c_double)
 c_ip = C.POINTER(C.c_int32)
 c_vp = C.c_void_p
+
+
+def _p(a):
+    return a.ctypes.data_as(c_dp)
+
+
+def _ip(a):
+    return a.ctypes.data_as(c_ip) if a is not None else None
+
+
+def profile_vector(dP_dV, deposited_power, sum_weights, n_beams):
+    """The library's profile layout [n_beams][n_psi | deposited | sum w] (a bundle's device profile; the vector the
+    processes of distributed.trace_sharded add) of per-beam parts, or of unbatched ones when n_beams is 1."""
+    return np.concatenate([np.reshape(dP_dV, (n_beams, -1)), np.reshape(deposited_power, (n_beams, 1)),
+                           np.reshape(sum_weights, (n_beams, 1))], axis=1).ravel()
+
+
+def split_profile_vector(vec, n_beams):
+    """(dP_dV, deposited_power, sum_weights) of a profile vector: [n_beams, n_psi] and [n_beams] arrays when n_beams > 1,
+    else [n_psi] and floats."""
+    rows = np.reshape(vec, (n_beams, -1))
+    if n_beams > 1:
+        return rows[:, :-2].copy(), rows[:, -2].copy(), rows[:, -1].copy()
+    return rows[0, :-2], float(rows[0, -2]), float(rows[0, -1])
+
+
+def exact_bins(n_words):
+    """The bins of an exact accumulator of n_words int64 (torj_exactsum.cuh: 2 status words, then 8 words per bin), that
+    is, the length of the profile vector it converts to."""
+    return (n_words - 2) // 8
 
 
 class TorjOptions(C.Structure):

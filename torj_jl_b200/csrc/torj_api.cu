@@ -1292,46 +1292,68 @@ static void drop_workspace(torj_ctx* c) {  // a workspace in an unknown state is
     c->ws = nullptr;
 }
 
-// The one-shot calls (torj_trace*, torj_multi_trace*) trace through the context's workspace c->ws with this call's rays,
-// trajectory window and beams. The workspace of the previous call is reused when the bundle shape is unchanged (no
-// cudaMalloc/cudaFree on the repeated-call path of make_beam scans).
+// The rays and beams of a one-shot call, or of one device's shard of it
+struct JobRays {
+    int64_t n_rays;
+    const double *pos, *dir, *weight, *freq_hz;
+    const int32_t* mode;
+    int32_t per_ray_fm, n_beams;
+    const int32_t* beam_id;
+};
+
+// A one-shot call (torj_trace*, torj_multi_trace*): its arguments after the plasma ones, in the C ABI's order
+struct HostJob : JobRays {
+    const torj_options* opt;  // psi levels, options and s_max
+    double s_max;
+    int32_t n_psi;
+    const double* psi_edges;
+    double *dP_dV, *deposited_power, *P_final, *P_dep;  // outputs
+    int32_t *n_points, *status;
+    int64_t traj_first, traj_count;  // trajectory window
+    int32_t traj_max_pts;
+    double *traj_s, *traj_xyz, *traj_P, *traj_dP_ds, *traj_dP_dV_ray;
+    torj_counters* counters;
+    int trace_oneshot(torj_ctx* c, int32_t n_pl, const torj_plasma* const* pls, const int32_t* beam_plasma) const;
+    int multi_trace(torj_multi* m, const char* fn, bool set_api, int32_t n_pl, const torj_mplasma* const* mps,
+                    const int32_t* beam_plasma);
+};
+#define TORJ_HOST_JOB                                                                                              \
+    HostJob {                                                                                                      \
+        {n_rays, pos, dir, weight, freq_hz, mode, per_ray_fm, n_beams, beam_id}, opt, s_max, n_psi, psi_edges, dP_dV, \
+            deposited_power, P_final, P_dep, n_points, status, traj_first, traj_count, traj_max_pts, traj_s, traj_xyz,  \
+            traj_P, traj_dP_ds, traj_dP_dV_ray, counters                                                           \
+    }
+
+// The one-shot calls (torj_trace*, torj_multi_trace*) trace through the context's workspace c->ws with the rays r, the
+// trajectory window [traj_first, traj_first + traj_count) and j's psi levels and options. The workspace of the previous
+// call is reused when the bundle shape is unchanged (no cudaMalloc/cudaFree on the repeated-call path of make_beam scans).
 static int workspace_trace(torj_ctx* c, int32_t n_pl, const torj_plasma* const* pls, const int32_t* beam_plasma,
-                           const torj_options* opt, int64_t n_rays, const double* pos, const double* dir, const double* weight,
-                           const double* freq_hz, const int32_t* mode, int32_t per_ray_fm, double s_max, int32_t n_psi,
-                           const double* psi_edges, int32_t n_beams, const int32_t* beam_id, int64_t traj_first,
-                           int64_t traj_count, int32_t traj_max_pts) {
+                           const HostJob& j, const JobRays& r, int64_t traj_first, int64_t traj_count) {
     torj_bundle* b = c->ws;
-    if (b && (b->n != n_rays || b->per_ray_fm != per_ray_fm)) {
+    if (b && (b->n != r.n_rays || b->per_ray_fm != r.per_ray_fm)) {
         drop_workspace(c);
         b = nullptr;
     }
     int rc = 0;
     if (!b) {
-        rc = torj_bundle_create(c, n_rays, pos, dir, weight, freq_hz, mode, per_ray_fm, &b);
+        rc = torj_bundle_create(c, r.n_rays, r.pos, r.dir, r.weight, r.freq_hz, r.mode, r.per_ray_fm, &b);
         if (rc) return rc;
         c->ws = b;
     } else {
         if (set_device(c)) return 1;
-        rc = bundle_upload(b, pos, dir, weight, freq_hz, mode);
+        rc = bundle_upload(b, r.pos, r.dir, r.weight, r.freq_hz, r.mode);
         if (rc) return rc;
     }
-    if (traj_count != b->traj_count || traj_first != b->traj_first || (traj_count > 0 && traj_max_pts != b->traj_max))
-        rc = torj_bundle_set_window(b, traj_first, traj_count, traj_max_pts);
-    if (!rc) rc = torj_bundle_set_beams(b, n_beams, beam_id);
-    if (!rc) rc = bundle_trace(b, n_pl, pls, beam_plasma, opt, s_max, n_psi, psi_edges);
+    if (traj_count != b->traj_count || traj_first != b->traj_first || (traj_count > 0 && j.traj_max_pts != b->traj_max))
+        rc = torj_bundle_set_window(b, traj_first, traj_count, j.traj_max_pts);
+    if (!rc) rc = torj_bundle_set_beams(b, r.n_beams, r.beam_id);
+    if (!rc) rc = bundle_trace(b, n_pl, pls, beam_plasma, j.opt, j.s_max, j.n_psi, j.psi_edges);
     return rc;
 }
 
 // torj_trace (one plasma) and torj_trace_plasmas
-static int trace_oneshot(torj_ctx* c, int32_t n_pl, const torj_plasma* const* pls, const int32_t* beam_plasma,
-                         const torj_options* opt, int64_t n_rays, const double* pos, const double* dir, const double* weight,
-                         const double* freq_hz, const int32_t* mode, int32_t per_ray_fm, double s_max, int32_t n_psi,
-                         const double* psi_edges, int32_t n_beams, const int32_t* beam_id, double* dP_dV, double* deposited_power,
-                         double* P_final, double* P_dep, int32_t* n_points, int32_t* status, int64_t traj_first, int64_t traj_count,
-                         int32_t traj_max_pts, double* traj_s, double* traj_xyz, double* traj_P, double* traj_dP_ds,
-                         double* traj_dP_dV_ray, torj_counters* counters) {
-    int rc = workspace_trace(c, n_pl, pls, beam_plasma, opt, n_rays, pos, dir, weight, freq_hz, mode, per_ray_fm, s_max, n_psi,
-                             psi_edges, n_beams, beam_id, traj_first, traj_count, traj_max_pts);
+int HostJob::trace_oneshot(torj_ctx* c, int32_t n_pl, const torj_plasma* const* pls, const int32_t* beam_plasma) const {
+    int rc = workspace_trace(c, n_pl, pls, beam_plasma, *this, *this, traj_first, traj_count);
     torj_bundle* b = c->ws;
     if (!rc) rc = torj_bundle_results(b, dP_dV, deposited_power, P_final, P_dep, n_points, status, counters);
     if (!rc && traj_count > 0) rc = torj_bundle_trajectories(b, traj_s, traj_xyz, traj_P, traj_dP_ds, traj_dP_dV_ray);
@@ -1347,9 +1369,7 @@ int torj_trace(torj_ctx* c, const torj_plasma* p, const torj_options* opt, int64
                double* deposited_power, double* P_final, double* P_dep, int32_t* n_points, int32_t* status, int64_t traj_first,
                int64_t traj_count, int32_t traj_max_pts, double* traj_s, double* traj_xyz, double* traj_P, double* traj_dP_ds,
                double* traj_dP_dV_ray, torj_counters* counters) {
-    return trace_oneshot(c, 1, &p, nullptr, opt, n_rays, pos, dir, weight, freq_hz, mode, per_ray_fm, s_max, n_psi, psi_edges,
-                         n_beams, beam_id, dP_dV, deposited_power, P_final, P_dep, n_points, status, traj_first, traj_count,
-                         traj_max_pts, traj_s, traj_xyz, traj_P, traj_dP_ds, traj_dP_dV_ray, counters);
+    return TORJ_HOST_JOB.trace_oneshot(c, 1, &p, nullptr);
 }
 
 int torj_trace_plasmas(torj_ctx* c, int32_t n_plasmas, const torj_plasma* const* plasmas, const int32_t* beam_plasma,
@@ -1363,9 +1383,7 @@ int torj_trace_plasmas(torj_ctx* c, int32_t n_plasmas, const torj_plasma* const*
     // refused before the workspace is touched; the bundle's beams are those torj_bundle_set_beams will set
     if (int rc = check_plasma_set("torj_trace_plasmas", c, n_plasmas, plasmas, beam_plasma, (beam_id && n_beams > 1) ? n_beams : 1))
         return rc;
-    return trace_oneshot(c, n_plasmas, plasmas, beam_plasma, opt, n_rays, pos, dir, weight, freq_hz, mode, per_ray_fm, s_max, n_psi,
-                         psi_edges, n_beams, beam_id, dP_dV, deposited_power, P_final, P_dep, n_points, status, traj_first,
-                         traj_count, traj_max_pts, traj_s, traj_xyz, traj_P, traj_dP_ds, traj_dP_dV_ray, counters);
+    return TORJ_HOST_JOB.trace_oneshot(c, n_plasmas, plasmas, beam_plasma);
 }
 
 // ---- single-process multi-GPU front end (what a Julia make_beam on an 8-GPU box calls) -------------------------
@@ -1604,13 +1622,8 @@ static void shard_indices(int64_t n_rays, int used, int d, int sharding, int64_t
 // Phase A on device d: gather the shard into pinned staging, upload, enqueue ray init + trace + finalize through the set's
 // copies on d. Phase B: (NCCL all-reduce of the device profile buffers, in place, one call per device thread;) results to
 // the host.
-static int multi_trace(torj_multi* m, const char* fn, bool set_api, int32_t n_pl, const torj_mplasma* const* mps,
-                       const int32_t* beam_plasma, const torj_options* opt, int64_t n_rays, const double* pos,
-                       const double* dir, const double* weight, const double* freq_hz, const int32_t* mode, int32_t per_ray_fm,
-                       double s_max, int32_t n_psi, const double* psi_edges, int32_t n_beams, const int32_t* beam_id,
-                       double* dP_dV, double* deposited_power, double* P_final, double* P_dep, int32_t* n_points,
-                       int32_t* status, int64_t traj_first, int64_t traj_count, int32_t traj_max_pts, double* traj_s,
-                       double* traj_xyz, double* traj_P, double* traj_dP_ds, double* traj_dP_dV_ray, torj_counters* counters) {
+int HostJob::multi_trace(torj_multi* m, const char* fn, bool set_api, int32_t n_pl, const torj_mplasma* const* mps,
+                         const int32_t* beam_plasma) {
     const int nd = (int)m->ctx.size();
     char msg[256];
     const bool have = n_pl >= 1 && mps;
@@ -1671,9 +1684,8 @@ static int multi_trace(torj_multi* m, const char* fn, bool set_api, int32_t n_pl
             for (int64_t j = 0; j < n; ++j)
                 if (S.gidx[j] >= traj_first && S.gidx[j] < traj_first + traj_count) { lo = std::min(lo, j); ++cntw; }
         wlo[d] = cntw ? lo : 0; wcnt[d] = cntw;  // contiguous in local order for both shardings
-        if (int rc = workspace_trace(c, n_pl, sets[d].data(), beam_plasma, opt, n, S.pos, S.dir, S.w,
-                                     S.freq, S.mode, per_ray_fm, s_max, n_psi, psi_edges, n_beams,
-                                     S.beam, wlo[d], wcnt[d], traj_max_pts))
+        if (int rc = workspace_trace(c, n_pl, sets[d].data(), beam_plasma, *this,
+                                     {n, S.pos, S.dir, S.w, S.freq, S.mode, per_ray_fm, n_beams, S.beam}, wlo[d], wcnt[d]))
             fail(rc);
     });
     bool all_ok = true;
@@ -1799,9 +1811,7 @@ int torj_multi_trace(torj_multi* m, const torj_mplasma* mp, const torj_options* 
                      double* dP_dV, double* deposited_power, double* P_final, double* P_dep, int32_t* n_points,
                      int32_t* status, int64_t traj_first, int64_t traj_count, int32_t traj_max_pts, double* traj_s,
                      double* traj_xyz, double* traj_P, double* traj_dP_ds, double* traj_dP_dV_ray, torj_counters* counters) {
-    return multi_trace(m, "torj_multi_trace", false, 1, &mp, nullptr, opt, n_rays, pos, dir, weight, freq_hz, mode, per_ray_fm,
-                       s_max, n_psi, psi_edges, n_beams, beam_id, dP_dV, deposited_power, P_final, P_dep, n_points, status,
-                       traj_first, traj_count, traj_max_pts, traj_s, traj_xyz, traj_P, traj_dP_ds, traj_dP_dV_ray, counters);
+    return TORJ_HOST_JOB.multi_trace(m, "torj_multi_trace", false, 1, &mp, nullptr);
 }
 
 int torj_multi_trace_plasmas(torj_multi* m, int32_t n_plasmas, const torj_mplasma* const* plasmas, const int32_t* beam_plasma,
@@ -1811,10 +1821,7 @@ int torj_multi_trace_plasmas(torj_multi* m, int32_t n_plasmas, const torj_mplasm
                              double* deposited_power, double* P_final, double* P_dep, int32_t* n_points, int32_t* status,
                              int64_t traj_first, int64_t traj_count, int32_t traj_max_pts, double* traj_s, double* traj_xyz,
                              double* traj_P, double* traj_dP_ds, double* traj_dP_dV_ray, torj_counters* counters) {
-    return multi_trace(m, "torj_multi_trace_plasmas", true, n_plasmas, plasmas, beam_plasma, opt, n_rays, pos, dir, weight,
-                       freq_hz, mode, per_ray_fm, s_max, n_psi, psi_edges, n_beams, beam_id, dP_dV, deposited_power, P_final,
-                       P_dep, n_points, status, traj_first, traj_count, traj_max_pts, traj_s, traj_xyz, traj_P, traj_dP_ds,
-                       traj_dP_dV_ray, counters);
+    return TORJ_HOST_JOB.multi_trace(m, "torj_multi_trace_plasmas", true, n_plasmas, plasmas, beam_plasma);
 }
 
 int torj_fp64_peak(torj_ctx* c, int32_t iters, double* tflops, double* ms) {

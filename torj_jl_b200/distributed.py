@@ -5,6 +5,8 @@ from __future__ import annotations
 
 import numpy as np
 
+from ._lib import exact_bins, profile_vector, split_profile_vector
+
 
 def shard_range(n_rays: int, rank: int, world_size: int) -> tuple[int, int]:
     """Contiguous block [lo, hi) of rank; sizes differ by at most one."""
@@ -125,7 +127,7 @@ class _ExactReduction:
             n_words, src, _ = self.agreed
             self._sum(torch.zeros(n_words, dtype=torch.int64, device=self.dev))
             self._agree_after(1)
-            vec = np.zeros((n_words - 2) // 8)  # a buffer's 2 status words, then 8 words per bin
+            vec = np.zeros(exact_bins(n_words))
             out = torch.zeros(len(vec), dtype=torch.float64, device=self.dev)
             self.dist.broadcast(out, src)
             local = dict(P_final=np.zeros(0), P_deposited_ray=np.zeros(0), n_points=np.zeros(0, dtype=np.int32),
@@ -149,8 +151,7 @@ class _ExactReduction:
                     pass
             raise
         self._agree_after(1)
-        vec_sum = np.concatenate([np.reshape(local["dP_dV"], (n_beams, -1)), np.reshape(local["deposited_power"], (n_beams, 1)),
-                                  np.reshape(local["sum_weights"], (n_beams, 1))], axis=1).ravel()
+        vec_sum = profile_vector(local["dP_dV"], local["deposited_power"], local["sum_weights"], n_beams)
         if self.agreed[2]:
             t = torch.from_numpy(vec_sum.copy()).to(self.dev)
             self.dist.broadcast(t, self.agreed[1])
@@ -206,22 +207,16 @@ def trace_sharded(trace_fn, ray_positions, ray_directions, ray_weights, *, n_bea
         local = trace_fn(pos[idx], dirs[idx], w[idx], **{k: v[idx] for k, v in per_ray.items()})
         if n_beams > 1:
             sw = np.bincount(per_ray["beam_id"][idx], weights=w[idx], minlength=n_beams)
-            vec = np.concatenate([np.reshape(local["dP_dV"], (n_beams, -1)), np.reshape(local["deposited_power"], (n_beams, 1)),
-                                  sw[:, None]], axis=1).ravel()
         else:
-            vec = np.concatenate([np.ravel(local["dP_dV"]), [float(local["deposited_power"]), float(np.sum(w[idx]))]])
+            sw = np.sum(w[idx])  # numpy's pairwise sum: a bincount would change the last bits
+        vec = profile_vector(local["dP_dV"], local["deposited_power"], sw, n_beams)
         t = torch.from_numpy(vec.copy())
         if device is not None:
             t = t.to(device)
         allreduce_profile(t)
         vec_sum = t.cpu().numpy()
-    if n_beams > 1:
-        rows = vec_sum.reshape(n_beams, -1)
-        out = dict(dP_dV=rows[:, :-2].copy(), deposited_power=rows[:, -2].copy(), sum_weights=rows[:, -1].copy(), local=local,
-                   idx=idx, local_vector=vec)
-    else:
-        out = dict(dP_dV=vec_sum[:-2], deposited_power=float(vec_sum[-2]), sum_weights=float(vec_sum[-1]), local=local, idx=idx,
-                   local_vector=vec)
+    dP_dV, deposited_power, sum_weights = split_profile_vector(vec_sum, n_beams)
+    out = dict(dP_dV=dP_dV, deposited_power=deposited_power, sum_weights=sum_weights, local=local, idx=idx, local_vector=vec)
     if gather_rays:
         mine = {k: np.asarray(local[k]) for k in ("P_final", "n_points", "status") if k in local}
         parts = [None] * world

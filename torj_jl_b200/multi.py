@@ -10,12 +10,8 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._lib import c_dp, c_ip, c_vp
+from ._lib import _p, c_vp
 from . import absorption
-
-
-def _p(a):
-    return a.ctypes.data_as(c_dp)
 
 
 class MultiGPU:
@@ -67,24 +63,15 @@ class MultiGPU:
         (torj_multi_trace_plasmas); each plasma's copies on the devices are made once and kept.
         exact_sum: the devices book exact fixed-point sums and add them as integers (torj_multi_set_exact_sum), so the
         profile has the bits of one device tracing the whole bundle, with NCCL or the host sum (at a fixed lanes_per_ray)."""
-        from .solve import _plasma_set, bundle_result, marshal_bundle
+        from .solve import _plasma_set, bundle_result, marshal_bundle, oneshot_args, plasma_call
         pls = _plasma_set(plasma, beam_plasma)
         m = marshal_bundle(ray_positions, ray_directions, ray_weights, f, mode, psi_dP_dV, beam_id, n_beams,
                            n_plasmas=len(pls) if pls else 1, beam_plasma=beam_plasma)
-        o, psi = m["out"], m["psi"]
         L = _lib.lib()
         opt = options or _lib.default_options()
         _lib.check(L.torj_multi_set_exact_sum(self.h, int(bool(exact_sum))))
-        rest = (C.byref(opt), m["n"], _p(m["pos"]), _p(m["dir"]), _p(m["w"]), _p(m["f"]), m["mode"].ctypes.data_as(c_ip),
-                m["per_ray"], float(s_max), len(psi), _p(psi), m["n_beams"],
-                m["beam"].ctypes.data_as(c_ip) if m["beam"] is not None else None, _p(o["prof"]), _p(o["dep"]), _p(o["Pf"]),
-                _p(o["Pd"]), o["npts"].ctypes.data_as(c_ip), o["st"].ctypes.data_as(c_ip), 0, 0, 0, None, None, None, None,
-                None, C.byref(o["cnt"]))
-        if pls is None:
-            _lib.check(L.torj_multi_trace(self.h, self._plasma(plasma), *rest))
-        else:
-            hs = (c_vp * len(pls))(*[self._plasma(p).value for p in pls])
-            _lib.check(L.torj_multi_trace_plasmas(self.h, len(pls), hs, m["beam_plasma"].ctypes.data_as(c_ip), *rest))
+        fn, pa = plasma_call(L, "torj_multi_trace", pls or plasma, m["beam_plasma"], self._plasma)
+        _lib.check(fn(self.h, *pa, *oneshot_args(m, opt, s_max)))
         return bundle_result(m)
 
     def make_beam_series(self, plasmas, r, phi, z, steering_angle_tor, steering_angle_pol, spot_size,

@@ -8,11 +8,7 @@ import numpy as np
 from scipy.interpolate import CubicSpline
 
 from . import _lib
-from ._lib import c_dp, c_vp
-
-
-def _p(a):
-    return a.ctypes.data_as(c_dp)
+from ._lib import _p, c_vp
 
 
 def _prefilter_2d(data_rz: np.ndarray) -> np.ndarray:

@@ -6,7 +6,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._lib import c_dp, c_ip
+from ._lib import _ip, _p, c_vp
 from .launch import launch_peripheral_rays
 from .plasma import Plasma
 from .synthetic import pol_tor_angles_2_vector
@@ -18,10 +18,6 @@ STATUS_TEXT = {
     4: "step limit reached", 5: "NaN in the ray state",
     6: "trajectory buffer too small",
 }
-
-
-def _p(a):
-    return a.ctypes.data_as(c_dp)
 
 
 def marshal_bundle(ray_positions, ray_directions, ray_weights, f, mode, psi_dP_dV, beam_id, n_beams, *, n_plasmas=1,
@@ -50,10 +46,33 @@ def marshal_bundle(ray_positions, ray_directions, ray_weights, f, mode, psi_dP_d
             raise ValueError(f"beam_plasma must lie in [0, {n_plasmas}) (one index into the plasmas per beam)")
         if n_plasmas > 1 and n_beams < 2:
             raise ValueError("several plasmas need several beams (beam_id, n_beams): a profile row belongs to one plasma")
-    out = dict(prof=np.zeros((n_beams, len(psi))), dep=np.zeros(n_beams), Pf=np.zeros(n), Pd=np.zeros(n),
-               npts=np.zeros(n, dtype=np.int32), st=np.zeros(n, dtype=np.int32), cnt=_lib.TorjCounters())
     return dict(pos=pos, dir=dr, n=n, w=wt, per_ray=per_ray, f=fr, mode=md, psi=psi, n_beams=n_beams, beam=bid,
-                beam_plasma=bp, out=out)
+                beam_plasma=bp, out=bundle_outputs(n, n_beams, len(psi)))
+
+
+def bundle_outputs(n, n_beams, n_psi):
+    """The result arrays of a bundle of n rays (`out` of marshal_bundle)."""
+    return dict(prof=np.zeros((n_beams, n_psi)), dep=np.zeros(n_beams), Pf=np.zeros(n), Pd=np.zeros(n),
+                npts=np.zeros(n, dtype=np.int32), st=np.zeros(n, dtype=np.int32), cnt=_lib.TorjCounters())
+
+
+def oneshot_args(m, opt, s_max, window=(0, 0, 0), traj=None):
+    """The arguments of torj_trace / torj_multi_trace (and their _plasmas forms) after the plasma ones, for the bundle m of
+    marshal_bundle, the trajectory window (first, count, max_pts) and trace_bundle's `traj` arrays (None: NULL)."""
+    o, psi = m["out"], m["psi"]
+    traj_bufs = [_p(a) for a in traj.values()] if traj is not None else [None] * 5
+    return (C.byref(opt), m["n"], _p(m["pos"]), _p(m["dir"]), _p(m["w"]), _p(m["f"]), _ip(m["mode"]), m["per_ray"],
+            float(s_max), len(psi), _p(psi), m["n_beams"], _ip(m["beam"]), _p(o["prof"]), _p(o["dep"]), _p(o["Pf"]),
+            _p(o["Pd"]), _ip(o["npts"]), _ip(o["st"]), *window, *traj_bufs, C.byref(o["cnt"]))
+
+
+def plasma_call(L, name, plasma, beam_plasma, handle):
+    """The library function of a trace through `plasma` and its plasma arguments: `name` with (handle(plasma),) for a
+    Plasma; `name`_plasmas with (n_plasmas, handles, beam_plasma) for a list of them."""
+    if isinstance(plasma, Plasma):
+        return getattr(L, name), (handle(plasma),)
+    hs = (c_vp * len(plasma))(*[handle(p).value for p in plasma])
+    return getattr(L, name + "_plasmas"), (len(plasma), hs, _ip(beam_plasma))
 
 
 def _plasma_list(plasma):
@@ -116,72 +135,67 @@ def trace_bundle(plasma, ray_positions, ray_directions, ray_weights, f, mode, s_
     ctx = ctx or _lib.context()
     L = _lib.lib()
     _lib.check(L.torj_ctx_set_exact_sum(ctx, int(bool(exact_sum))))
-    n, psi, o = m["n"], m["psi"], m["out"]
     opt = options or _lib.default_options()
     t_first, t_count = trajectories if trajectories else (0, 0)
     if t_count and traj_max_pts is None:
         traj_max_pts = 2 + int(opt.n_segments * (np.ceil(s_max / opt.n_segments / opt.dtmax) + 8))
     tm = int(traj_max_pts or 0)
+    window = (t_first, t_count, tm)
     ts = np.zeros((t_count, tm)); txyz = np.zeros((t_count, 3, tm)); tP = np.zeros((t_count, tm))
-    tdP = np.zeros((t_count, tm)); tprof = np.zeros((t_count, len(psi)))
+    tdP = np.zeros((t_count, tm)); tprof = np.zeros((t_count, len(m["psi"])))
     traj = dict(traj_s=ts, traj_xyz=txyz, traj_P=tP, traj_dP_ds=tdP, traj_dP_dV_ray=tprof)
     if reduce_exact is not None:
-        return _trace_reduced(L, ctx, plasma, pls, m, opt, s_max, (t_first, t_count, tm), traj, reduce_exact)
-    rest = (C.byref(opt), n, _p(m["pos"]), _p(m["dir"]), _p(m["w"]), _p(m["f"]), m["mode"].ctypes.data_as(c_ip), m["per_ray"],
-            float(s_max), len(psi), _p(psi), m["n_beams"], m["beam"].ctypes.data_as(c_ip) if m["beam"] is not None else None,
-            _p(o["prof"]), _p(o["dep"]), _p(o["Pf"]), _p(o["Pd"]), o["npts"].ctypes.data_as(c_ip), o["st"].ctypes.data_as(c_ip),
-            t_first, t_count, tm, _p(ts), _p(txyz), _p(tP), _p(tdP), _p(tprof), C.byref(o["cnt"]))
-    if pls is None:
-        _lib.check(L.torj_trace(ctx, plasma.handle(ctx), *rest))
-    else:
-        hs = (_lib.c_vp * len(pls))(*[p.handle(ctx).value for p in pls])
-        _lib.check(L.torj_trace_plasmas(ctx, len(pls), hs, m["beam_plasma"].ctypes.data_as(c_ip), *rest))
+        bh = c_vp()
+        _lib.check(L.torj_bundle_create(ctx, m["n"], _p(m["pos"]), _p(m["dir"]), _p(m["w"]), _p(m["f"]), _ip(m["mode"]),
+                                        m["per_ray"], C.byref(bh)))
+        return _trace_resident(ctx, bh, m, pls or plasma, m["beam_plasma"], opt, s_max, traj=traj, reduce_exact=reduce_exact,
+                               prepare=[(L.torj_bundle_set_beams, bh, m["n_beams"], _ip(m["beam"])),
+                                        (L.torj_bundle_set_window, bh, *window)])
+    fn, pa = plasma_call(L, "torj_trace", pls or plasma, m["beam_plasma"], lambda p: p.handle(ctx))
+    _lib.check(fn(ctx, *pa, *oneshot_args(m, opt, s_max, window, traj)))
     res = bundle_result(m)
     res.update(traj)
     return res
 
 
-def _trace_reduced(L, ctx, plasma, pls, m, opt, s_max, window, traj, reduce_exact):
-    """trace_bundle with reduce_exact: the same trace on a resident bundle, whose exact words reduce_exact sums across
-    processes before they are converted (torj_bundle_device_exact_words / torj_bundle_finalize_exact)."""
-    import torch
-
-    n, psi, o, nb = m["n"], m["psi"], m["out"], m["n_beams"]
-    t_first, t_count, tm = window
-    bh = _lib.c_vp()
-    _lib.check(L.torj_bundle_create(ctx, n, _p(m["pos"]), _p(m["dir"]), _p(m["w"]), _p(m["f"]), m["mode"].ctypes.data_as(c_ip),
-                                    m["per_ray"], C.byref(bh)))
+def _trace_resident(ctx, bh, m, plasma, beam_plasma, opt, s_max, *, prepare=(), traj=None, reduce_exact=None):
+    """Trace the bundle bh that the caller has just created, and destroy it however the call ends: the library calls
+    `prepare` [(fn, *args)], the trace through `plasma`, reduce_exact's sum of the exact words (see trace_bundle), then
+    the results into m's arrays (ray weights too when m["out"] has "w") and the trajectories into traj's arrays."""
+    L = _lib.lib()
+    o, nb, psi = m["out"], m["n_beams"], m["psi"]
+    res = dict(traj or {})
     try:
-        _lib.check(L.torj_bundle_set_beams(bh, nb, m["beam"].ctypes.data_as(c_ip) if m["beam"] is not None else None))
-        _lib.check(L.torj_bundle_set_window(bh, t_first, t_count, tm))
-        if pls is None:
-            _lib.check(L.torj_bundle_trace(bh, plasma.handle(ctx), C.byref(opt), float(s_max), len(psi), _p(psi)))
-        else:
-            hs = (_lib.c_vp * len(pls))(*[p.handle(ctx).value for p in pls])
-            _lib.check(L.torj_bundle_trace_plasmas(bh, len(pls), hs, m["beam_plasma"].ctypes.data_as(c_ip), C.byref(opt),
-                                                   float(s_max), len(psi), _p(psi)))
-        ptr, n_words = _lib.c_vp(), C.c_int64()
-        _lib.check(L.torj_bundle_device_exact_words(bh, C.byref(ptr), C.byref(n_words)))
-        n_vec = nb * (len(psi) + 2)
-        # the library works on its context's stream, the reduction on torch's current one: each waits for the other
-        _lib.check(L.torj_ctx_sync(ctx))
-        local_vector = device_tensor(L.torj_bundle_device_profile(bh), n_vec, "<f8").cpu().numpy()
-        words = device_tensor(ptr.value, n_words.value, "<i8")
-        reduce_exact(words)
-        if words.is_cuda:
-            torch.cuda.current_stream(words.device).synchronize()
-        _lib.check(L.torj_bundle_finalize_exact(bh))
-        _lib.check(L.torj_bundle_results(bh, _p(o["prof"]), _p(o["dep"]), _p(o["Pf"]), _p(o["Pd"]), o["npts"].ctypes.data_as(c_ip),
-                                         o["st"].ctypes.data_as(c_ip), C.byref(o["cnt"])))
-        if t_count:
-            _lib.check(L.torj_bundle_trajectories(bh, *(_p(traj[k]) for k in ("traj_s", "traj_xyz", "traj_P", "traj_dP_ds",
-                                                                             "traj_dP_dV_ray"))))
-        sw = device_tensor(L.torj_bundle_device_profile(bh), n_vec, "<f8").cpu().numpy().reshape(nb, -1)[:, -1]
+        for fn, *args in prepare:
+            _lib.check(fn(*args))
+        fn, pa = plasma_call(L, "torj_bundle_trace", plasma, beam_plasma, lambda p: p.handle(ctx))
+        _lib.check(fn(bh, *pa, C.byref(opt), float(s_max), len(psi), _p(psi)))
+        if reduce_exact is not None:
+            import torch
+
+            ptr, n_words = c_vp(), C.c_int64()
+            _lib.check(L.torj_bundle_device_exact_words(bh, C.byref(ptr), C.byref(n_words)))
+            n_vec = nb * (len(psi) + 2)
+            # the library works on its context's stream, the reduction on torch's current one: each waits for the other
+            _lib.check(L.torj_ctx_sync(ctx))
+            local_vector = device_tensor(L.torj_bundle_device_profile(bh), n_vec, "<f8").cpu().numpy()
+            words = device_tensor(ptr.value, n_words.value, "<i8")
+            reduce_exact(words)
+            if words.is_cuda:
+                torch.cuda.current_stream(words.device).synchronize()
+            _lib.check(L.torj_bundle_finalize_exact(bh))
+        _lib.check(L.torj_bundle_results(bh, _p(o["prof"]), _p(o["dep"]), _p(o["Pf"]), _p(o["Pd"]), _ip(o["npts"]),
+                                         _ip(o["st"]), C.byref(o["cnt"])))
+        if "w" in o:
+            _lib.check(L.torj_bundle_rays(bh, None, None, _p(o["w"])))
+        if traj is not None and len(traj["traj_s"]):
+            _lib.check(L.torj_bundle_trajectories(bh, *(_p(a) for a in traj.values())))
+        if reduce_exact is not None:
+            vec = device_tensor(L.torj_bundle_device_profile(bh), n_vec, "<f8").cpu().numpy()
+            res.update(sum_weights=_lib.split_profile_vector(vec, nb)[2], local_vector=local_vector)
     finally:
         L.torj_bundle_destroy(bh)
-    res = bundle_result(m)
-    res.update(traj, sum_weights=sw.copy() if nb > 1 else float(sw[0]), local_vector=local_vector)
-    return res
+    return {**bundle_result(m), **res}
 
 
 def cylindrical_state(xyz, P):
@@ -208,13 +222,22 @@ def make_ray(plasma: Plasma, x0, N_vacuum, f, mode, s_max, psi_dP_dV, *, options
     return s, u, r["traj_P"][0, :n].copy(), r["traj_dP_dV_ray"][0].copy(), float(r["P_deposited_ray"][0])
 
 
+def launch_geometry(r, phi, z, steering_angle_tor, steering_angle_pol):
+    """make_beam's launch point x0 = (r cos phi, r sin phi, z) (reference src/solve.jl:212-215) and direction N0
+    (src/solve.jl:211); componentwise, so arrays of n launchers give [3, n] each."""
+    return (np.array([r * np.cos(phi), r * np.sin(phi), z]),
+            pol_tor_angles_2_vector(steering_angle_pol, steering_angle_tor))
+
+
+GEOMETRY = ("r", "phi", "z", "steering_angle_tor", "steering_angle_pol")  # launch_geometry's keys of a launcher
+
+
 def make_beam(plasma: Plasma, r, phi, z, steering_angle_tor, steering_angle_pol, spot_size, inverse_curvature_radius,
               f, mode, s_max, psi_dP_dV, *, options=None, ctx=None, exact_sum=False, **kwargs):
     """make_beam(...) -> (arc_lengths, trajectories, ray_powers, dP_dV, deposited_power, ray_weights)
     — reference src/solve.jl:209-210,241; kwargs go to launch_peripheral_rays (src/solve.jl:216-217).
     exact_sum: see trace_bundle."""
-    N0 = pol_tor_angles_2_vector(steering_angle_pol, steering_angle_tor)  # src/solve.jl:211
-    x0 = np.array([r * np.cos(phi), r * np.sin(phi), z])                  # src/solve.jl:212-215
+    x0, N0 = launch_geometry(r, phi, z, steering_angle_tor, steering_angle_pol)
     pos, dirs, wts = launch_peripheral_rays(x0, N0, spot_size, inverse_curvature_radius, f, **kwargs)
     n = len(wts)
     res = trace_bundle(plasma, pos, dirs, wts, float(f), int(mode), s_max, psi_dP_dV, options=options, ctx=ctx,
@@ -257,42 +280,26 @@ def _make_beams_device(plasma, launchers, s_max, psi_dP_dV, options, ctx, exact_
     if N_rings < 2:
         raise ValueError(f"N_rings = {N_rings} < 2 which is the minimum")
     nl = len(launchers)
-    x0 = np.array([[q["r"] * np.cos(q["phi"]), q["r"] * np.sin(q["phi"]), q["z"]] for q in launchers]).T.copy()
-    N0 = np.array([pol_tor_angles_2_vector(q["steering_angle_pol"], q["steering_angle_tor"]) for q in launchers]).T.copy()
-    w = np.array([q["spot_size"] for q in launchers], dtype=np.float64)
-    irc = np.array([q["inverse_curvature_radius"] for q in launchers], dtype=np.float64)
-    f = np.array([q["f"] for q in launchers], dtype=np.float64)
-    md = np.array([q["mode"] for q in launchers], dtype=np.int32)
+
+    def col(k, dtype=np.float64):
+        return np.array([q[k] for q in launchers], dtype=dtype)
+    x0, N0 = launch_geometry(*map(col, GEOMETRY))
+    w, irc, f, md = col("spot_size"), col("inverse_curvature_radius"), col("f"), col("mode", np.int32)
     gx, gw = np.polynomial.hermite.hermgauss(2 * N_rings + 2)
-    bh = _lib.c_vp(); n = C.c_int64()
-    _lib.check(L.torj_bundle_create_from_launchers(ctx, nl, _p(x0), _p(N0), _p(w), _p(irc), _p(f), md.ctypes.data_as(c_ip),
-                                                   int(N_rings), int(min_azimuthal_points), int(bool(normalize_weight_sum)),
-                                                   _p(np.ascontiguousarray(gx)), _p(np.ascontiguousarray(gw)), C.byref(bh),
-                                                   C.byref(n)))
-    try:
-        n = int(n.value)
-        psi = np.ascontiguousarray(psi_dP_dV, dtype=np.float64)
-        opt = options or _lib.default_options()
-        _lib.check(L.torj_ctx_set_exact_sum(ctx, int(bool(exact_sum))))
-        if pls is None:
-            _lib.check(L.torj_bundle_trace(bh, plasma.handle(ctx), C.byref(opt), float(s_max), len(psi), _p(psi)))
-        else:
-            hs = (_lib.c_vp * len(pls))(*[p.handle(ctx).value for p in pls])
-            _lib.check(L.torj_bundle_trace_plasmas(bh, len(pls), hs, bp.ctypes.data_as(c_ip), C.byref(opt), float(s_max),
-                                                   len(psi), _p(psi)))
-        prof = np.zeros((nl, len(psi))); dep = np.zeros(nl)
-        Pf = np.zeros(n); Pd = np.zeros(n); npts = np.zeros(n, dtype=np.int32); st = np.zeros(n, dtype=np.int32)
-        cnt = _lib.TorjCounters()
-        _lib.check(L.torj_bundle_results(bh, _p(prof), _p(dep), _p(Pf), _p(Pd), npts.ctypes.data_as(c_ip),
-                                         st.ctypes.data_as(c_ip), C.byref(cnt)))
-        wt = np.zeros(n)
-        _lib.check(L.torj_bundle_rays(bh, None, None, _p(wt)))
-    finally:
-        L.torj_bundle_destroy(bh)
-    per = n // nl
-    res = dict(dP_dV=prof, deposited_power=dep, P_final=Pf, P_deposited_ray=Pd, n_points=npts, status=st,
-               counters=cnt.as_dict())
-    return prof, dep, [wt[i * per:(i + 1) * per] for i in range(nl)], [Pf[i * per:(i + 1) * per] for i in range(nl)], res
+    psi = np.ascontiguousarray(psi_dP_dV, dtype=np.float64)
+    bh, n = c_vp(), C.c_int64()
+    _lib.check(L.torj_bundle_create_from_launchers(ctx, nl, _p(x0), _p(N0), _p(w), _p(irc), _p(f), _ip(md), int(N_rings),
+                                                   int(min_azimuthal_points), int(bool(normalize_weight_sum)), _p(gx), _p(gw),
+                                                   C.byref(bh), C.byref(n)))
+    m = dict(out=dict(bundle_outputs(n.value, nl, len(psi)), w=np.zeros(n.value)), n_beams=nl, psi=psi)
+    res = _trace_resident(ctx, bh, m, pls or plasma, bp, options or _lib.default_options(), s_max,
+                          prepare=[(L.torj_ctx_set_exact_sum, ctx, int(bool(exact_sum)))])
+    wt, Pf = m["out"]["w"], res["P_final"]
+    # [n_launchers, n_psi] and [n_launchers] for one launcher too
+    res.update(dP_dV=np.atleast_2d(res["dP_dV"]), deposited_power=np.atleast_1d(res["deposited_power"]))
+    per = len(Pf) // nl
+    return (res["dP_dV"], res["deposited_power"], [wt[i * per:(i + 1) * per] for i in range(nl)],
+            [Pf[i * per:(i + 1) * per] for i in range(nl)], res)
 
 
 def make_beams(plasma, launchers, s_max, psi_dP_dV, *, options=None, ctx=None, device_launch=False, exact_sum=False, **kwargs):
@@ -307,8 +314,7 @@ def make_beams(plasma, launchers, s_max, psi_dP_dV, *, options=None, ctx=None, d
     pls, bp = _launcher_plasmas(plasma, launchers)
     P, D, W, F, M, B = [], [], [], [], [], []
     for b, L in enumerate(launchers):
-        N0 = pol_tor_angles_2_vector(L["steering_angle_pol"], L["steering_angle_tor"])
-        x0 = np.array([L["r"] * np.cos(L["phi"]), L["r"] * np.sin(L["phi"]), L["z"]])
+        x0, N0 = launch_geometry(*(L[k] for k in GEOMETRY))
         p, d, w = launch_peripheral_rays(x0, N0, L["spot_size"], L["inverse_curvature_radius"], L["f"], **kwargs)
         P.append(p); D.append(d); W.append(w)
         F.append(np.full(len(w), float(L["f"]))); M.append(np.full(len(w), int(L["mode"]), dtype=np.int32))
@@ -343,8 +349,7 @@ def beam_series(trace, plasmas, r, phi, z, steering_angle_tor, steering_angle_po
     if pls is None:
         pls = [plasmas]
     K = len(pls)
-    N0 = pol_tor_angles_2_vector(steering_angle_pol, steering_angle_tor)
-    x0 = np.array([r * np.cos(phi), r * np.sin(phi), z])
+    x0, N0 = launch_geometry(r, phi, z, steering_angle_tor, steering_angle_pol)
     pos, dirs, wts = launch_peripheral_rays(x0, N0, spot_size, inverse_curvature_radius, f, **kwargs)
     n = len(wts)
     res = trace(pls, np.tile(pos, (K, 1)), np.tile(dirs, (K, 1)), np.tile(wts, K), float(f), int(mode), s_max, psi_dP_dV,
